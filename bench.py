@@ -16,6 +16,7 @@ timed region: each rank's trace kernel stores them there itself over NVLink (CUD
 mapping, turtle_b200.dist.PeerRecords), with an NCCL gather as the fall-back.
 
     python bench.py [--gpus N] [--steps K] [--warmup W] [--rays R] [--impl reference]
+                    [--dump-outputs DIR]
 
 prints ONE JSON line (see the keys at the bottom of main()).
   value      whole-job Mrays/s with rays resident in HBM (device-pointer C ABI call,
@@ -55,6 +56,8 @@ ALTITUDE_MAX, MAX_STEPS = 9000.0, 100000
 N_AZ = N_EL = 4096
 BYTES_PER_RAY = 48 + 96  # position + direction in, result record out
 BYTES_PER_SAMPLE = 8     # four 16-bit nodes
+# --dump-outputs: a fixed, seeded sample of the records (120 B per ray as float64: 32 MB)
+DUMP_RAYS, DUMP_SEED = 1 << 18, 0x7075727474
 
 
 def _synth():
@@ -104,6 +107,25 @@ def fan_subsample(rank, world, stride, n_total):
     r = np.arange(0, n_total, stride, dtype=np.int64)
     az, el = synth.fan_angles(r, N_AZ, N_EL, part=rank, parts=world)
     return synth.np_from_horizontal(np.full(len(r), DET_LAT), np.full(len(r), DET_LON), az, el)
+
+
+def dump_sample(n):
+    """Rows of a batch of n rays that --dump-outputs writes: all of them up to DUMP_RAYS,
+    else the same seeded sample of DUMP_RAYS rows on every run (ascending)."""
+    if n <= DUMP_RAYS:
+        return np.arange(n, dtype=np.int64)
+    return np.sort(np.random.default_rng(DUMP_SEED).choice(n, DUMP_RAYS, replace=False))
+
+
+def dump_outputs(directory, rays, records):
+    """DIR/<field>.npy for every field of the result records (float64; the integer fields
+    are exact in it) and DIR/ray.npy, the index of each record's ray in the rank's fan of
+    N_AZ x N_EL rays: the same numbering in both arms, whatever part of the fan they trace."""
+    os.makedirs(directory, exist_ok=True)
+    np.save(os.path.join(directory, "ray.npy"), rays.astype(np.float64))
+    for name in records.dtype.names:
+        np.save(os.path.join(directory, name + ".npy"),
+                np.ascontiguousarray(records[name], dtype=np.float64))
 
 
 class ClockSampler:
@@ -181,10 +203,13 @@ def run_reference(args):
         cpu_trace(d, H, 0, args.gpus, stride * 8, n_total, cores)
     t_all, rays_all, steps_all = 0., 0, 0
     for _ in range(args.steps):
-        _, steps, seconds, n = cpu_trace(d, H, 0, args.gpus, stride, n_total, cores)
+        res, steps, seconds, n = cpu_trace(d, H, 0, args.gpus, stride, n_total, cores)
         t_all += seconds
         rays_all += n
         steps_all += steps
+    if args.dump_outputs:
+        rows = dump_sample(len(res))
+        dump_outputs(args.dump_outputs, rows * stride, res[rows])
     value = rays_all / t_all / 1e6
     line = {
         "impl": "reference", "metric": "Mrays/s", "value": value, "unit": "Mrays/s",
@@ -248,7 +273,14 @@ def main():
     ap.add_argument("--no-e2e", action="store_true")
     ap.add_argument("--ctas-per-sm", type=int, default=0)
     ap.add_argument("--threads", type=int, default=0)
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="after the timed steps, write the result records of the last one "
+                         "(rank 0's rays, at most %d of them: a fixed seeded sample) as "
+                         "DIR/<field>.npy in float64, and DIR/ray.npy: the index of each "
+                         "ray in the fan" % DUMP_RAYS)
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     if args.warmup < 3 and args.impl == "b200":
         args.warmup = 3  # timing rule: at least 3 warm-up steps
 
@@ -388,6 +420,11 @@ def main():
         status = peer.tensor.view(world, n, 96)[:, :, 76:80].contiguous().view(torch.int32)
         assert int((status < 0).sum().item()) == 0 and int((status > 4).sum().item()) == 0
         d_res.copy_(peer.tensor[:n])
+    if args.dump_outputs and rank == 0:
+        rows = dump_sample(n)
+        picked = d_res.index_select(0, torch.from_numpy(rows).to(dev)).cpu().numpy()
+        rays = rows if full else rows * ((N_AZ * N_EL) // n)
+        dump_outputs(args.dump_outputs, rays, picked.view(tb.TRACE_RESULT).reshape(len(rows)))
 
     # kernel alone (no gather), CUDA events on the launching stream: the roofline input
     k0, k1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)

@@ -4,7 +4,7 @@
 pthread ray loop of trace_driver.c. Three libraries are of interest:
 
   REF     oracle/_ref/libturtle_ref.so  the unmodified reference (built by
-          oracle/Makefile from /root/reference; travels to the GPU box prebuilt)
+          oracle/Makefile from REF_SOURCES below)
   REF_FMA oracle/_ref/libturtle_ref_fma.so  the same sources built with FMA contraction:
           the rounding-noise floor of the path (oracle/parity.py), never the checker
   PORT    oracle/liboracle.so           the plain-C restatement (turtle_oracle.c)
@@ -19,6 +19,9 @@ import os
 import numpy as np
 
 HERE = os.path.dirname(os.path.abspath(__file__))
+# the unmodified reference's sources, which oracle/Makefile builds _ref/ from (same default)
+REF_SOURCES = os.environ.get("TURTLE_REF") or os.path.join(os.path.dirname(os.path.dirname(HERE)),
+                                                           "reference")
 REF = os.path.join(HERE, "_ref", "libturtle_ref.so")
 # the same sources with FMA contraction: the rounding-noise floor, not an oracle
 REF_FMA = os.path.join(HERE, "_ref", "libturtle_ref_fma.so")

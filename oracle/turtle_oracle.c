@@ -20,7 +20,7 @@
  * it can arbitrate when the product's simplifications are questioned.
  *
  * PINNING: tests/test_oracle.py checks this restatement bit-for-bit against the
- * compiled reference (oracle/_ref/libturtle_ref.so, when /root/reference is
+ * compiled reference (oracle/_ref/libturtle_ref.so, when the reference's sources are
  * available), against the golden vectors under tests/golden/ that were generated
  * from the reference (tests/golden/make_golden.py), and against the closed-form
  * assertions of the reference's own test-suite (tests/test-turtle.c, listed in

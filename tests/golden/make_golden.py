@@ -1,7 +1,7 @@
 """Generate the golden vectors of tests/golden/ from the UNMODIFIED reference.
 
-Run in the build container (where /root/reference exists and oracle/Makefile has
-built oracle/_ref/libturtle_ref.so):
+Run where oracle/Makefile has built oracle/_ref/libturtle_ref.so from the reference's
+sources (TURTLE_REF):
 
     python tests/golden/make_golden.py
 
@@ -45,6 +45,7 @@ def geodesy(ref, out):
     out.update(geo_lat=lat, geo_lon=lon, geo_alt=alt, geo_ecef=ecef, geo_ecef_all=ecef_all,
                geo_back_lat=la, geo_back_lon=lo, geo_back_alt=al, hor_az=az, hor_el=el,
                hor_dir=d, hor_back_az=az2, hor_back_el=el2)
+    shrink_geodesy(out, n)
     pla = rng.uniform(41., 51., 1024)
     plo = rng.uniform(-5., 9., 1024)
     out.update(proj_lat=pla, proj_lon=plo)
@@ -54,6 +55,18 @@ def geodesy(ref, out):
         key = t.replace(" ", "_").replace(".", "p")
         out["proj_%s_x" % key], out["proj_%s_y" % key] = x, y
         out["proj_%s_lat" % key], out["proj_%s_lon" % key] = bla, blo
+
+
+def shrink_geodesy(out, n):
+    """Keep every other random row (and all the special ones) of the n-row geodesy
+    vectors, so that the stored file stays under 1 MB."""
+    keep = np.r_[0:n - 6:2, n - 6:n]
+    keep_all = np.r_[keep, n:n + 5]  # + the pole / axis inputs of ecef_all
+    for k in ("geo_lat", "geo_lon", "geo_alt", "geo_ecef", "hor_az", "hor_el", "hor_dir",
+              "hor_back_az", "hor_back_el"):
+        out[k] = out[k][keep]
+    for k in ("geo_ecef_all", "geo_back_lat", "geo_back_lon", "geo_back_alt"):
+        out[k] = out[k][keep_all]
 
 
 def maps(ref, out):

@@ -1,6 +1,6 @@
 """Generate the file-format fixtures of tests/golden/io/ with the UNMODIFIED reference.
 
-Run in the build container (oracle/_ref/libturtle_ref.so built, /root/reference present):
+Run where oracle/_ref/libturtle_ref.so is built and the reference's sources are present:
 
     python tests/golden/make_io_golden.py
 

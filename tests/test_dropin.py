@@ -11,7 +11,6 @@ from oracle import harness as H
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 SRC = os.path.join(ROOT, "tests", "c", "dropin_stepper.c")
-REF_INCLUDE = "/root/reference/include"
 
 
 def build(tmp, name, include, libdir, lib):
@@ -30,12 +29,14 @@ def test_c_caller_compiles_and_runs_against_our_abi(tmp_path):
     assert all(int(l.split()[1]) > 5 for l in lines[:-1])
 
 
-@pytest.mark.skipif(not (os.path.exists(H.REF) and os.path.isdir(REF_INCLUDE)),
-                    reason="reference library / header not available here")
+@pytest.mark.skipif(not (os.path.exists(H.REF) and
+                         os.path.isdir(os.path.join(H.REF_SOURCES, "include"))),
+                    reason="needs the reference's sources (TURTLE_REF) and oracle/_ref built from them")
 def test_same_bits_as_the_reference(tmp_path):
     ours = build(str(tmp_path), "ours", os.path.join(ROOT, "include"),
                  os.path.join(ROOT, "turtle_b200"), "turtle_b200")
-    ref = build(str(tmp_path), "ref", REF_INCLUDE, os.path.dirname(H.REF), "turtle_ref")
+    ref = build(str(tmp_path), "ref", os.path.join(H.REF_SOURCES, "include"),
+                os.path.dirname(H.REF), "turtle_ref")
     a = subprocess.check_output([ours, "24"], text=True)
     b = subprocess.check_output([ref, "24"], text=True)
     assert a == b

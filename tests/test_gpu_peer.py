@@ -75,7 +75,7 @@ def _worker(rank, size, port, stack_dir, n, out_path):
 
 def test_peer_records_world2(small_stack, tmp_path):
     if tb.device_count() < 2:
-        pytest.skip("needs 2 GPUs (run under gpurun --gpus 2)")
+        pytest.skip("needs 2 GPUs")
     n = 60000 + 3
     out = str(tmp_path / "peer.npy")
     mp.spawn(_worker, args=(2, 29731 + os.getpid() % 1000, small_stack, n, out), nprocs=2,

@@ -18,7 +18,7 @@ from turtle_b200 import synth
 
 needs_floor = pytest.mark.skipif(
     not (H.available(H.REF) and H.available(H.REF_FMA)),
-    reason="needs oracle/_ref (built where /root/reference exists)")
+    reason="needs oracle/_ref (built where the reference's sources are found)")
 
 
 def records(n):

@@ -1,7 +1,8 @@
-"""The reference's own example programs, UNMODIFIED (compiled from where they lie under
-/root/reference/examples), linked once against the unmodified reference library and once
-against libturtle_b200.so + include/turtle.h: same files written, same text printed. This is
-the drop-in claim of INTEGRATION.md section 1 taken literally -- example-projection
+"""The reference's own example programs, UNMODIFIED (compiled from where they lie, in the
+examples/ of the reference's sources: oracle.harness.REF_SOURCES), linked once against the
+unmodified reference library and once against libturtle_b200.so + include/turtle.h: same
+files written, same text printed. This is the drop-in claim of INTEGRATION.md section 1
+taken literally -- example-projection
 (stack -> Lambert 93 map -> PNG), example-demo (map meta data, projections, ECEF,
 horizontal angles), example-stepper (the hot path: geoid + flat / stack / map layer, local
 approximation on and off, a ray marched to 2 km of altitude) and example-pthread (clients of
@@ -19,14 +20,16 @@ import numpy as np
 import pytest
 
 import turtle_b200 as tb
+from oracle import harness as H
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
-EXAMPLES = "/root/reference/examples"
-REF_LIB = os.path.join(ROOT, "oracle", "_ref", "libturtle_ref.so")
+EXAMPLES = os.path.join(H.REF_SOURCES, "examples")
+REF_LIB = H.REF
 
 pytestmark = pytest.mark.skipif(
-    not os.path.isdir(EXAMPLES) or not os.path.exists(REF_LIB) or shutil.which("gcc") is None,
-    reason="needs /root/reference, the built reference and gcc")
+    not os.path.isdir(EXAMPLES) or not os.path.exists(REF_LIB) or
+    shutil.which("gcc") is None,
+    reason="needs the reference's sources (TURTLE_REF), oracle/_ref built from them and gcc")
 
 
 def _shim(tmp):
@@ -70,7 +73,8 @@ def world(tmp_path_factory):
         f.write("#include <time.h>\ntime_t time(time_t * t) { if (t) *t = 42; return 42; }\n")
     subprocess.run(["gcc", "-shared", "-fPIC", "-o", os.path.join(tmp, "fixed_time.so"),
                     os.path.join(tmp, "fixed_time.c")], check=True)
-    sides = {"reference": ("/root/reference/include", os.path.dirname(REF_LIB), "turtle_ref"),
+    sides = {"reference": (os.path.join(H.REF_SOURCES, "include"), os.path.dirname(REF_LIB),
+                           "turtle_ref"),
              "product": (os.path.join(ROOT, "include"), os.path.join(ROOT, "turtle_b200"),
                          "turtle_b200")}
     for side, (inc, libdir, lib) in sides.items():

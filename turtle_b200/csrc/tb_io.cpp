@@ -1,7 +1,7 @@
 /*
  * tb_io.cpp -- readers / writers of the reference's DEM formats (see tb_io.hpp).
  *
- * Reference behaviour restated per format (file:line in /root/reference):
+ * Reference behaviour restated per format (file:line in the reference's sources):
  *   hgt  src/turtle/io/hgt.c:61-147      name -> origin and size; big-endian int16, north first
  *   png  src/turtle/io/png16.c:195-377   16-bit gray, JSON "topography" object in a text chunk
  *        src/turtle/io/png16.c:456-546   writer: tEXt "Comment" with %a formatted bounds
