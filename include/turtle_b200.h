@@ -291,7 +291,8 @@ TURTLE_API enum turtle_return turtle_stepper_trace_crossings_device(
 /* ---- one turtle_stepper_step for n independent particles -------------------
  * Same outputs as the scalar call (any output pointer may be NULL; direction
  * NULL = query mode, position untouched). `states` may be NULL: every particle
- * then starts from a reset stepper (exact when range <= 0). */
+ * then starts from a reset stepper (exact when range <= 0). States may be destroyed
+ * before or after the plan they were created for. */
 TURTLE_API enum turtle_return turtle_states_create(
     struct turtle_plan * plan, size_t n, struct turtle_states ** states);
 TURTLE_API void turtle_states_destroy(struct turtle_states ** states);

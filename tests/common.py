@@ -18,11 +18,12 @@ class Scene:
         self.range, self.slope, self.resolution = range, slope, resolution
 
     def oracle(self, library=None, locked=False):
+        """`locked`: one flag for all stacks, or one per stack."""
         d = H.Driver(library or H.best_oracle())
         for m in self.maps:
             d.map_create(m["nx"], m["ny"], m["x"], m["y"], m["z"], m["projection"], m["values"])
-        for s in self.stacks:
-            d.stack_create(s, locked=locked)
+        for i, s in enumerate(self.stacks):
+            d.stack_create(s, locked=locked[i] if isinstance(locked, (list, tuple)) else locked)
         d.geometry(self.ops, geoid=self.geoid, range=self.range, slope=self.slope,
                    resolution=self.resolution)
         return d
@@ -73,6 +74,68 @@ def geoid_map():
     vals = 30. + 10. * np.sin(np.radians(lon))[None, :] * np.cos(np.radians(lat))[:, None]
     return dict(nx=361, ny=181, x=(0., 360.), y=(-90., 90.), z=(-100., 100.), projection=None,
                 values=vals)
+
+
+TAGS = ["Lambert 93", "Lambert I", "Lambert II", "Lambert IIe", "Lambert III", "Lambert IV",
+        "UTM 31N", "UTM 3.0N", None]
+
+
+def second_stack(directory):
+    """A tile stack that differs from conftest's `small_stack` in extent (1 x 3 tiles from
+    N45 E001), tile resolution (3601 nodes) and the missing tile (45, 1), so that a wrong
+    tile table offset or a wrong per-stack tile shape changes the answer. Its terrain has
+    another seed."""
+    synth.write_hgt_stack(directory, 45, 1, 1, 3, n=3601, seed=synth.SEED + 1, skip=((45, 1),))
+    return directory
+
+
+def random_map(rng, ref):
+    tag = TAGS[rng.integers(len(TAGS))]
+    nx, ny = int(rng.integers(20, 120)), int(rng.integers(20, 120))
+    lat_c, lon_c = rng.uniform(45.3, 46.7), rng.uniform(2.3, 3.7)
+    if tag is None:
+        half = rng.uniform(0.02, 0.3)
+        x, y = (lon_c - half, lon_c + half), (lat_c - half, lat_c + half)
+    else:
+        cx, cy = ref.project(tag, [lat_c], [lon_c])
+        half = rng.uniform(1000., 20000.)
+        x, y = (cx[0] - half, cx[0] + half), (cy[0] - half, cy[0] + half)
+    values = np.resize(synth.fbm_grid(np.arange(nx) * rng.uniform(1, 8),
+                                      np.arange(ny) * rng.uniform(1, 8),
+                                      seed=int(rng.integers(1 << 30))), (ny, nx))
+    return dict(nx=nx, ny=ny, x=x, y=y, z=(0., 3000.), projection=tag,
+                values=values * rng.uniform(500, 3000))
+
+
+def random_scene(rng, ref, tiles, tiles2=None):
+    """1 - 3 layers of 1 - 3 data each: flat, tile stacks and maps in nine projections
+    (geodetic maps included), offsets, geoid on or off, local approximation range 0 / 1 /
+    10 / 100, random slope and resolution factors. With `tiles2` every stack datum is one
+    of the two stacks at random. Rays over lat 44.9 - 47.1, lon 1.9 - 4.1 see all of it."""
+    n_maps = int(rng.integers(0, 4))
+    maps = [random_map(rng, ref) for _ in range(n_maps)]
+    geoid = -1
+    if rng.random() < 0.4:
+        maps.append(geoid_map())
+        geoid = len(maps) - 1
+    stacks = [tiles] if tiles2 is None else [tiles, tiles2]
+    ops = []
+    for layer in range(int(rng.integers(1, 4))):
+        if layer > 0:
+            ops.append((H.ADD_LAYER, 0, 0.))
+        for _ in range(int(rng.integers(1, 4))):
+            kind = rng.integers(3)
+            offset = float(rng.uniform(-50, 50) + 400. * layer)
+            if (kind == 1) and (n_maps > 0):
+                ops.append((H.ADD_MAP, int(rng.integers(n_maps)), offset))
+            elif (kind == 0) and (rng.random() < 0.5):
+                ops.append((H.ADD_FLAT, 0, float(rng.uniform(-100, 500) + 400 * layer)))
+            else:
+                ops.append((H.ADD_STACK, int(rng.integers(len(stacks))) if tiles2 else 0,
+                            offset))
+    return Scene(maps=maps, stacks=stacks, ops=ops, geoid=geoid,
+                 range=[0., 1., 10., 100.][rng.integers(4)], slope=float(rng.uniform(0.1, 1.)),
+                 resolution=float(10 ** rng.uniform(-3, 0)))
 
 
 def ulp_distance(a, b):

@@ -133,3 +133,19 @@ def test_position_batch(small_stack):
     assert (wi == -1).any()
     with pytest.raises(tb.TurtleError):
         plan.position(la, lo, h, 5)
+
+
+def test_states_outlive_their_plan(small_stack):
+    """Particle states may be destroyed after their plan (a garbage collector finalises
+    the two in any order): that leaves no CUDA error behind for the next call to report."""
+    import ctypes
+    sc = c3(small_stack, 1., -1)
+    stepper, maps, stacks = sc.product()
+    plan = stepper.freeze(0)
+    states = plan.states(100)
+    tb.api.lib.turtle_plan_destroy(ctypes.byref(plan.handle))
+    assert not plan.handle
+    del states
+    other = stepper.freeze(0)
+    pos, idx = other.position([45.5], [2.5], [1.], 0)
+    assert idx[0] >= 0

@@ -1,6 +1,6 @@
-"""Random geometries, host side: 1 - 3 layers of 1 - 3 data each (flat / tile stack / maps
-in nine projections, geodetic maps included), offsets, geoid on or off, local approximation
-range 0 / 1 / 10 / 100, random slope and resolution factors, stacks with and without a lock
+"""Random geometries, host side: 1 - 3 layers of 1 - 3 data each (flat / two distinct tile
+stacks / maps in nine projections, geodetic maps included), offsets, geoid on or off, local
+approximation range 0 / 1 / 10 / 100, random slope and resolution factors, stacks with and without a lock
 (= through turtle_client). Whole rays and short random walks through the product's scalar
 path (the tb_core.cuh the kernels are built from, instantiated for the host) and through the
 oracle's C restatement give the reference's records byte for byte.
@@ -13,13 +13,10 @@ import numpy as np
 import pytest
 
 from oracle import harness as H
-from tests.common import Scene, geoid_map
+from tests.common import random_scene, second_stack
 from turtle_b200 import synth
 
 pytestmark = pytest.mark.skipif(not os.path.exists(H.REF), reason="oracle/_ref not built")
-
-TAGS = ["Lambert 93", "Lambert I", "Lambert II", "Lambert IIe", "Lambert III", "Lambert IV",
-        "UTM 31N", "UTM 3.0N", None]
 
 
 @pytest.fixture(scope="module")
@@ -29,54 +26,16 @@ def tiles(tmp_path_factory):
     return d
 
 
-def random_map(rng, ref):
-    tag = TAGS[rng.integers(len(TAGS))]
-    nx, ny = int(rng.integers(20, 120)), int(rng.integers(20, 120))
-    lat_c, lon_c = rng.uniform(45.3, 46.7), rng.uniform(2.3, 3.7)
-    if tag is None:
-        half = rng.uniform(0.02, 0.3)
-        x, y = (lon_c - half, lon_c + half), (lat_c - half, lat_c + half)
-    else:
-        cx, cy = ref.project(tag, [lat_c], [lon_c])
-        half = rng.uniform(1000., 20000.)
-        x, y = (cx[0] - half, cx[0] + half), (cy[0] - half, cy[0] + half)
-    values = np.resize(synth.fbm_grid(np.arange(nx) * rng.uniform(1, 8),
-                                      np.arange(ny) * rng.uniform(1, 8),
-                                      seed=int(rng.integers(1 << 30))), (ny, nx))
-    return dict(nx=nx, ny=ny, x=x, y=y, z=(0., 3000.), projection=tag,
-                values=values * rng.uniform(500, 3000))
-
-
-def random_scene(rng, ref, tiles):
-    n_maps = int(rng.integers(0, 4))
-    maps = [random_map(rng, ref) for _ in range(n_maps)]
-    geoid = -1
-    if rng.random() < 0.4:
-        maps.append(geoid_map())
-        geoid = len(maps) - 1
-    ops = []
-    for layer in range(int(rng.integers(1, 4))):
-        if layer > 0:
-            ops.append((H.ADD_LAYER, 0, 0.))
-        for _ in range(int(rng.integers(1, 4))):
-            kind = rng.integers(3)
-            offset = float(rng.uniform(-50, 50) + 400. * layer)
-            if (kind == 1) and (n_maps > 0):
-                ops.append((H.ADD_MAP, int(rng.integers(n_maps)), offset))
-            elif (kind == 0) and (rng.random() < 0.5):
-                ops.append((H.ADD_FLAT, 0, float(rng.uniform(-100, 500) + 400 * layer)))
-            else:
-                ops.append((H.ADD_STACK, 0, offset))
-    return Scene(maps=maps, stacks=[tiles], ops=ops, geoid=geoid,
-                 range=[0., 1., 10., 100.][rng.integers(4)], slope=float(rng.uniform(0.1, 1.)),
-                 resolution=float(10 ** rng.uniform(-3, 0)))
+@pytest.fixture(scope="module")
+def tiles2(tmp_path_factory):
+    return second_stack(str(tmp_path_factory.mktemp("random_geometries_2")))
 
 
 @pytest.mark.parametrize("lib", [H.PRODUCT, H.PORT], ids=["product", "restatement"])
 @pytest.mark.parametrize("seed", range(24))
-def test_host_paths_are_the_reference(tiles, seed, lib):
+def test_host_paths_are_the_reference(tiles, tiles2, seed, lib):
     rng = np.random.default_rng(1000 + seed)
-    scene = random_scene(rng, H.Driver(H.REF), tiles)
+    scene = random_scene(rng, H.Driver(H.REF), tiles, tiles2)
     locked = bool(rng.random() < 0.3)
     ref, ours = scene.oracle(H.REF, locked=locked), scene.oracle(lib, locked=locked)
     n = 300

@@ -120,15 +120,42 @@ def test_reference_client_memo_quirk(sw_stack, mixed_stack):
     assert ours.tobytes() == b.tobytes()  # the product follows the memoryless stack
 
 
-def test_geometry_limits_are_reported():
-    """More layers than the flattened geometry holds: an error, not a truncation."""
+def _small_map(projection, x=(0., 1.), y=(0., 1.)):
+    return tb.Map(2, 2, x, y, (0., 10.), projection, np.zeros((2, 2)))
+
+
+def _over_the_limit(tmp_path, over, excess):
+    """A stepper holding the limit of `over` + `excess`."""
     s = tb.Stepper(range=0.)
-    for k in range(9):
-        s.add_layer()
-        s.add_flat(float(k))
-    with pytest.raises(tb.TurtleError) as e:
-        s.step(tb.ecef_from_geodetic(45., 3., 100.))
-    assert "geometry too large" in str(e.value)
+    if over == "layers":
+        for k in range(8 + excess):
+            s.add_layer()
+            s.add_flat(float(k))
+    elif over == "metas":  # data in the layers, one flat datum
+        for k in range(24 + excess):
+            s.add_flat(float(k))
+    elif over == "data":
+        for k in range(12 + excess):
+            s.add_map(_small_map(None, (2. + 0.01 * k, 2.5), (45., 45.5)))
+    elif over == "transforms":  # distinct projections
+        for p in ("Lambert 93", "Lambert II", "UTM 31N", "UTM 32N", "Lambert IV")[:4 + excess]:
+            s.add_map(_small_map(p, (5e5, 5.1e5), (5e6, 5.1e6)))
+    else:
+        for k in range(4 + excess):
+            d = str(tmp_path / ("stack%d" % k))
+            synth.write_hgt_stack(d, 45, 2 + k, 1, 1, n=11)
+            s.add_stack(tb.Stack(d))
+    return s
+
+
+def test_geometry_limits_are_reported(tmp_path):
+    """One more layer, meta, datum, transform or stack than the flattened geometry holds
+    (8, 24, 12, 4, 4): an error, not a truncation. At the limit it is accepted."""
+    for over in ("layers", "metas", "data", "transforms", "stacks"):
+        with pytest.raises(tb.TurtleError) as e:
+            _over_the_limit(tmp_path, over, 1).step(tb.ecef_from_geodetic(45., 3., 100.))
+        assert "geometry too large" in str(e.value), over
+        _over_the_limit(tmp_path, over, 0).step(tb.ecef_from_geodetic(45., 3., 100.))
 
 
 def test_pole_and_axis_positions():

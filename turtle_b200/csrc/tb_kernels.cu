@@ -1022,6 +1022,7 @@ __global__ void __launch_bounds__(128, 5)
                 double p[3] = { 0., 0., 0. };
                 unsigned in_range = 0u; /* LLA: transforms whose reference is in range */
                 const bool sampling = !started;
+                bool cached = false;  /* the tentative sample is the published one */
                 if (sampling && (!LLA || (mode != MODE_REBUILD))) {
                         double step = 0.;
                         if (mode == MODE_TENT)
@@ -1036,8 +1037,13 @@ __global__ void __launch_bounds__(128, 5)
                                 p[1] += SF(F_DIR + 1) * step;
                                 p[2] += SF(F_DIR + 2) * step;
                         }
-                        if (LLA) { /* the range tests of this sample, ONCE; a stale Jacobian
-                                    * about to be read is rebuilt first */
+                        /* stepper.c:708-710: a step that does not move the particle (direction
+                         * 0 0 0) ends on the last sampled position, whose sample is the cached
+                         * one -- nothing is evaluated, no reference point moves */
+                        cached = (mode == MODE_TENT) && (p[0] == SF(F_LASTPOS)) &&
+                            (p[1] == SF(F_LASTPOS + 1)) && (p[2] == SF(F_LASTPOS + 2));
+                        if (LLA && !cached) { /* the range tests of this sample, ONCE; a stale
+                                               * Jacobian about to be read is rebuilt first */
                                 in_range = tb::lla_range_mask(G, V, p);
                                 const unsigned due = in_range & (unsigned)SI(I_PEND);
                                 if (due != 0u) {
@@ -1051,7 +1057,15 @@ __global__ void __launch_bounds__(128, 5)
                 if (!started) {
                         /* ---- one ECEF -> geodetic transform ------------------------- */
                         tb::Sample S;
-                        {
+                        if (cached) {
+                                S.lat = SF(F_LAT);
+                                S.lon = SF(F_LON);
+                                S.alt = SF(F_ALT);
+                                S.elev0 = SF(F_ELEV0);
+                                S.elev1 = SF(F_ELEV1);
+                                S.idx0 = SI(I_IDX0);
+                                S.idx1 = SI(I_IDX1);
+                        } else {
                                 int rb_t = 0, rb_axis = 0;
                                 bool heavy = true;
                                 if (LLA && (mode == MODE_REBUILD)) {
@@ -1672,6 +1686,7 @@ struct turtle_plan {
 
 struct turtle_states {
         struct turtle_plan * plan;
+        int device;        /* the plan's: destroying the states does not need the plan */
         size_t n;
         double * d_states; /* PS_FIELDS + G.lla_rows field rows of `stride` particles */
         size_t stride;
@@ -3149,6 +3164,7 @@ extern "C" enum turtle_return turtle_states_create(
                 return tbh::raise(FN(&turtle_states_create), TURTLE_RETURN_MEMORY_ERROR,
                     BATCH_CU, __LINE__, "could not allocate memory");
         states->plan = plan;
+        states->device = plan->device;
         states->n = n;
         states->d_states = NULL;
         states->stride = (std::max<size_t>(n, 1) + 31) / 32 * 32;
@@ -3168,7 +3184,7 @@ extern "C" enum turtle_return turtle_states_create(
 extern "C" void turtle_states_destroy(struct turtle_states ** states)
 {
         if ((states == NULL) || (*states == NULL)) return;
-        cudaSetDevice((*states)->plan->device);
+        cudaSetDevice((*states)->device);
         cudaFree((*states)->d_states);
         delete *states;
         *states = NULL;
