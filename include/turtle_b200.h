@@ -83,7 +83,7 @@ struct turtle_trace_result {
         int32_t n_changes;  /* number of steps that ended in another medium */
 };
 
-/* Kernel counters of the last trace/step call on a plan. */
+/* Kernel counters of the last trace/step/horizon call on a plan. */
 struct turtle_plan_counters {
         uint64_t rays;     /* rays or particles processed */
         uint64_t steps;    /* turtle_stepper_step equivalents */
@@ -263,6 +263,58 @@ TURTLE_API enum turtle_return turtle_stepper_trace_fields_device(struct turtle_p
     size_t n, const double * position, const double * direction,
     const struct turtle_trace_rule * rule, const struct turtle_trace_fields * fields,
     void * stream);
+
+/* ---- the horizon of a station ------------------------------------------------------------
+ * For each azimuth, the elevation that separates the rays from `position` that enter the
+ * ground from the rays that reach open sky: the contour of a muography transmission map and
+ * the edge of its open-sky calibration region. The probe at elevation e is the ray with
+ * direction turtle_ecef_from_horizontal(latitude, longitude, azimuth, e), traced under `rule`
+ * exactly as turtle_stepper_trace_batch traces it (reset stepper, same steps, same bits). It
+ * is OBSTRUCTED when one of its steps ends in a medium >= 0 other than the station's -- it
+ * stops right there -- and CLEAR when the rule stops it first (leaving the data is clear).
+ * The search runs on the device: each round traces 32 probes of one azimuth and narrows the
+ * bracket to [highest obstructed probe, next probe above it] until it is at most
+ * `tolerance` degrees wide. Every probe made above elevation[1] was clear. Over terrain that
+ * is a graph over the sphere, obstruction is monotone in elevation and the bracket holds the
+ * horizon; wherever the stepper's resolution breaks that at the sub-centimetre scale, it is
+ * still a bracket of the predicate above.
+ *
+ * The azimuths' sines and cosines are taken on the host, as for a fan; the elevations of the
+ * probes are made on the device, with the device's sine and cosine (within an ulp of the
+ * host's): the two probe directions are returned so that either end can be re-traced. The
+ * ends of a bracket that no probe established (BELOW, ABOVE, INVALID) are NaN, with
+ * medium[1] = -1 and clear_status = -1. The arguments are checked before the plan or the
+ * device is used: a tolerance <= 0 or a window that is empty, reversed or not within
+ * [-90, 90] is TURTLE_RETURN_DOMAIN_ERROR, a missing position, azimuth table or result
+ * array TURTLE_RETURN_BAD_ADDRESS. `azimuth` (degrees) is HOST memory in both variants;
+ * `results` is host memory for turtle_stepper_horizon and device memory for the
+ * asynchronous _device variant. The plan counters report the probes as rays, with their
+ * steps and samples. */
+enum turtle_horizon_status {
+        TURTLE_HORIZON_FOUND = 0,  /* elevation[0] obstructed, elevation[1] clear, width <= tolerance */
+        TURTLE_HORIZON_BELOW = 1,  /* the ray at elevation_min is already clear */
+        TURTLE_HORIZON_ABOVE = 2,  /* the ray at elevation_max is still obstructed */
+        TURTLE_HORIZON_INVALID = 3 /* station or direction not finite, or station without data */
+};
+struct turtle_horizon {            /* 96 bytes, one per azimuth */
+        double elevation[2];       /* [obstructed, clear] bracket, degrees */
+        double direction[2][3];    /* the two probe rays that were traced (ECEF, unit) */
+        double length;             /* obstructed probe: path length to its first medium change */
+        int32_t medium[2];         /* station's medium, medium the obstructed probe enters */
+        int32_t status;            /* enum turtle_horizon_status */
+        int32_t clear_status;      /* enum turtle_trace_status of the clear probe */
+        int32_t n_probes;          /* rays traced for this azimuth */
+        int32_t n_iterations;      /* loop iterations of the warp that searched it (the time
+                                    * of the search, in samples one after the other) */
+};
+TURTLE_API enum turtle_return turtle_stepper_horizon(struct turtle_plan * plan,
+    double latitude, double longitude, const double position[3], size_t n_azimuth,
+    const double * azimuth, double elevation_min, double elevation_max, double tolerance,
+    const struct turtle_trace_rule * rule, struct turtle_horizon * results);
+TURTLE_API enum turtle_return turtle_stepper_horizon_device(struct turtle_plan * plan,
+    double latitude, double longitude, const double position[3], size_t n_azimuth,
+    const double * azimuth, double elevation_min, double elevation_max, double tolerance,
+    const struct turtle_trace_rule * rule, struct turtle_horizon * results, void * stream);
 
 /* ---- the stream of medium changes along every ray (SURVEY.md section 8f, N4) --------
  * What a Monte-Carlo engine integrates over the steps -- column density, energy loss per

@@ -172,6 +172,9 @@ SIGNATURES = {
     "turtle_stepper_trace_crossings": (_I, [_P, _N, _P, _P, C.POINTER(TraceRule), _P, _P, _I]),
     "turtle_stepper_trace_crossings_device": (_I, [_P, _N, _P, _P, C.POINTER(TraceRule), _P, _P,
                                                    _I, _P]),
+    "turtle_stepper_horizon": (_I, [_P, _D, _D, _P, _N, _P, _D, _D, _D, C.POINTER(TraceRule), _P]),
+    "turtle_stepper_horizon_device": (_I, [_P, _D, _D, _P, _N, _P, _D, _D, _D,
+                                           C.POINTER(TraceRule), _P, _P]),
     # particle steps
     "turtle_states_create": (_I, [_P, _N, _PP]),
     "turtle_states_destroy": (None, [_PP]),

@@ -23,6 +23,14 @@ assert TRACE_CROSSING.itemsize == 16
 
 TRACE_ALTITUDE, TRACE_DOMAIN, TRACE_LENGTH, TRACE_STEPS, TRACE_INVALID = range(5)
 
+HORIZON_RESULT = np.dtype([
+    ("elevation", "<f8", (2,)), ("direction", "<f8", (2, 3)), ("length", "<f8"),
+    ("medium", "<i4", (2,)), ("status", "<i4"), ("clear_status", "<i4"), ("n_probes", "<i4"),
+    ("n_iterations", "<i4")])
+assert HORIZON_RESULT.itemsize == 96
+
+HORIZON_FOUND, HORIZON_BELOW, HORIZON_ABOVE, HORIZON_INVALID = range(4)
+
 
 class TurtleError(RuntimeError):
     def __init__(self, code, message):
@@ -507,6 +515,28 @@ class Plan:
         _check(lib.turtle_stepper_trace_batch_device(
             self._p, n, _ptr(position), _ptr(direction), C.byref(rule), _ptr(results),
             C.c_void_p(stream) if stream else None))
+
+    # ---- the horizon of a station (turtle_stepper_horizon) -------------------------------
+    def horizon(self, latitude, longitude, position, azimuth, rule, elevation=(-90., 90.),
+                tolerance=1e-6):
+        """Horizon bracket of the station for each azimuth (degrees): a HORIZON_RESULT array."""
+        az = _f8(azimuth).reshape(-1)
+        pos = (C.c_double * 3)(*[float(x) for x in position])
+        results = np.zeros(len(az), dtype=HORIZON_RESULT)
+        _check(lib.turtle_stepper_horizon(self._p, latitude, longitude, pos, len(az), _ptr(az),
+                                          elevation[0], elevation[1], tolerance, C.byref(rule),
+                                          _ptr(results)))
+        return results
+
+    def horizon_device(self, latitude, longitude, position, azimuth, rule, results,
+                       elevation=(-90., 90.), tolerance=1e-6, stream=None):
+        """turtle_stepper_horizon_device: `azimuth` on the host, `results` a device tensor of
+        len(azimuth) * 96 bytes; asynchronous on `stream`."""
+        az = _f8(azimuth).reshape(-1)
+        pos = (C.c_double * 3)(*[float(x) for x in position])
+        _check(lib.turtle_stepper_horizon_device(
+            self._p, latitude, longitude, pos, len(az), _ptr(az), elevation[0], elevation[1],
+            tolerance, C.byref(rule), _ptr(results), C.c_void_p(stream) if stream else None))
 
     def step(self, position, direction=None, states=None):
         """One turtle_stepper_step per particle, host arrays. Returns a dict of arrays;

@@ -795,6 +795,404 @@ __global__ void __launch_bounds__(128, MINB)
         }
 }
 
+/* ---- horizon search (turtle_stepper_horizon) -------------------------------------------- */
+
+/* Arguments of the horizon kernel. A kernel of its own rather than a variant of trace_kernel:
+ * members added to TraceArgs cost every trace kernel registers (see CompactArgs). */
+struct HorizonArgs {
+        const double2 * az; /* { sin az, cos az } per azimuth, taken on the host (fan_upload) */
+        unsigned long long n;
+        double origin[3], e[3], north[3], up[3]; /* the station and its East / North / Up frame */
+        double elevation_min, elevation_max, tolerance;
+        double altitude_min, altitude_max, length_max;
+        int max_steps;
+        turtle_horizon * results;
+        /* [0] next azimuth, [1] steps, [2] samples, [4] Jacobian columns, [6] probes */
+        unsigned long long * cursor;
+};
+
+/* Rows of the lane store that a probe uses differently from a traced ray. */
+enum { F_PROBE = F_LEN,          /* elevation of the probe, degrees */
+       I_OUTCOME = I_HASH,       /* HORIZON_OBSTRUCTED, or the trace status of a clear probe */
+       I_STATION = I_NCHANGES }; /* medium of the station: the probe's first sample */
+enum { HORIZON_OBSTRUCTED = -1, HORIZON_ROUNDS_MAX = 64 };
+
+/* K-ary search for the horizon, one azimuth per warp at a time. Each round the 32 lanes
+ * trace 32 probe rays with the sample-granular state machine of trace_kernel (the same
+ * samples, steps and bits as a traced ray: a probe is a prefix of the trace of its ray),
+ * ending a probe at its first step into a medium >= 0 other than the station's. When the
+ * round's last probe has ended, a ballot narrows the bracket to [highest obstructed probe,
+ * next probe above it]. Round 0 probes both ends of the window and 30 points between
+ * them, every later round 32 points inside the bracket (33 x narrower). Lanes whose probe
+ * has ended wait for the slowest probe of the round: the azimuth's record counts the loop
+ * iterations it took (n_iterations) so that the cost of that wait can be measured. */
+template <bool LLA, bool PROJ, int MINB, int SHAPE>
+__global__ void __launch_bounds__(128, MINB)
+    horizon_kernel(const __grid_constant__ tb::Geometry G, const HorizonArgs A)
+{
+        constexpr int NF = LLA ? N_F_LLA : N_F_BASE, NI = LLA ? N_I : N_I_BASE;
+        __shared__ LaneStoreT<NF, NI> store;
+        __shared__ turtle_horizon record[4]; /* one per warp: the azimuth being searched */
+        const unsigned tid = threadIdx.x;
+        const unsigned lane = tid & 31u;
+        const unsigned FULL = 0xffffffffu;
+        turtle_horizon & R = record[tid >> 5];
+#define SF(k) store.f[((k) < NF) ? (k) : 0][tid]
+#define SI(k) store.i[((k) < NI) ? (k) : 0][tid]
+        extern __shared__ double lla_store[];
+        const tb::LlaShared V = { lla_store + tid };
+        unsigned my_steps = 0u, my_samples = 0u, my_rebuilds = 0u, my_probes = 0u;
+        int mode = MODE_DONE;
+        bool active = false; /* warp uniform: R holds an azimuth being searched */
+        unsigned long long azimuth = 0ull;
+        int round = 0;
+        double2 sc = make_double2(0., 0.);
+
+        for (;;) {
+                if (__all_sync(FULL, mode == MODE_DONE)) {
+                        /* ---- the round is over: narrow the bracket (warp uniform) ---- */
+                        bool finished = true;
+                        if (active) {
+                                const int outcome = SI(I_OUTCOME);
+                                const unsigned obstructed =
+                                    __ballot_sync(FULL, outcome == HORIZON_OBSTRUCTED);
+                                const bool invalid =
+                                    __any_sync(FULL, outcome == TURTLE_TRACE_INVALID);
+                                const double lo = R.elevation[0], hi = R.elevation[1];
+                                __syncwarp();
+                                int status = TURTLE_HORIZON_FOUND;
+                                int low_end = -1, high_end = -1; /* lanes now holding the ends */
+                                if (invalid) {
+                                        status = TURTLE_HORIZON_INVALID;
+                                } else if (round == 0) {
+                                        if (!(obstructed & 1u)) {
+                                                status = TURTLE_HORIZON_BELOW;
+                                                high_end = 0;
+                                        } else if (obstructed >> 31) {
+                                                status = TURTLE_HORIZON_ABOVE;
+                                                low_end = 31;
+                                        } else {
+                                                low_end = 31 - __clz((int)obstructed);
+                                                high_end = low_end + 1;
+                                        }
+                                } else if (obstructed == 0u) {
+                                        high_end = 0;
+                                } else {
+                                        low_end = 31 - __clz((int)obstructed);
+                                        if (low_end < 31) high_end = low_end + 1;
+                                }
+                                if ((int)lane == low_end) {
+                                        R.elevation[0] = SF(F_PROBE);
+                                        for (int c = 0; c < 3; c++) R.direction[0][c] = SF(F_DIR + c);
+                                        R.length = SF(F_TOTAL);
+                                        R.medium[1] = SI(I_IDX0);
+                                }
+                                if ((int)lane == high_end) {
+                                        R.elevation[1] = SF(F_PROBE);
+                                        for (int c = 0; c < 3; c++) R.direction[1][c] = SF(F_DIR + c);
+                                        R.clear_status = SI(I_OUTCOME);
+                                }
+                                if (lane == 0u) {
+                                        if (round == 0) R.medium[0] = SI(I_STATION);
+                                        R.status = status;
+                                        R.n_probes += 32;
+                                }
+                                __syncwarp();
+                                round++;
+                                /* the search ends at the tolerance, or when the probes can no
+                                 * longer split the bracket (it is a few doubles wide) */
+                                finished = (status != TURTLE_HORIZON_FOUND) ||
+                                    !(R.elevation[1] - R.elevation[0] > A.tolerance) ||
+                                    ((R.elevation[0] == lo) && (R.elevation[1] == hi)) ||
+                                    (round >= HORIZON_ROUNDS_MAX);
+                                if (finished) {
+                                        /* the 96-byte record, twelve lanes side by side */
+                                        if (lane < 12u)
+                                                reinterpret_cast<unsigned long long *>(A.results + azimuth)[lane] =
+                                                    reinterpret_cast<const unsigned long long *>(&R)[lane];
+                                        __syncwarp();
+                                }
+                        }
+                        if (finished) { /* ---- next azimuth: one atomicAdd per warp ---- */
+                                unsigned long long a = 0ull;
+                                if (lane == 0u) a = atomicAdd(A.cursor, 1ull);
+                                azimuth = __shfl_sync(FULL, a, 0);
+                                if (azimuth >= A.n) break;
+                                active = true;
+                                round = 0;
+                                sc = __ldg(A.az + azimuth);
+                                if (lane == 0u) {
+                                        const double nan = __longlong_as_double(0x7ff8000000000000ll);
+                                        R.elevation[0] = R.elevation[1] = R.length = nan;
+                                        for (int c = 0; c < 3; c++)
+                                                R.direction[0][c] = R.direction[1][c] = nan;
+                                        R.medium[0] = R.medium[1] = -1;
+                                        R.status = TURTLE_HORIZON_INVALID;
+                                        R.clear_status = -1;
+                                        R.n_probes = 0;
+                                        R.n_iterations = 0;
+                                }
+                                __syncwarp();
+                        }
+                        /* ---- the probes of this round, one per lane ---- */
+                        double el;
+                        if (round == 0) {
+                                el = (lane == 31u) ? A.elevation_max :
+                                    A.elevation_min + (A.elevation_max - A.elevation_min) *
+                                                          ((double)lane / 31.);
+                        } else {
+                                const double lo = R.elevation[0], hi = R.elevation[1];
+                                el = lo + (hi - lo) * ((double)(lane + 1u) / 33.);
+                        }
+                        /* turtle_ecef_from_horizontal (ecef.c:160-178) on the host's sine and
+                         * cosine of the azimuth and the device's of the elevation */
+                        double s_el, c_el;
+                        sincos(el * M_PI / 180., &s_el, &c_el);
+                        const double r0 = c_el * sc.x, r1 = c_el * sc.y, r2 = s_el;
+                        double dir[3];
+                        for (int c = 0; c < 3; c++) {
+                                SF(F_POS + c) = A.origin[c];
+                                dir[c] = r0 * A.e[c] + r1 * A.north[c] + r2 * A.up[c];
+                                SF(F_DIR + c) = dir[c];
+                        }
+                        SF(F_PROBE) = el;
+                        SF(F_TOTAL) = 0.;
+                        SI(I_NSTEPS) = 0;
+                        SI(I_IDX0) = -1;
+                        mode = MODE_INIT;
+                        if (LLA) { /* a reset stepper (stepper.c:647-651) */
+                                SI(I_PEND) = 0;
+                                SF(F_LASTPOS) = SF(F_LASTPOS + 1) = SF(F_LASTPOS + 2) = DBL_MAX;
+                                tb::lla_reset(G, V);
+                        }
+                        const double origin[3] = { A.origin[0], A.origin[1], A.origin[2] };
+                        if (!finite3(origin) || !finite3(dir)) {
+                                SI(I_OUTCOME) = TURTLE_TRACE_INVALID;
+                                SI(I_STATION) = -1;
+                                mode = MODE_DONE;
+                        }
+                        if (lane == 0u) my_probes += 32u;
+                        continue;
+                }
+                if (lane == 0u) R.n_iterations++;
+                if (mode == MODE_DONE) continue;
+
+                /* ---- one sample per lane: as in trace_kernel ---- */
+                tb::Sample S;
+                double moved[3] = { 0., 0., 0. };
+                if (SHAPE == tb::SHAPE_STACK) {
+                        double p[3] = { SF(F_POS), SF(F_POS + 1), SF(F_POS + 2) };
+                        if (mode != MODE_INIT) {
+                                const double step = (mode == MODE_TENT) ?
+                                    SF(F_DS) : 0.5 * (SF(F_DS0) + SF(F_DS1));
+                                p[0] += SF(F_DIR) * step;
+                                p[1] += SF(F_DIR + 1) * step;
+                                p[2] += SF(F_DIR + 2) * step;
+                        }
+                        tb::sample_single_stack(tb::NodesGlobal(), G, p, S);
+                        moved[0] = p[0];
+                        moved[1] = p[1];
+                        moved[2] = p[2];
+                } else {
+                        double p[3];
+                        int rb_t = 0, rb_axis = 0;
+                        bool heavy = true;
+                        unsigned in_range = 0u;
+                        if (!LLA || (mode != MODE_REBUILD)) {
+                                double step = 0.;
+                                if (mode == MODE_TENT)
+                                        step = SF(F_DS);
+                                else if (mode == MODE_BISECT)
+                                        step = 0.5 * (SF(F_DS0) + SF(F_DS1));
+                                p[0] = SF(F_POS);
+                                p[1] = SF(F_POS + 1);
+                                p[2] = SF(F_POS + 2);
+                                if (mode != MODE_INIT) {
+                                        p[0] += SF(F_DIR) * step;
+                                        p[1] += SF(F_DIR + 1) * step;
+                                        p[2] += SF(F_DIR + 2) * step;
+                                }
+                                if (LLA) {
+                                        in_range = tb::lla_range_mask(G, V, p);
+                                        const unsigned due = in_range & (unsigned)SI(I_PEND);
+                                        if (due != 0u) {
+                                                SI(I_RESUME) = mode;
+                                                SI(I_RB_MASK) = (int)due;
+                                                SI(I_RB_AXIS) = 0;
+                                                mode = MODE_REBUILD;
+                                        }
+                                }
+                        }
+                        if (LLA && (mode == MODE_REBUILD)) {
+                                rb_t = __ffs(SI(I_RB_MASK)) - 1;
+                                rb_axis = SI(I_RB_AXIS);
+                                const int row0 = G.lla_row[rb_t];
+                                p[0] = tb::lla_at(V, row0);
+                                p[1] = tb::lla_at(V, row0 + 1);
+                                p[2] = tb::lla_at(V, row0 + 2);
+                                if (rb_axis == 0) p[0] += 10.;
+                                else if (rb_axis == 1) p[1] += 10.;
+                                else p[2] += 10.;
+                        } else if (LLA) {
+                                heavy = !((in_range >> G.lla_first) & 1u);
+                        }
+                        double pre[3] = { 0., 0., 0. };
+                        if (heavy) tb::geodetic_with_geoid(G, p, pre);
+                        if (LLA && (mode == MODE_REBUILD)) {
+                                tb::rebuild_column<PROJ>(G, V, rb_t, rb_axis, pre);
+                                my_rebuilds++;
+                                if (rb_axis == 2) {
+                                        SI(I_RB_MASK) &= ~(1 << rb_t);
+                                        SI(I_PEND) &= ~(1 << rb_t);
+                                        SI(I_RB_AXIS) = 0;
+                                        if (SI(I_RB_MASK) == 0) mode = SI(I_RESUME);
+                                } else {
+                                        SI(I_RB_AXIS) = rb_axis + 1;
+                                }
+                                continue;
+                        }
+                        double last_pos[3] = { 0., 0., 0. };
+                        unsigned stale = 0u;
+                        if (LLA) {
+                                last_pos[0] = SF(F_LASTPOS);
+                                last_pos[1] = SF(F_LASTPOS + 1);
+                                last_pos[2] = SF(F_LASTPOS + 2);
+                                stale = (unsigned)SI(I_PEND);
+                        }
+                        tb::sample_geometry<LLA, PROJ, true>(G, V, stale, last_pos,
+                            mode != MODE_BISECT, p, S, heavy ? pre : NULL, in_range);
+                        if (LLA) {
+                                SI(I_PEND) = (int)stale;
+                                if (mode != MODE_BISECT) {
+                                        SF(F_LASTPOS) = last_pos[0];
+                                        SF(F_LASTPOS + 1) = last_pos[1];
+                                        SF(F_LASTPOS + 2) = last_pos[2];
+                                }
+                        }
+                }
+                compiler_fence();
+                my_samples++;
+
+                /* ---- state update: trace_kernel's, but for the end of a probe ---- */
+                bool settle = false;
+                bool publish = false;
+                const int medium0 = SI(I_MEDIUM0);
+                double ds = SF(F_DS);
+                if (mode == MODE_INIT) {
+                        publish = true;
+                        settle = true;
+                } else if (mode == MODE_TENT) {
+                        if (SHAPE == tb::SHAPE_STACK) {
+                                SF(F_POS) = moved[0];
+                                SF(F_POS + 1) = moved[1];
+                                SF(F_POS + 2) = moved[2];
+                        } else {
+                                SF(F_POS) += SF(F_DIR) * ds;
+                                SF(F_POS + 1) += SF(F_DIR + 1) * ds;
+                                SF(F_POS + 2) += SF(F_DIR + 2) * ds;
+                        }
+                        publish = true;
+                        if (S.idx0 != medium0) {
+                                SF(F_DS0) = -ds;
+                                SF(F_DS1) = 0.;
+                                mode = MODE_BISECT;
+                                settle = !(0. - (-ds) > 1E-08);
+                        } else {
+                                settle = true;
+                        }
+                } else {
+                        double ds0 = SF(F_DS0), ds1 = SF(F_DS1);
+                        const double ds2 = 0.5 * (ds0 + ds1);
+                        if (S.idx0 == medium0) {
+                                ds0 = ds2;
+                                SF(F_DS0) = ds0;
+                        } else {
+                                ds1 = ds2;
+                                SF(F_DS1) = ds1;
+                                publish = true;
+                                if (LLA) {
+                                        SF(F_LASTPOS) = SF(F_POS) + SF(F_DIR) * ds2;
+                                        SF(F_LASTPOS + 1) = SF(F_POS + 1) + SF(F_DIR + 1) * ds2;
+                                        SF(F_LASTPOS + 2) = SF(F_POS + 2) + SF(F_DIR + 2) * ds2;
+                                }
+                        }
+                        if (!(ds1 - ds0 > 1E-08)) {
+                                ds += ds1;
+                                SF(F_POS) += SF(F_DIR) * ds1;
+                                SF(F_POS + 1) += SF(F_DIR + 1) * ds1;
+                                SF(F_POS + 2) += SF(F_DIR + 2) * ds1;
+                                settle = true;
+                        }
+                }
+                if (publish) {
+                        SF(F_ALT) = S.alt;
+                        SF(F_ELEV0) = S.elev0;
+                        SF(F_ELEV1) = S.elev1;
+                        SI(I_IDX0) = S.idx0;
+                        SI(I_IDX1) = S.idx1;
+                }
+                if (!settle) continue;
+
+                tb::Sample last;
+                last.lat = last.lon = 0.;
+                last.alt = publish ? S.alt : SF(F_ALT);
+                last.elev0 = publish ? S.elev0 : SF(F_ELEV0);
+                last.elev1 = publish ? S.elev1 : SF(F_ELEV1);
+                last.idx0 = publish ? S.idx0 : SI(I_IDX0);
+                last.idx1 = publish ? S.idx1 : SI(I_IDX1);
+                double total = SF(F_TOTAL);
+                int n_steps = SI(I_NSTEPS);
+                int outcome = TURTLE_TRACE_INVALID + 1; /* none yet */
+                if (mode == MODE_INIT) {
+                        SI(I_STATION) = last.idx0;
+                        if (last.idx0 < 0) outcome = TURTLE_TRACE_INVALID; /* station without data */
+                } else {
+                        total += ds;
+                        SF(F_TOTAL) = total;
+                        n_steps++;
+                        SI(I_NSTEPS) = n_steps;
+                        my_steps++;
+                        /* the only new stop condition: the first step into another medium
+                         * that is not "outside of the data" (that one ends the trace) */
+                        if ((last.idx0 != medium0) && (last.idx0 >= 0))
+                                outcome = HORIZON_OBSTRUCTED;
+                }
+                if (outcome > TURTLE_TRACE_INVALID) {
+                        if (last.idx0 < 0)
+                                outcome = TURTLE_TRACE_DOMAIN;
+                        else if (!(last.alt < A.altitude_max) || !(last.alt > A.altitude_min))
+                                outcome = TURTLE_TRACE_ALTITUDE;
+                        else if (total >= A.length_max)
+                                outcome = TURTLE_TRACE_LENGTH;
+                        else if (n_steps >= A.max_steps)
+                                outcome = TURTLE_TRACE_STEPS;
+                }
+                if (outcome <= TURTLE_TRACE_INVALID) {
+                        SI(I_OUTCOME) = outcome;
+                        mode = MODE_DONE;
+                } else {
+                        SI(I_MEDIUM0) = last.idx0;
+                        SF(F_DS) = tb::step_length(G, last);
+                        mode = MODE_TENT;
+                }
+        }
+#undef SF
+#undef SI
+
+        unsigned long long steps64 = my_steps, samples64 = my_samples, rebuilds64 = my_rebuilds;
+        for (int o = 16; o > 0; o >>= 1) {
+                steps64 += __shfl_down_sync(FULL, steps64, o);
+                samples64 += __shfl_down_sync(FULL, samples64, o);
+                if (LLA) rebuilds64 += __shfl_down_sync(FULL, rebuilds64, o);
+        }
+        if (lane == 0u) {
+                atomicAdd(A.cursor + 1, steps64);
+                atomicAdd(A.cursor + 2, samples64);
+                if (LLA) atomicAdd(A.cursor + 4, rebuilds64);
+                atomicAdd(A.cursor + 6, (unsigned long long)my_probes);
+        }
+}
+
 /* Longest-expected-first scheduling: the number of steps of a ray grows as it runs
  * closer to the horizontal (it stays near the ground), and the kernel time is bounded
  * below by the LATEST-starting long ray. Key = |sin(elevation)| w.r.t. the geocentric
@@ -2566,6 +2964,7 @@ extern "C" void turtle_plan_counters_sync(struct turtle_plan * plan)
                 plan->counters.samples = c[2];
                 plan->counters.rebuilds = c[4];
                 plan->counters.window_hits = c[5];
+                if (c[6] != 0ull) plan->counters.rays = c[6]; /* the probes of a horizon search */
         }
 }
 
@@ -3077,6 +3476,136 @@ extern "C" enum turtle_return turtle_stepper_trace_fields_device(struct turtle_p
         const DeviceIo io = { position, direction, NULL, NULL, fields };
         CUDA_TRY(fn, launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
                          (cudaStream_t)stream));
+        return TURTLE_RETURN_SUCCESS;
+}
+
+/* ---- the horizon of a station ---------------------------------------------------------- */
+
+/* Arguments first (no plan, no device needed), then the device, then the plan. */
+static enum turtle_return check_horizon(turtle_function_t * fn, const struct turtle_plan * plan,
+    const double * position, size_t n_azimuth, const double * azimuth, double elevation_min,
+    double elevation_max, double tolerance, const struct turtle_trace_rule * rule,
+    const struct turtle_horizon * results)
+{
+        if ((position == NULL) || ((n_azimuth > 0) && ((azimuth == NULL) || (results == NULL))))
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
+                    "missing station position, azimuths or results");
+        if (!(tolerance > 0.))
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "invalid tolerance %g (must be > 0)", tolerance);
+        if (!(elevation_min >= -90.) || !(elevation_max <= 90.) || !(elevation_min < elevation_max))
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "invalid elevation window [%g, %g] (must be an interval of [-90, 90])",
+                    elevation_min, elevation_max);
+        enum turtle_return rc = check_rule(fn, rule);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n_azimuth == 0)) return rc;
+        rc = require_device(fn, (plan != NULL) ? plan->device : 0);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        if (plan == NULL)
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__, "missing plan");
+        return TURTLE_RETURN_SUCCESS;
+}
+
+/* Queue the search on `stream`: azimuth table (fan_upload), counters, kernel. */
+static cudaError_t launch_horizon(struct turtle_plan * plan, double latitude, double longitude,
+    const double position[3], size_t n_azimuth, const double * azimuth, double elevation_min,
+    double elevation_max, double tolerance, const struct turtle_trace_rule * rule,
+    struct turtle_horizon * results, cudaStream_t stream)
+{
+        memset(&plan->counters, 0x0, sizeof(plan->counters));
+        const int slot = next_device_slot(plan);
+        unsigned long long * d_counters = plan->d_counters + CTR * slot;
+        struct turtle_fan fan;
+        memset(&fan, 0x0, sizeof fan);
+        fan.latitude = latitude;
+        fan.longitude = longitude;
+        for (int c = 0; c < 3; c++) fan.position[c] = position[c];
+        fan.n_azimuth = n_azimuth;
+        fan.azimuth = azimuth;
+        FanTables T;
+        cudaError_t err = fan_upload(plan, slot, &fan, 1, 0, stream, &T);
+        if (err == cudaSuccess)
+                err = cudaMemsetAsync(d_counters, 0x0, CTR * sizeof(unsigned long long), stream);
+        if (err != cudaSuccess) return err;
+        HorizonArgs A;
+        memset(&A, 0x0, sizeof A);
+        A.az = T.az;
+        A.n = n_azimuth;
+        for (int c = 0; c < 3; c++) {
+                A.origin[c] = T.origin[c];
+                A.e[c] = T.e[c];
+                A.north[c] = T.n[c];
+                A.up[c] = T.u[c];
+        }
+        A.elevation_min = elevation_min;
+        A.elevation_max = elevation_max;
+        A.tolerance = tolerance;
+        A.altitude_min = rule->altitude_min;
+        A.altitude_max = rule->altitude_max;
+        A.length_max = rule->length_max;
+        A.max_steps = rule->max_steps;
+        A.results = results;
+        A.cursor = d_counters;
+        /* one azimuth per warp: the grid of the trace kernels, without the warps that would
+         * find no azimuth */
+        int blocks, threads;
+        const int per_sm = trace_grid(plan, 0, &blocks, &threads);
+        const size_t warps = (size_t)threads / 32;
+        blocks = (int)std::min<size_t>((size_t)plan->sm_count * per_sm, (n_azimuth + warps - 1) / warps);
+        const bool lla = plan->G.range > 0.;
+        bool proj = false;
+        for (int t = 0; t < plan->G.n_transforms; t++)
+                if (plan->G.transforms[t].type != tb::PROJ_GEODETIC) proj = true;
+        const bool stack_shape = plan->specialise && (tb::geometry_shape(plan->G) == tb::SHAPE_STACK);
+        void (*kernel)(const tb::Geometry, const HorizonArgs) =
+            stack_shape ? horizon_kernel<false, false, 6, tb::SHAPE_STACK> :
+            (lla && proj) ? horizon_kernel<true, true, 4, tb::SHAPE_GENERIC> :
+            lla ? horizon_kernel<true, false, 4, tb::SHAPE_GENERIC> :
+            proj ? horizon_kernel<false, true, 6, tb::SHAPE_GENERIC> :
+                   horizon_kernel<false, false, 6, tb::SHAPE_GENERIC>;
+        const size_t dynamic = lla ? lla_bytes(plan) : 0;
+        if (dynamic > 0)
+                cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dynamic);
+        kernel<<<blocks, threads, dynamic, stream>>>(plan->G, A);
+        plan->counters.launches++;
+        return cudaGetLastError();
+}
+
+extern "C" enum turtle_return turtle_stepper_horizon_device(struct turtle_plan * plan,
+    double latitude, double longitude, const double position[3], size_t n_azimuth,
+    const double * azimuth, double elevation_min, double elevation_max, double tolerance,
+    const struct turtle_trace_rule * rule, struct turtle_horizon * results, void * stream)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_horizon_device);
+        enum turtle_return rc = check_horizon(fn, plan, position, n_azimuth, azimuth,
+            elevation_min, elevation_max, tolerance, rule, results);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n_azimuth == 0)) return rc;
+        CUDA_TRY(fn, cudaSetDevice(plan->device));
+        CUDA_TRY(fn, launch_horizon(plan, latitude, longitude, position, n_azimuth, azimuth,
+                         elevation_min, elevation_max, tolerance, rule, results,
+                         (cudaStream_t)stream));
+        return TURTLE_RETURN_SUCCESS;
+}
+
+extern "C" enum turtle_return turtle_stepper_horizon(struct turtle_plan * plan,
+    double latitude, double longitude, const double position[3], size_t n_azimuth,
+    const double * azimuth, double elevation_min, double elevation_max, double tolerance,
+    const struct turtle_trace_rule * rule, struct turtle_horizon * results)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_horizon);
+        enum turtle_return rc = check_horizon(fn, plan, position, n_azimuth, azimuth,
+            elevation_min, elevation_max, tolerance, rule, results);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n_azimuth == 0)) return rc;
+        CUDA_TRY(fn, cudaSetDevice(plan->device));
+        struct turtle_horizon * d_results = NULL;
+        const size_t bytes = n_azimuth * sizeof(*d_results);
+        CUDA_TRY(fn, cudaMalloc((void **)&d_results, bytes));
+        cudaError_t err = launch_horizon(plan, latitude, longitude, position, n_azimuth, azimuth,
+            elevation_min, elevation_max, tolerance, rule, d_results, NULL);
+        if (err == cudaSuccess) err = cudaMemcpy(results, d_results, bytes, cudaMemcpyDeviceToHost);
+        cudaFree(d_results);
+        CUDA_TRY(fn, err);
+        turtle_plan_counters_sync(plan);
         return TURTLE_RETURN_SUCCESS;
 }
 
@@ -4139,6 +4668,8 @@ extern "C" const char * tb_batch_function_name(turtle_function_t * caller)
         NAME(turtle_stack_elevation_batch_device);
         NAME(turtle_stepper_trace_crossings);
         NAME(turtle_stepper_trace_crossings_device);
+        NAME(turtle_stepper_horizon);
+        NAME(turtle_stepper_horizon_device);
         NAME(turtle_b200_peer_alloc);
         NAME(turtle_b200_peer_free);
         NAME(turtle_b200_peer_export);
