@@ -391,7 +391,13 @@ TURTLE_API enum turtle_return turtle_stepper_position_batch(
     double * position, int * data_index);
 
 /* ---- frame transforms (ref: src/turtle/ecef.c:41-55,63-130,160-178) ---------
- * Run on the current CUDA device. Output pointers of to_geodetic may be NULL. */
+ * Run on the current CUDA device. Output pointers of to_geodetic may be NULL.
+ * to_geodetic: the altitude has the bits of turtle_ecef_to_geodetic, latitude and
+ * longitude are within 4 ulp of it, for points at least 50 km from the centre of the
+ * Earth. Closer, the arguments of the arcsine in Olson's method leave the range its
+ * device polynomial is fitted for and the latitude is not bounded (the reference's own
+ * method returns NaN below about 40 km). Where x or y is denormal or infinite the
+ * longitude is NaN (the device arctangent divides through a reciprocal). */
 TURTLE_API enum turtle_return turtle_ecef_to_geodetic_batch(size_t n,
     const double * ecef, double * latitude, double * longitude,
     double * altitude);

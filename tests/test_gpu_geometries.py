@@ -32,7 +32,7 @@ from tests.common import Scene, geoid_map, lambert_map, random_scene, second_sta
 from tests.test_crossings import _consistent
 from tests.test_fan import FIELDS, columns, fan_rays
 from tests.test_gpu_trace import check, noise_floor
-from tests.test_scenes_extra import mixed_stack, sw_stack  # noqa: F401  (fixtures)
+from tests.test_scenes_extra import mixed_stack, sw_stack, utm_south_map  # noqa: F401
 from turtle_b200 import synth
 
 pytestmark = pytest.mark.gpu
@@ -46,7 +46,8 @@ FRANCE = (44.9, 47.1, 1.9, 4.1)
 CHILE = (-35.1, -32.9, -72.1, -69.9)
 RANDOM_SEEDS = range(24)
 NAMED = ["two_projections_r0", "three_projections_lla", "shared_projection_union",
-         "map_first", "geodetic_map_first", "shared_map", "stacks_x4", "at_the_limits"]
+         "map_first", "geodetic_map_first", "shared_map", "stacks_x4", "at_the_limits",
+         "antimeridian_r0", "antimeridian_lla", "high_latitude", "polar_cap", "south_west_lla"]
 RULE = dict(altitude_max=6000., length_max=3e4, max_steps=5000)
 
 
@@ -55,12 +56,50 @@ def tiles2(tmp_path_factory):
     return second_stack(str(tmp_path_factory.mktemp("second_stack")))
 
 
+@pytest.fixture(scope="module")
+def globe_stacks(tmp_path_factory):
+    """Stacks away from France: `seam` (write_seam_stack) and `arctic`, 2 x 2 tiles at
+    N78 - N79, E015 - E016 (1/1200 deg cells of about 8 m in longitude)."""
+    seam = write_seam_stack(str(tmp_path_factory.mktemp("seam_stack")))
+    arctic = str(tmp_path_factory.mktemp("arctic_stack"))
+    synth.write_hgt_stack(arctic, 78, 15, 2, 2, n=1201)
+    return dict(seam=seam, arctic=arctic)
+
+
+def write_seam_stack(directory):
+    """2 x 2 tiles S01E179, S01W180, N00E179, N00W180 around the antimeridian on the equator:
+    a tile table of 360 columns, 358 of them empty. The terrain is continuous across the
+    seam, as in a real elevation model: the W180 tiles continue the node lattice of the E179
+    ones. (With a step in the terrain exactly on the seam, a ray crossing it under the higher
+    ground changes medium there, its bisection converges onto longitude 180, and which side a
+    sample lands on hinges on the last ulp of its longitude, 3 nm: a grazing ray of the parity
+    protocol in every such crossing.)"""
+    os.makedirs(directory, exist_ok=True)
+    for lat in (-1, 0):
+        for lon, origin in ((179, 179), (-180, -181)):
+            nodes = synth.tile_nodes(lat, lon, -1, origin, 1201)
+            name = synth.hgt_name(lat, lon)[:-4] + ".SRTMGL3.hgt"
+            nodes[::-1].astype(">i2").tofile(os.path.join(directory, name))
+    return directory
+
+
+def wrap(lon):
+    """Longitudes in (-180, 180]."""
+    lon = np.asarray(lon, dtype=np.float64)
+    return np.where(lon > 180., lon - 360., np.where(lon <= -180., lon + 360., lon))
+
+
+def dlon(a, b):
+    """|a - b| modulo 360 (degrees): -180 and 180 are the same meridian."""
+    return np.abs((np.asarray(a) - np.asarray(b) + 180.) % 360. - 180.)
+
+
 class Case:
-    """A scene, where its rays start (lat0, lat1, lon0, lon1 boxes; `ground`: bands where a
-    third of the rays and walkers start just over the ground of layer 0) and which of its
-    stacks the oracle may share between threads (a lock makes the reference go through
-    turtle_client, whose memo of a missing tile is history dependent for negative
-    coordinates: see test_reference_client_memo_quirk)."""
+    """A scene, where its rays start (lat0, lat1, lon0, lon1 boxes, where lon0 > lon1 is a box
+    across the antimeridian; `ground`: bands where a third of the rays and walkers start just
+    over the ground of layer 0) and which of its stacks the oracle may share between threads
+    (a lock makes the reference go through turtle_client, whose memo of a missing tile is
+    history dependent for negative coordinates: see test_reference_client_memo_quirk)."""
 
     def __init__(self, scene, boxes=(FRANCE,), ground=(), locked=True, center=(45.6, 2.7)):
         self.scene, self.boxes, self.ground = scene, list(boxes), list(ground)
@@ -75,8 +114,83 @@ def _map_at(ora, tag, lat, lon, half, n, seed):
                 z=(0., 3000.), projection=tag, values=vals)
 
 
-def named_case(name, ora, small, tiles2, mixed, sw):
+def seam_maps(ora):
+    """The maps of the antimeridian scenes: a UTM 1N map wholly west of its zone (x 140 -
+    166.02 km, y 40 - 70 km: 179.77 E to 8 - 25 m west of 180, whose unwrapped inverse
+    projection lies at -180.23 - -180.0001), a UTM 60N map across 180 deg and a geodetic
+    map whose east edge is the meridian 180 itself."""
+    def fbm(n, seed):
+        return synth.fbm_grid(np.arange(n) * 4., np.arange(n) * 4., seed=seed) * 2500.
+    utm1 = dict(nx=131, ny=151, x=(140e3, 166020.), y=(40e3, 70e3), z=(0., 3000.),
+                projection="UTM 1N", values=np.resize(fbm(151, 31), (151, 131)))
+    cx, cy = ora.project("UTM 60N", [-0.3], [180.])
+    utm60 = dict(nx=161, ny=161, x=(cx[0] - 16e3, cx[0] + 16e3), y=(cy[0] - 16e3, cy[0] + 16e3),
+                 z=(0., 3000.), projection="UTM 60N", values=fbm(161, 32))
+    geo = dict(nx=121, ny=61, x=(179.4, 180.), y=(-0.9, -0.6), z=(0., 3000.), projection=None,
+               values=np.resize(fbm(121, 33), (61, 121)))
+    return [utm1, utm60, geo]
+
+
+def seam_ground(ora, utm1):
+    """Ground bands within metres of the antimeridian (1.5E-04 deg = 17 m) and of the
+    borders of the UTM 1N map."""
+    bands = [(-0.9, 0.9, 180. - 1.5e-4, -180. + 1.5e-4)]
+    (la0, la1), (lo0, lo1) = ora.project("UTM 1N", utm1["x"], utm1["y"], inverse=True)
+    lo0, lo1 = wrap(lo0), wrap(lo1)
+    bands += [(la0 - 2e-4, la0 + 2e-4, lo0, lo1), (la1 - 2e-4, la1 + 2e-4, lo0, lo1),
+              (la0, la1, lo0 - 2e-4, lo0 + 2e-4), (la0, la1, lo1 - 2e-4, lo1 + 2e-4)]
+    return bands
+
+
+def named_case(name, ora, small, tiles2, mixed, sw, globe):
     A, F, S, L = H.ADD_MAP, H.ADD_FLAT, H.ADD_STACK, H.ADD_LAYER
+    if name in ("antimeridian_r0", "antimeridian_lla"):
+        # layer 0 evaluates the UTM 60N map (across 180: no box), the UTM 1N map, the
+        # geodetic map, the stack (360 columns, over the equator) and the flat; layer 1 the
+        # UTM 1N map again. At range 0 every sample over the UTM 1N map has a longitude near
+        # +179.9 and must not be culled by a box taken at -180.1. At range 10 the references
+        # of the UTM 60N transform, evaluated first, fall within 10 m of the seam, and the
+        # longitude linearised from them is off by up to 360 deg for samples over the UTM 1N
+        # map, whose union box comes within metres of 180: that box must not be used
+        maps = seam_maps(ora)
+        sc = Scene(maps=maps, stacks=[globe["seam"]],
+                   ops=[(F, 0, -300.), (S, 0, 0.), (A, 2, 30.), (A, 0, 0.), (A, 1, 10.),
+                        (L, 0, 0.), (A, 0, 700.)],
+                   range=0. if name == "antimeridian_r0" else 10.)
+        return Case(sc, boxes=[(-0.95, 0.95, 179.1, -179.1), (0.35, 0.65, 179.75, 179.95)],
+                    ground=seam_ground(ora, maps[0]), locked=False, center=(0.5, 179.85))
+    if name == "high_latitude":
+        # UTM 33N far north: the grid is turned by up to 15 deg (convergence), the second map
+        # reaches 84 N, the union box of the transform is widened by 1 / cos(lat)
+        maps = [_map_at(ora, "UTM 33N", 78.9, 15.9, 15000., 151, 34),
+                _map_at(ora, "UTM 33N", 83.78, 15.0, 25000., 151, 35), geoid_map()]
+        sc = Scene(maps=maps, stacks=[globe["arctic"]],
+                   ops=[(F, 0, -200.), (S, 0, 0.), (A, 0, 20.), (L, 0, 0.), (A, 1, 300.)],
+                   geoid=2, range=1.)
+        (la0, la1), (lo0, lo1) = ora.project("UTM 33N", maps[0]["x"], maps[0]["y"], inverse=True)
+        ground = [(la0 - 2e-4, la0 + 2e-4, lo0, lo1), (la0, la1, lo1 - 5e-4, lo1 + 5e-4)]
+        return Case(sc, boxes=[(77.9, 80.1, 14.9, 17.1), (83.5, 84.05, 14.0, 16.0)],
+                    ground=ground, center=(78.9, 15.9))
+    if name == "polar_cap":
+        # a geodetic map over the whole cap: rays from within 55 m of the axis cross it, their
+        # longitude flips by 180 deg, and the Jacobian of the longitude diverges there
+        n = 361
+        geo = dict(nx=n, ny=41, x=(-180., 180.), y=(89., 90.), z=(0., 3000.), projection=None,
+                   values=np.resize(synth.fbm_grid(np.arange(n) * 3., np.arange(41) * 3.,
+                                                   seed=36), (41, n)) * 1500.)
+        sc = Scene(maps=[geo], ops=[(F, 0, -50.), (A, 0, 0.)], range=100.)
+        return Case(sc, boxes=[(89.5, 90., -180., 180.)], ground=[(89.9995, 90., -180., 180.)],
+                    center=(89.9999, 30.))
+    if name == "south_west_lla":
+        # the Chilean scene of test_scenes_extra (UTM 19S map over a stack in negative
+        # coordinates) under the local approximation
+        m = utm_south_map()
+        sc = Scene(maps=[m], stacks=[sw], ops=[(S, 0, 0.), (A, 0, 0.), (L, 0, 0.), (S, 0, 800.)],
+                   range=10.)
+        (la0, la1), (lo0, lo1) = ora.project("UTM 19S", m["x"], m["y"], inverse=True)
+        return Case(sc, boxes=[CHILE, (la0 - 0.01, la1 + 0.01, lo0 - 0.01, lo1 + 0.01)],
+                    ground=[(la0 - 2e-4, la0 + 2e-4, lo0, lo1)], locked=False,
+                    center=(0.5 * (la0 + la1), 0.5 * (lo0 + lo1)))
     if name == "two_projections_r0":
         # layer 0 evaluates the UTM 30N map first, then the Lambert map, then the stack. Far
         # from its central meridian the UTM grid is turned by ~4 degrees, so its geodetic
@@ -202,7 +316,7 @@ def _draw(boxes, n, rng, h=(-300., 4000.)):
     la, lo = np.empty(n), np.empty(n)
     for b, idx in zip(boxes, parts):
         la[idx] = rng.uniform(b[0], b[1], len(idx))
-        lo[idx] = rng.uniform(b[2], b[3], len(idx))
+        lo[idx] = wrap(rng.uniform(b[2], b[3] + (360. if b[3] < b[2] else 0.), len(idx)))
     return la, lo, rng.uniform(h[0], h[1], n)
 
 
@@ -219,7 +333,7 @@ def _origins(case, n, rng):
 
 
 @pytest.fixture(scope="module", params=["random_%02d" % s for s in RANDOM_SEEDS] + NAMED)
-def case(request, small_stack, tiles2, mixed_stack, sw_stack):  # noqa: F811
+def case(request, small_stack, tiles2, mixed_stack, sw_stack, globe_stacks):  # noqa: F811
     """One scene: its oracle, its plan, N_RAYS random rays and the oracle's records and
     crossings of them, shared by the tests of the scene."""
     ora0 = H.Driver(H.best_oracle())
@@ -228,7 +342,7 @@ def case(request, small_stack, tiles2, mixed_stack, sw_stack):  # noqa: F811
         seed = int(name[-2:])
         c = Case(random_scene(np.random.default_rng(5000 + seed), ora0, small_stack, tiles2))
     else:
-        c = named_case(name, ora0, small_stack, tiles2, mixed_stack, sw_stack)
+        c = named_case(name, ora0, small_stack, tiles2, mixed_stack, sw_stack, globe_stacks)
     c.name = name
     c.ora = c.scene.oracle(locked=c.locked)
     c.threads = os.cpu_count() if np.all(c.locked) else 1
@@ -285,6 +399,8 @@ def test_samples_vs_oracle(case):
     assert np.abs(got["step"] - want["step"])[same].max() < 1e-6
     assert np.abs(got["altitude"] - want["altitude"])[same].max() < 1e-6
     assert ulp_distance(got["latitude"], want["latitude"])[same].max() <= 64
+    # atan2 of a y of either sign of zero is +-180: the same meridian
+    assert dlon(got["longitude"], want["longitude"])[same].max() <= 1e-11
     e_w, e_g = want["elevation"][same], got["elevation"][same]
     assert np.array_equal(np.abs(e_w) > 1e300, np.abs(e_g) > 1e300)  # +-DBL_MAX sentinels
     small = np.abs(e_w) < 1e300

@@ -1220,7 +1220,13 @@ enum turtle_return tbh::stepper_flatten(struct turtle_stepper * s,
 /* Geodetic footprint of a projected map (tb::DataDesc::box): the border of the map is
  * walked node by node through the inverse projection; the box is widened by 1E-06 deg
  * (0.1 m) plus a bound on the bulge of an edge between two nodes, and dropped when the
- * footprint wraps in longitude or is not finite. */
+ * footprint wraps in longitude, reaches +-180 deg or +-89 deg, or is not finite.
+ *
+ * The inverse UTM projection returns lon0 + atan2(...), which is not wrapped: a UTM 1N
+ * map west of its zone unprojects to about -180.2 deg while its samples, from atan2, lie
+ * at +179.8 deg and the projection, periodic in longitude, still sees them on the map. So
+ * longitudes are brought into the (-180, 180] range of the samples first, and a footprint
+ * that straddles or touches the antimeridian is not boxed at all. */
 static void map_geodetic_box(const struct turtle_map * m, const tb::ProjDesc & P, tb::DataDesc & d)
 {
         d.boxed = 0;
@@ -1236,6 +1242,7 @@ static void map_geodetic_box(const struct turtle_map * m, const tb::ProjDesc & P
                         double la, lo;
                         tb::unproject(P, x, y, la, lo);
                         if (!isfinite(la) || !isfinite(lo)) return;
+                        lo = remainder(lo, 360.); /* exact, in [-180, 180] */
                         la0 = std::min(la0, la);
                         la1 = std::max(la1, la);
                         lo0 = std::min(lo0, lo);
@@ -1257,7 +1264,10 @@ static void map_geodetic_box(const struct turtle_map * m, const tb::ProjDesc & P
         d.box[1] = la1 + margin;
         d.box[2] = lo0 - margin;
         d.box[3] = lo1 + margin;
-        d.boxed = 1;
+        /* a footprint across the antimeridian has border nodes on both sides of it and
+         * spans more than 90 deg after the wrap (dropped above); one that comes within
+         * the margin of it may still bulge across */
+        d.boxed = (d.box[2] > -180.) && (d.box[3] < 180.);
 }
 
 /* Does the closed footprint of a tile meet the region of a residency plan? */
@@ -1475,14 +1485,26 @@ enum turtle_return tbh::flatten_into(struct turtle_stepper * s, tb_flat_geometry
                 }
                 /* (a sample in range is within r sqrt 3 of its reference point) */
                 const double r = (G.range > 0.) ? G.range : 0.;
-                const double slack = 4. * (r * r / TB_WGS84_B + 2. * r + 1E-03) / TB_WGS84_B * 180. /
-                    M_PI / std::max(0.02,
+                const double rad = 180. / M_PI / TB_WGS84_B;
+                const double slack = 4. * (r * r / TB_WGS84_B + 2. * r + 1E-03) * rad /
+                    std::max(cos(89. * M_PI / 180.),
                         cos(std::max(fabs(G.tbox[t][0]), fabs(G.tbox[t][1])) * M_PI / 180.));
-                G.tboxed[t] = any && all && isfinite(slack);
                 G.tbox[t][0] -= slack;
                 G.tbox[t][1] += slack;
                 G.tbox[t][2] -= slack;
                 G.tbox[t][3] += slack;
+                /* Near the antimeridian the longitude a sample is culled with cannot be
+                 * trusted: it may be linearised from a reference point whose finite
+                 * difference Jacobian (10 m steps, stepper.c:144-162) jumps by 360 deg
+                 * across the seam. A box that comes within the slack plus those 10 m of
+                 * +-180 is dropped. So is one that reaches +-89 deg, the latitude up to
+                 * which the slack above is conservative. */
+                const double seam = slack + 40. * rad /
+                    std::max(cos(89. * M_PI / 180.),
+                        cos(std::max(fabs(G.tbox[t][0]), fabs(G.tbox[t][1])) * M_PI / 180.));
+                G.tboxed[t] = any && all && isfinite(slack) &&
+                    (G.tbox[t][2] - seam > -180.) && (G.tbox[t][3] + seam < 180.) &&
+                    (G.tbox[t][0] > -89.) && (G.tbox[t][1] < 89.);
         }
         G.host_stack = load_tiles ? &host_stack_lookup : NULL;
         G.host_context = load_tiles ? (void *)s : NULL;
