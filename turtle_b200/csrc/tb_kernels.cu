@@ -2020,6 +2020,8 @@ namespace {
 const int N_SLOTS = 3;              /* host-pointer pipeline depth */
 const int DEV_SLOTS = 8;            /* device-pointer calls that may be in flight per plan */
 const int ALL_SLOTS = N_SLOTS + DEV_SLOTS;
+const int HOST_SLICES = DEV_SLOTS;  /* counter blocks of the slices of a host-pointer fan, after
+                                     * the ALL_SLOTS blocks */
 const int CTR = 8;                  /* counters per launch: [0] queue cursor, [1] steps,
                                      * [2] samples, [3] stream time-out, [4] Jacobian columns */
 const size_t CHUNK_RAYS = 1u << 20; /* rays per pipeline chunk (one kernel per chunk) */
@@ -2040,8 +2042,14 @@ struct turtle_plan {
         size_t bytes;
         turtle_residency_report report;
         std::vector<struct turtle_stack *> pinned;
-        unsigned long long * d_counters; /* ALL_SLOTS blocks of CTR counters */
+        unsigned long long * d_counters; /* ALL_SLOTS + HOST_SLICES blocks of CTR counters */
         int dev_slot;                    /* block of the latest device-pointer call */
+        /* per device slot: recorded on the caller's stream after the last operation of the
+         * call that holds the slot (NULL until the slot is first used), and the number of
+         * the device-pointer call that took it */
+        cudaEvent_t slot_done[DEV_SLOTS];
+        unsigned long long slot_call[DEV_SLOTS];
+        unsigned long long dev_calls;
         turtle_plan_counters counters;
         /* ray scheduling (turtle_plan_schedule_set) */
         int schedule;
@@ -2231,6 +2239,11 @@ static enum turtle_return freeze_plan(turtle_function_t * fn, struct turtle_step
         plan->d_tiles = NULL;
         plan->d_counters = NULL;
         plan->dev_slot = N_SLOTS;
+        for (int s = 0; s < DEV_SLOTS; s++) {
+                plan->slot_done[s] = NULL;
+                plan->slot_call[s] = 0;
+        }
+        plan->dev_calls = 0;
         plan->schedule = 0;
         plan->specialise = 1;
         plan->pipeline_mode = 0;
@@ -2354,7 +2367,7 @@ static enum turtle_return freeze_plan(turtle_function_t * fn, struct turtle_step
                     cudaMemcpyHostToDevice);
         if (err == cudaSuccess)
                 err = cudaMalloc((void **)&plan->d_counters,
-                    ALL_SLOTS * CTR * sizeof(unsigned long long));
+                    (ALL_SLOTS + HOST_SLICES) * CTR * sizeof(unsigned long long));
         if (err != cudaSuccess) {
                 turtle_plan_destroy(&plan);
                 return tbh::raise(fn, TURTLE_RETURN_LIBRARY_ERROR, BATCH_CU, __LINE__,
@@ -2473,6 +2486,8 @@ extern "C" void turtle_plan_destroy(struct turtle_plan ** plan_)
                 cudaFree(plan->d_sched[s]);
                 cudaFree(plan->d_sched_tmp[s]);
         }
+        for (int s = 0; s < DEV_SLOTS; s++)
+                if (plan->slot_done[s] != NULL) cudaEventDestroy(plan->slot_done[s]);
         cudaFree(plan->d_all_in);
         cudaFree(plan->d_all_out);
         cudaFree(plan->d_field_pool);
@@ -2715,11 +2730,54 @@ static void trace_start(const struct turtle_plan * plan, int per_sm, int blocks,
 
 /* Device-pointer calls are asynchronous: up to DEV_SLOTS of them may be in flight on a
  * plan (on different streams -- how a caller backfills the tail of one batch with the
- * head of the next); each takes the next counter block / schedule buffers of the ring. */
-static int next_device_slot(struct turtle_plan * plan)
+ * head of the next). Each takes a slot of the ring -- counter block (the queue cursor of its
+ * kernel), schedule buffers, fan / azimuth tables -- that no call in flight holds: the first
+ * one after the latest slot whose event (release_device_slot) has completed, so that calls
+ * made one after the other go round the ring. Calls may complete in any order (a long call
+ * on one stream, short ones on another): when every slot is held, the host waits for the
+ * call that took its slot first. The slot is *slot on return, and the caller must release
+ * it on its stream once it has queued the call's last operation, also when that failed. */
+static cudaError_t next_device_slot(struct turtle_plan * plan, int * slot)
 {
-        plan->dev_slot = N_SLOTS + (plan->dev_slot - N_SLOTS + 1) % DEV_SLOTS;
-        return plan->dev_slot;
+        int s = -1, oldest = -1;
+        for (int k = 1; (k <= DEV_SLOTS) && (s < 0); k++) {
+                const int t = (plan->dev_slot - N_SLOTS + k) % DEV_SLOTS;
+                if (plan->slot_done[t] == NULL) {
+                        const cudaError_t err = cudaEventCreateWithFlags(&plan->slot_done[t],
+                            cudaEventDisableTiming);
+                        if (err != cudaSuccess) return err;
+                        s = t;
+                        break;
+                }
+                const cudaError_t q = cudaEventQuery(plan->slot_done[t]);
+                if (q == cudaSuccess) {
+                        s = t;
+                } else if (q == cudaErrorNotReady) {
+                        cudaGetLastError(); /* still in flight: not an error of this call */
+                        if ((oldest < 0) || (plan->slot_call[t] < plan->slot_call[oldest]))
+                                oldest = t;
+                } else {
+                        return q;
+                }
+        }
+        if (s < 0) {
+                const cudaError_t err = cudaEventSynchronize(plan->slot_done[oldest]);
+                if (err != cudaSuccess) return err;
+                s = oldest;
+        }
+        plan->slot_call[s] = ++plan->dev_calls;
+        plan->dev_slot = N_SLOTS + s;
+        *slot = N_SLOTS + s;
+        return cudaSuccess;
+}
+
+/* The slot is free again once `stream` has done what is queued on it so far. `err`: the
+ * status of the call, returned unless it is a success. */
+static cudaError_t release_device_slot(struct turtle_plan * plan, int slot, cudaStream_t stream,
+    cudaError_t err)
+{
+        const cudaError_t rec = cudaEventRecord(plan->slot_done[slot - N_SLOTS], stream);
+        return (err != cudaSuccess) ? err : rec;
 }
 
 /* Device state of a streamed call: [0] watermark, then one counter per chunk. */
@@ -2891,11 +2949,13 @@ extern "C" enum turtle_return turtle_stepper_trace_batch_device(
         CUDA_TRY(&turtle_stepper_trace_batch_device, cudaSetDevice(plan->device));
         memset(&plan->counters, 0x0, sizeof(plan->counters));
         plan->counters.rays = n;
-        const int slot = next_device_slot(plan);
+        int slot;
+        CUDA_TRY(&turtle_stepper_trace_batch_device, next_device_slot(plan, &slot));
         const DeviceIo io = { position, direction, NULL, results, NULL };
+        const cudaError_t err = launch_trace(plan, slot, n, io, rule,
+            plan->d_counters + CTR * slot, (cudaStream_t)stream);
         CUDA_TRY(&turtle_stepper_trace_batch_device,
-            launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
-                (cudaStream_t)stream));
+            release_device_slot(plan, slot, (cudaStream_t)stream, err));
         return TURTLE_RETURN_SUCCESS;
 }
 
@@ -2915,11 +2975,13 @@ extern "C" enum turtle_return turtle_stepper_trace_crossings_device(
         CUDA_TRY(fn, cudaSetDevice(plan->device));
         memset(&plan->counters, 0x0, sizeof(plan->counters));
         plan->counters.rays = n;
-        const int slot = next_device_slot(plan);
+        int slot;
+        CUDA_TRY(fn, next_device_slot(plan, &slot));
         const DeviceIo io = { position, direction, NULL, results, NULL };
-        CUDA_TRY(fn, launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
-                         (cudaStream_t)stream, NULL, (max_crossings > 0) ? crossings : NULL,
-                         max_crossings));
+        const cudaError_t err = launch_trace(plan, slot, n, io, rule,
+            plan->d_counters + CTR * slot, (cudaStream_t)stream, NULL,
+            (max_crossings > 0) ? crossings : NULL, max_crossings);
+        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
         return TURTLE_RETURN_SUCCESS;
 }
 
@@ -2953,12 +3015,11 @@ static cudaError_t plan_pipeline(struct turtle_plan * plan, size_t rays)
         return err;
 }
 
-extern "C" void turtle_plan_counters_sync(struct turtle_plan * plan)
+/* The step / sample counters of the launch that used counter block `slot`, once it is over. */
+static void read_counters(struct turtle_plan * plan, int slot)
 {
-        /* device-pointer calls: the caller has synchronised its stream */
         unsigned long long c[CTR];
-        cudaSetDevice(plan->device);
-        if (cudaMemcpy(c, plan->d_counters + CTR * plan->dev_slot, sizeof c,
+        if (cudaMemcpy(c, plan->d_counters + CTR * slot, sizeof c,
                 cudaMemcpyDeviceToHost) == cudaSuccess) {
                 plan->counters.steps = c[1];
                 plan->counters.samples = c[2];
@@ -2966,6 +3027,13 @@ extern "C" void turtle_plan_counters_sync(struct turtle_plan * plan)
                 plan->counters.window_hits = c[5];
                 if (c[6] != 0ull) plan->counters.rays = c[6]; /* the probes of a horizon search */
         }
+}
+
+extern "C" void turtle_plan_counters_sync(struct turtle_plan * plan)
+{
+        /* device-pointer calls: the caller has synchronised its stream */
+        cudaSetDevice(plan->device);
+        read_counters(plan, plan->dev_slot);
 }
 
 /* ---- fans and field arrays ------------------------------------------------------------- */
@@ -3303,7 +3371,7 @@ static enum turtle_return trace_rounds(turtle_function_t * fn, struct turtle_pla
  * rays, first), each a RESIDENT compact kernel followed by the copy of its records / field
  * slices to the host, alternating on two streams: the copy of a slice runs under the
  * kernel of the next, and the SMs that the tail of one slice leaves idle are taken by the
- * head of the next (concurrent launches on one plan, see next_device_slot). Only the copy
+ * head of the next (concurrent launches on one plan). Only the copy
  * of the last slice is exposed. (The streamed kernel -- chunk flags, fences, a lane-side
  * watermark -- does the same at 5 % more kernel time; it stays the path of calls that
  * must stream rays in.) */
@@ -3354,7 +3422,8 @@ static enum turtle_return trace_fan_sliced(turtle_function_t * fn, struct turtle
         CUDA_TRY(fn, fan_upload(plan, 0, fan, bundle, 0, lanes[0], &tables));
         CUDA_TRY(fn, cudaEventRecord(plan->ev0[0], lanes[0]));
         CUDA_TRY(fn, cudaStreamWaitEvent(lanes[1], plan->ev0[0], 0));
-        int slots[DEV_SLOTS];
+        /* a host-pointer call: counter blocks of its own, none of the device-pointer ring */
+        unsigned long long * d_counters = plan->d_counters + CTR * ALL_SLOTS;
         plan->counters.launches = 0;
         for (size_t k = 0; k < n_slices; k++) {
                 const size_t first = k * per_slice;
@@ -3370,9 +3439,7 @@ static enum turtle_return trace_fan_sliced(turtle_function_t * fn, struct turtle
                 const DeviceIo io = { NULL, NULL, &slice,
                         (results != NULL) ? plan->d_all_out + first : NULL,
                         (n_fields > 0) ? &d_fields : NULL };
-                slots[k] = next_device_slot(plan);
-                CUDA_TRY(fn, launch_trace(plan, slots[k], m, io, rule,
-                                 plan->d_counters + CTR * slots[k], st));
+                CUDA_TRY(fn, launch_trace(plan, 0, m, io, rule, d_counters + CTR * k, st));
                 if (results != NULL)
                         CUDA_TRY(fn, cudaMemcpyAsync(results + first, plan->d_all_out + first,
                                          m * sizeof(turtle_trace_result), cudaMemcpyDeviceToHost, st));
@@ -3393,8 +3460,7 @@ static enum turtle_return trace_fan_sliced(turtle_function_t * fn, struct turtle
         memset(&plan->counters, 0x0, sizeof(plan->counters));
         for (size_t k = 0; k < n_slices; k++) {
                 unsigned long long c[CTR];
-                CUDA_TRY(fn, cudaMemcpy(c, plan->d_counters + CTR * slots[k], sizeof c,
-                                 cudaMemcpyDeviceToHost));
+                CUDA_TRY(fn, cudaMemcpy(c, d_counters + CTR * k, sizeof c, cudaMemcpyDeviceToHost));
                 plan->counters.steps += c[1];
                 plan->counters.samples += c[2];
                 plan->counters.rebuilds += c[4];
@@ -3438,12 +3504,15 @@ extern "C" enum turtle_return turtle_stepper_trace_fan_device(struct turtle_plan
         CUDA_TRY(fn, cudaSetDevice(plan->device));
         memset(&plan->counters, 0x0, sizeof(plan->counters));
         plan->counters.rays = n;
-        const int slot = next_device_slot(plan);
+        int slot;
+        CUDA_TRY(fn, next_device_slot(plan, &slot));
         FanTables tables;
-        CUDA_TRY(fn, fan_upload(plan, slot, fan, bundle, 0, (cudaStream_t)stream, &tables));
+        cudaError_t err = fan_upload(plan, slot, fan, bundle, 0, (cudaStream_t)stream, &tables);
         const DeviceIo io = { NULL, NULL, &tables, results, fields };
-        CUDA_TRY(fn, launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
-                         (cudaStream_t)stream));
+        if (err == cudaSuccess)
+                err = launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
+                    (cudaStream_t)stream);
+        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
         return TURTLE_RETURN_SUCCESS;
 }
 
@@ -3472,10 +3541,12 @@ extern "C" enum turtle_return turtle_stepper_trace_fields_device(struct turtle_p
         CUDA_TRY(fn, cudaSetDevice(plan->device));
         memset(&plan->counters, 0x0, sizeof(plan->counters));
         plan->counters.rays = n;
-        const int slot = next_device_slot(plan);
+        int slot;
+        CUDA_TRY(fn, next_device_slot(plan, &slot));
         const DeviceIo io = { position, direction, NULL, NULL, fields };
-        CUDA_TRY(fn, launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
-                         (cudaStream_t)stream));
+        const cudaError_t err = launch_trace(plan, slot, n, io, rule,
+            plan->d_counters + CTR * slot, (cudaStream_t)stream);
+        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
         return TURTLE_RETURN_SUCCESS;
 }
 
@@ -3506,14 +3577,15 @@ static enum turtle_return check_horizon(turtle_function_t * fn, const struct tur
         return TURTLE_RETURN_SUCCESS;
 }
 
-/* Queue the search on `stream`: azimuth table (fan_upload), counters, kernel. */
-static cudaError_t launch_horizon(struct turtle_plan * plan, double latitude, double longitude,
+/* Queue the search on `stream`: azimuth table (fan_upload), counters, kernel; with the
+ * counter block and tables of `slot`. */
+static cudaError_t launch_horizon(struct turtle_plan * plan, int slot, double latitude,
+    double longitude,
     const double position[3], size_t n_azimuth, const double * azimuth, double elevation_min,
     double elevation_max, double tolerance, const struct turtle_trace_rule * rule,
     struct turtle_horizon * results, cudaStream_t stream)
 {
         memset(&plan->counters, 0x0, sizeof(plan->counters));
-        const int slot = next_device_slot(plan);
         unsigned long long * d_counters = plan->d_counters + CTR * slot;
         struct turtle_fan fan;
         memset(&fan, 0x0, sizeof fan);
@@ -3581,9 +3653,12 @@ extern "C" enum turtle_return turtle_stepper_horizon_device(struct turtle_plan *
             elevation_min, elevation_max, tolerance, rule, results);
         if ((rc != TURTLE_RETURN_SUCCESS) || (n_azimuth == 0)) return rc;
         CUDA_TRY(fn, cudaSetDevice(plan->device));
-        CUDA_TRY(fn, launch_horizon(plan, latitude, longitude, position, n_azimuth, azimuth,
-                         elevation_min, elevation_max, tolerance, rule, results,
-                         (cudaStream_t)stream));
+        int slot;
+        CUDA_TRY(fn, next_device_slot(plan, &slot));
+        const cudaError_t err = launch_horizon(plan, slot, latitude, longitude, position,
+            n_azimuth, azimuth, elevation_min, elevation_max, tolerance, rule, results,
+            (cudaStream_t)stream);
+        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
         return TURTLE_RETURN_SUCCESS;
 }
 
@@ -3600,12 +3675,13 @@ extern "C" enum turtle_return turtle_stepper_horizon(struct turtle_plan * plan,
         struct turtle_horizon * d_results = NULL;
         const size_t bytes = n_azimuth * sizeof(*d_results);
         CUDA_TRY(fn, cudaMalloc((void **)&d_results, bytes));
-        cudaError_t err = launch_horizon(plan, latitude, longitude, position, n_azimuth, azimuth,
-            elevation_min, elevation_max, tolerance, rule, d_results, NULL);
+        /* a host-pointer call: the counter block and tables of the host pipeline's slot 0 */
+        cudaError_t err = launch_horizon(plan, 0, latitude, longitude, position, n_azimuth,
+            azimuth, elevation_min, elevation_max, tolerance, rule, d_results, NULL);
         if (err == cudaSuccess) err = cudaMemcpy(results, d_results, bytes, cudaMemcpyDeviceToHost);
         cudaFree(d_results);
         CUDA_TRY(fn, err);
-        turtle_plan_counters_sync(plan);
+        read_counters(plan, 0);
         return TURTLE_RETURN_SUCCESS;
 }
 
@@ -3742,11 +3818,12 @@ extern "C" enum turtle_return turtle_states_reset(struct turtle_states * states)
 
 /* Launch the walk kernel: n particles, n_steps turtle_stepper_step each (1: the step_batch
  * calls, states used in place; > 1: turtle_stepper_walk_batch, state resident in the lane
- * store for the whole launch). */
+ * store for the whole launch). A device-pointer call (`ring`) takes its counter block from
+ * the ring of in-flight calls, a host-pointer call uses the one of the host pipeline. */
 static enum turtle_return launch_walk(turtle_function_t * fn, struct turtle_plan * plan,
     struct turtle_states * states, size_t n, int n_steps, bool multi, double * position,
     const double * direction, double * latitude, double * longitude, double * altitude,
-    double * elevation, double * step, int * index, void * stream)
+    double * elevation, double * step, int * index, void * stream, bool ring)
 {
         if ((states != NULL) && ((states->plan != plan) || (states->n < n)))
                 return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
@@ -3766,12 +3843,18 @@ static enum turtle_return launch_walk(turtle_function_t * fn, struct turtle_plan
         A.step = step;
         A.index = index;
         A.n_steps = n_steps;
-        A.counters = plan->d_counters + CTR * next_device_slot(plan);
+        int slot = 0;
+        if (ring) CUDA_TRY(fn, next_device_slot(plan, &slot));
+        A.counters = plan->d_counters + CTR * slot;
         const int threads = 128;
         int blocks = (int)std::min<size_t>((n + threads - 1) / threads,
             (size_t)plan->sm_count * 5);
         cudaStream_t st = (cudaStream_t)stream;
-        CUDA_TRY(fn, cudaMemsetAsync(A.counters, 0x0, CTR * sizeof(unsigned long long), st));
+        cudaError_t err = cudaMemsetAsync(A.counters, 0x0, CTR * sizeof(unsigned long long), st);
+        if (err != cudaSuccess) {
+                if (ring) release_device_slot(plan, slot, st, err);
+                CUDA_TRY(fn, err);
+        }
         const bool lla = plan->G.range > 0.;
         bool proj = false;
         for (int t = 0; t < plan->G.n_transforms; t++)
@@ -3815,7 +3898,9 @@ static enum turtle_return launch_walk(turtle_function_t * fn, struct turtle_plan
         plan->counters.launches++;
         plan->counters.rays = n;
         plan->counters.steps = (direction != NULL) ? n * (size_t)n_steps : 0;
-        CUDA_TRY(fn, cudaGetLastError());
+        err = cudaGetLastError();
+        if (ring) err = release_device_slot(plan, slot, st, err);
+        CUDA_TRY(fn, err);
         return TURTLE_RETURN_SUCCESS;
 }
 
@@ -3826,7 +3911,8 @@ extern "C" enum turtle_return turtle_stepper_step_batch_device(
     int * index, void * stream)
 {
         return launch_walk(FN(&turtle_stepper_step_batch_device), plan, states, n, 1, false,
-            position, direction, latitude, longitude, altitude, elevation, step, index, stream);
+            position, direction, latitude, longitude, altitude, elevation, step, index, stream,
+            true);
 }
 
 /* n_steps successive turtle_stepper_step per particle in one launch (turtle_b200.h). */
@@ -3840,7 +3926,7 @@ extern "C" enum turtle_return turtle_stepper_walk_batch_device(struct turtle_pla
                 return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
                     "a walk needs at least one step and its directions");
         return launch_walk(fn, plan, states, n, n_steps, true, position, direction, latitude,
-            longitude, altitude, elevation, step, index, stream);
+            longitude, altitude, elevation, step, index, stream, true);
 }
 
 /* Small RAII helper for the host-pointer wrappers of the simple kernels. */
@@ -3906,11 +3992,14 @@ extern "C" enum turtle_return turtle_stepper_trace_crossings(
         CUDA_TRY(fn, buf.get((void **)&d_res, NULL, n * sizeof(*d_res), false));
         CUDA_TRY(fn, buf.get((void **)&d_cross, NULL, cross_bytes ? cross_bytes : 16, false));
         CUDA_TRY(fn, cudaMemset(d_cross, 0x0, cross_bytes ? cross_bytes : 16));
-        rc = turtle_stepper_trace_crossings_device(plan, n, d_pos, d_dir, rule, d_res, d_cross,
-            max_crossings, NULL);
-        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        /* the counter block and schedule buffers of the host pipeline's slot 0 */
+        memset(&plan->counters, 0x0, sizeof(plan->counters));
+        plan->counters.rays = n;
+        const DeviceIo io = { d_pos, d_dir, NULL, d_res, NULL };
+        CUDA_TRY(fn, launch_trace(plan, 0, n, io, rule, plan->d_counters, NULL, NULL,
+                         (max_crossings > 0) ? d_cross : NULL, max_crossings));
         CUDA_TRY(fn, cudaDeviceSynchronize());
-        turtle_plan_counters_sync(plan);
+        read_counters(plan, 0);
         CUDA_TRY(fn, cudaMemcpy(results, d_res, n * sizeof(*d_res), cudaMemcpyDeviceToHost));
         if (cross_bytes)
                 CUDA_TRY(fn, cudaMemcpy(crossings, d_cross, cross_bytes, cudaMemcpyDeviceToHost));
@@ -3976,8 +4065,8 @@ extern "C" enum turtle_return turtle_stepper_step_batch(struct turtle_plan * pla
         DEV_OUT(&turtle_stepper_step_batch, B, d_el, elevation, n * 2 * sizeof(double));
         DEV_OUT(&turtle_stepper_step_batch, B, d_step, step, n * sizeof(double));
         DEV_OUT(&turtle_stepper_step_batch, B, d_idx, index, n * 2 * sizeof(int));
-        enum turtle_return rc = turtle_stepper_step_batch_device(plan, states, n, d_pos, d_dir,
-            d_lat, d_lon, d_alt, d_el, d_step, d_idx, NULL);
+        enum turtle_return rc = launch_walk(FN(&turtle_stepper_step_batch), plan, states, n, 1,
+            false, d_pos, d_dir, d_lat, d_lon, d_alt, d_el, d_step, d_idx, NULL, false);
         if (rc != TURTLE_RETURN_SUCCESS) return rc;
         CUDA_TRY(&turtle_stepper_step_batch, cudaDeviceSynchronize());
         if (direction != NULL)
@@ -4014,8 +4103,8 @@ extern "C" enum turtle_return turtle_stepper_walk_batch(struct turtle_plan * pla
         DEV_OUT(fn, B, d_el, elevation, m * 2 * sizeof(double));
         DEV_OUT(fn, B, d_step, step, m * sizeof(double));
         DEV_OUT(fn, B, d_idx, index, m * 2 * sizeof(int));
-        enum turtle_return rc = turtle_stepper_walk_batch_device(plan, states, n, n_steps, d_pos,
-            d_dir, d_lat, d_lon, d_alt, d_el, d_step, d_idx, NULL);
+        enum turtle_return rc = launch_walk(fn, plan, states, n, n_steps, true, d_pos, d_dir,
+            d_lat, d_lon, d_alt, d_el, d_step, d_idx, NULL, false);
         if (rc != TURTLE_RETURN_SUCCESS) return rc;
         CUDA_TRY(fn, cudaDeviceSynchronize());
         DEV_BACK(fn, position, d_pos, n * 3 * sizeof(double));
