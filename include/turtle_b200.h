@@ -99,17 +99,17 @@ struct turtle_plan_counters {
 
 /* Threading: a plan carries the streams, staging buffers and counters of the calls made
  * through it, and is used from one host thread at a time. HOST-pointer calls (`*_batch`,
- * `_trace_fan`, `_trace_fields`, `_trace_crossings`, `_horizon`) return when their results are
+ * `_trace_fan[s]`, `_trace_fields`, `_trace_crossings`, `_horizon[s]`) return when their results are
  * in place: ONE at a time per plan. DEVICE-pointer calls (`*_device`) are asynchronous on the
  * caller's stream: that is how a caller with several batches hides the tail of one (a launch
  * ends when its slowest ray does) behind the head of the next. A device-pointer call is IN
  * FLIGHT from its return until its stream has done all it queued; up to 8 may be in flight on
  * one plan, on streams of the caller's choice, and they may complete in any order. Each holds
  * one of 8 slots of the plan (the queue cursor of its kernel, its schedule buffers and its
- * fan / azimuth tables) until it completes; a ninth call waits on the host until the call
+ * fan / azimuth / station tables) until it completes; a ninth call waits on the host until the call
  * that took its slot first is over. Host-pointer calls have slots of their own and may be
  * made while device-pointer calls are in flight; those that stage their arrays in device
- * memory of their own (turtle_stepper_step_batch, _walk_batch, _trace_crossings, _horizon)
+ * memory of their own (turtle_stepper_step_batch, _walk_batch, _trace_crossings, _horizon[s])
  * free it before they return, which waits for the device to be idle. After the caller has
  * synchronised, turtle_plan_counters_sync reports the device-pointer call issued last.
  * Several plans (one per host thread or per device) are independent; they share nothing but
@@ -263,6 +263,36 @@ TURTLE_API enum turtle_return turtle_stepper_trace_fan_device(struct turtle_plan
     const struct turtle_fan * fan, const struct turtle_trace_rule * rule,
     struct turtle_trace_result * results, const struct turtle_trace_fields * fields,
     void * stream);
+/* One angle grid shot from n_station stations in ONE call: site surveys, joint inversions of
+ * several telescopes, the shadows of an antenna array. Ray r = s * (n_azimuth * n_elevation)
+ * + q, where q is the ray order of struct turtle_fan (bands of `bundle` elevations) and s the
+ * station: ray r is, record and fields byte for byte, ray q of turtle_stepper_trace_fan with
+ * the fan { latitude[s], longitude[s], position + 3 * s, n_azimuth, n_elevation, azimuth,
+ * elevation, bundle }. The frame of every station is taken on the host by the calls of
+ * turtle_ecef_from_horizontal, as for one fan. All arrays of the struct are HOST memory, also
+ * for the _device variant; `results` and `fields` (n_station * n_azimuth * n_elevation rays)
+ * are host memory here and device memory in the _device variant, which is ONE launch. A
+ * station without data or with a non-finite latitude or position gives what the one-station
+ * call gives for it (TURTLE_TRACE_INVALID rays for a non-finite position); it is not an error
+ * of the call. The arguments are checked before the plan or the device is used; n_station = 0
+ * or an empty grid does nothing. The plan counters report all the rays. */
+struct turtle_fans {
+        size_t n_station;
+        const double * latitude;    /* [n_station] degrees: local frame of station s */
+        const double * longitude;   /* [n_station] degrees */
+        const double * position;    /* [n_station][3] ECEF origin of the rays of station s */
+        size_t n_azimuth, n_elevation;
+        const double * azimuth;     /* degrees, shared by every station */
+        const double * elevation;
+        size_t bundle;
+};
+TURTLE_API enum turtle_return turtle_stepper_trace_fans(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    struct turtle_trace_result * results, const struct turtle_trace_fields * fields);
+TURTLE_API enum turtle_return turtle_stepper_trace_fans_device(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    struct turtle_trace_result * results, const struct turtle_trace_fields * fields,
+    void * stream);
 /* turtle_stepper_trace_batch with field arrays instead of records. */
 TURTLE_API enum turtle_return turtle_stepper_trace_fields(struct turtle_plan * plan, size_t n,
     const double * position, const double * direction, const struct turtle_trace_rule * rule,
@@ -323,6 +353,24 @@ TURTLE_API enum turtle_return turtle_stepper_horizon_device(struct turtle_plan *
     double latitude, double longitude, const double position[3], size_t n_azimuth,
     const double * azimuth, double elevation_min, double elevation_max, double tolerance,
     const struct turtle_trace_rule * rule, struct turtle_horizon * results, void * stream);
+/* The horizons of n_station stations in ONE call (the horizon of every antenna of an array,
+ * a sky-view raster with one station per node): results[s * n_azimuth + i] is, byte for
+ * byte, results[i] of turtle_stepper_horizon(plan, latitude[s], longitude[s], position +
+ * 3 * s, n_azimuth, azimuth, ...), n_probes and n_iterations included. latitude, longitude
+ * ([n_station], degrees), position ([n_station][3]) and azimuth are HOST memory in both
+ * variants. A station without data or with non-finite values gives TURTLE_HORIZON_INVALID
+ * records, as alone; a missing array is TURTLE_RETURN_BAD_ADDRESS, a bad window or tolerance
+ * TURTLE_RETURN_DOMAIN_ERROR, checked before the plan or the device is used; n_station = 0 or
+ * n_azimuth = 0 does nothing. The plan counters report the probes of all stations as rays. */
+TURTLE_API enum turtle_return turtle_stepper_horizons(struct turtle_plan * plan,
+    size_t n_station, const double * latitude, const double * longitude, const double * position,
+    size_t n_azimuth, const double * azimuth, double elevation_min, double elevation_max,
+    double tolerance, const struct turtle_trace_rule * rule, struct turtle_horizon * results);
+TURTLE_API enum turtle_return turtle_stepper_horizons_device(struct turtle_plan * plan,
+    size_t n_station, const double * latitude, const double * longitude, const double * position,
+    size_t n_azimuth, const double * azimuth, double elevation_min, double elevation_max,
+    double tolerance, const struct turtle_trace_rule * rule, struct turtle_horizon * results,
+    void * stream);
 
 /* ---- the stream of medium changes along every ray (SURVEY.md section 8f, N4) --------
  * What a Monte-Carlo engine integrates over the steps -- column density, energy loss per

@@ -59,6 +59,14 @@ class Fan(C.Structure):
                 ("elevation", C.c_void_p), ("bundle", C.c_size_t)]
 
 
+class Fans(C.Structure):
+    """struct turtle_fans (include/turtle_b200.h): one angle grid, n_station stations."""
+    _fields_ = [("n_station", C.c_size_t), ("latitude", C.c_void_p), ("longitude", C.c_void_p),
+                ("position", C.c_void_p), ("n_azimuth", C.c_size_t),
+                ("n_elevation", C.c_size_t), ("azimuth", C.c_void_p),
+                ("elevation", C.c_void_p), ("bundle", C.c_size_t)]
+
+
 class PlanCounters(C.Structure):
     """struct turtle_plan_counters (include/turtle_b200.h)."""
     _fields_ = [("rays", C.c_uint64), ("steps", C.c_uint64),
@@ -165,6 +173,10 @@ SIGNATURES = {
                                       C.POINTER(TraceFields)]),
     "turtle_stepper_trace_fan_device": (_I, [_P, C.POINTER(Fan), C.POINTER(TraceRule), _P,
                                              C.POINTER(TraceFields), _P]),
+    "turtle_stepper_trace_fans": (_I, [_P, C.POINTER(Fans), C.POINTER(TraceRule), _P,
+                                       C.POINTER(TraceFields)]),
+    "turtle_stepper_trace_fans_device": (_I, [_P, C.POINTER(Fans), C.POINTER(TraceRule), _P,
+                                              C.POINTER(TraceFields), _P]),
     "turtle_stepper_trace_fields": (_I, [_P, _N, _P, _P, C.POINTER(TraceRule),
                                          C.POINTER(TraceFields)]),
     "turtle_stepper_trace_fields_device": (_I, [_P, _N, _P, _P, C.POINTER(TraceRule),
@@ -175,6 +187,10 @@ SIGNATURES = {
     "turtle_stepper_horizon": (_I, [_P, _D, _D, _P, _N, _P, _D, _D, _D, C.POINTER(TraceRule), _P]),
     "turtle_stepper_horizon_device": (_I, [_P, _D, _D, _P, _N, _P, _D, _D, _D,
                                            C.POINTER(TraceRule), _P, _P]),
+    "turtle_stepper_horizons": (_I, [_P, _N, _P, _P, _P, _N, _P, _D, _D, _D,
+                                     C.POINTER(TraceRule), _P]),
+    "turtle_stepper_horizons_device": (_I, [_P, _N, _P, _P, _P, _N, _P, _D, _D, _D,
+                                            C.POINTER(TraceRule), _P, _P]),
     # particle steps
     "turtle_states_create": (_I, [_P, _N, _PP]),
     "turtle_states_destroy": (None, [_PP]),

@@ -9,7 +9,7 @@ import ctypes as C
 
 import numpy as np
 
-from ._lib import (ERROR_HANDLER, Fan, MapInfo, PlanCounters, TraceFields, Residency, ResidencyReport, TraceRule,
+from ._lib import (ERROR_HANDLER, Fan, Fans, MapInfo, PlanCounters, TraceFields, Residency, ResidencyReport, TraceRule,
                    lib)
 
 TRACE_RESULT = np.dtype([
@@ -496,6 +496,35 @@ class Plan:
             self._p, C.byref(fan[0]), C.byref(rule), _ptr(results) if results is not None else None,
             C.byref(f) if f is not None else None, C.c_void_p(stream) if stream else None))
 
+    @staticmethod
+    def make_fans(latitude, longitude, position, azimuth, elevation, bundle=1):
+        """struct turtle_fans: one angle grid from every station (latitude[s], longitude[s],
+        position[s]), over host arrays (kept alive by the returned pair). Ray
+        s * len(azimuth) * len(elevation) + q is ray q of station s's make_fan."""
+        la, lo = _f8(latitude).reshape(-1), _f8(longitude).reshape(-1)
+        pos = _f8(position, (-1, 3))
+        az, el = _f8(azimuth).reshape(-1), _f8(elevation).reshape(-1)
+        if not len(la) == len(lo) == len(pos):
+            raise ValueError("one latitude, longitude and position per station")
+        fans = Fans(len(la), _ptr(la), _ptr(lo), _ptr(pos), len(az), len(el), _ptr(az), _ptr(el),
+                    bundle)
+        return fans, (la, lo, pos, az, el)
+
+    def trace_fans(self, fans, rule, results=None, fields=None):
+        """turtle_stepper_trace_fans: host records and / or host field arrays out."""
+        f = self._fields_struct(fields) if fields else None
+        _check(lib.turtle_stepper_trace_fans(
+            self._p, C.byref(fans[0]), C.byref(rule), _ptr(results) if results is not None else None,
+            C.byref(f) if f is not None else None))
+        return results, fields
+
+    def trace_fans_device(self, fans, rule, results=None, fields=None, stream=None):
+        """turtle_stepper_trace_fans_device: device records / fields, one launch, asynchronous."""
+        f = self._fields_struct(fields) if fields else None
+        _check(lib.turtle_stepper_trace_fans_device(
+            self._p, C.byref(fans[0]), C.byref(rule), _ptr(results) if results is not None else None,
+            C.byref(f) if f is not None else None, C.c_void_p(stream) if stream else None))
+
     def trace_fields(self, position, direction, rule, fields):
         """turtle_stepper_trace_fields: host rays in, host field arrays out."""
         position, direction = _f8(position, (-1, 3)), _f8(direction, (-1, 3))
@@ -537,6 +566,37 @@ class Plan:
         _check(lib.turtle_stepper_horizon_device(
             self._p, latitude, longitude, pos, len(az), _ptr(az), elevation[0], elevation[1],
             tolerance, C.byref(rule), _ptr(results), C.c_void_p(stream) if stream else None))
+
+    @staticmethod
+    def _stations(latitude, longitude, position):
+        la, lo = _f8(latitude).reshape(-1), _f8(longitude).reshape(-1)
+        pos = _f8(position, (-1, 3))
+        if not len(la) == len(lo) == len(pos):
+            raise ValueError("one latitude, longitude and position per station")
+        return la, lo, pos
+
+    def horizons(self, latitude, longitude, position, azimuth, rule, elevation=(-90., 90.),
+                 tolerance=1e-6):
+        """turtle_stepper_horizons: the horizon of every station (latitude[s], longitude[s],
+        position[s]) for each azimuth -> HORIZON_RESULT array [n_station, n_azimuth]."""
+        la, lo, pos = self._stations(latitude, longitude, position)
+        az = _f8(azimuth).reshape(-1)
+        results = np.zeros((len(la), len(az)), dtype=HORIZON_RESULT)
+        _check(lib.turtle_stepper_horizons(self._p, len(la), _ptr(la), _ptr(lo), _ptr(pos),
+                                           len(az), _ptr(az), elevation[0], elevation[1],
+                                           tolerance, C.byref(rule), _ptr(results)))
+        return results
+
+    def horizons_device(self, latitude, longitude, position, azimuth, rule, results,
+                        elevation=(-90., 90.), tolerance=1e-6, stream=None):
+        """turtle_stepper_horizons_device: stations and azimuths on the host, `results` a
+        device tensor of n_station * len(azimuth) * 96 bytes; asynchronous on `stream`."""
+        la, lo, pos = self._stations(latitude, longitude, position)
+        az = _f8(azimuth).reshape(-1)
+        _check(lib.turtle_stepper_horizons_device(
+            self._p, len(la), _ptr(la), _ptr(lo), _ptr(pos), len(az), _ptr(az), elevation[0],
+            elevation[1], tolerance, C.byref(rule), _ptr(results),
+            C.c_void_p(stream) if stream else None))
 
     def step(self, position, direction=None, states=None):
         """One turtle_stepper_step per particle, host arrays. Returns a dict of arrays;

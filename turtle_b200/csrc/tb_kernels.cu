@@ -88,14 +88,16 @@ struct TraceArgs {
  * own, of the COMPACT kernels only -- the mere presence of these members in TraceArgs
  * costs every trace kernel four registers. */
 struct CompactArgs {
-        /* fan input (turtle_stepper_trace_fan; TraceArgs::position == NULL): every ray starts at
-         * fan_origin; direction of ray (i, j) from the host's sines / cosines of the
-         * angles, fan_az[i] = { sin az, cos az }, fan_el[j] = { cos el, sin el }, and the
-         * local East / North / Up vectors (ecef.c:136-178) */
+        /* fan input (turtle_stepper_trace_fan[s]; TraceArgs::position == NULL): ray r belongs to
+         * station s = r / fan_per_station and starts at its origin; direction of ray (i, j)
+         * from the host's sines / cosines of the angles, fan_az[i] = { sin az, cos az },
+         * fan_el[j] = { cos el, sin el }, and the station's East / North / Up vectors
+         * (ecef.c:136-178). fan_station[12 s ...]: origin, East, North, Up of station s. */
         const double2 * fan_az;
         const double2 * fan_el;
-        double fan_origin[3], fan_e[3], fan_n[3], fan_u[3];
-        unsigned long long fan_naz, fan_bundle, fan_ray0; /* ray0: first ray of this launch */
+        const double * fan_station;
+        unsigned long long fan_naz, fan_bundle, fan_per_station;
+        unsigned long long fan_ray0; /* first ray of this launch */
         /* field outputs (turtle_trace_fields: device arrays, any NULL), when use_fields */
         turtle_trace_fields fields;
         int use_fields;
@@ -207,13 +209,16 @@ __device__ __forceinline__ void compiler_fence() { asm volatile("" ::: "memory")
 /* Compact input / output of the trace kernel (COMPACT variants only: the kernels of
  * turtle_stepper_trace_fan / _fields; the others do not carry this code). */
 
-/* Direction of ray r of a fan: the products and sums of turtle_ecef_from_horizontal
- * (ecef.c:170-177) on the host's sines / cosines of the two angles. */
+/* Origin and direction of ray r of a fan: the products and sums of
+ * turtle_ecef_from_horizontal (ecef.c:170-177) on the host's sines / cosines of the two
+ * angles and the frame of the ray's station, read once per ray. */
 __device__ __forceinline__ void fan_ray(const CompactArgs & A, unsigned long long r, double pos[3],
     double dir[3])
 {
         const unsigned long long per_band = A.fan_naz * A.fan_bundle;
-        const unsigned long long rr = r + A.fan_ray0;
+        const unsigned long long rs = r + A.fan_ray0;
+        const unsigned long long s = rs / A.fan_per_station;
+        const unsigned long long rr = rs - s * A.fan_per_station;
         const unsigned long long band = rr / per_band;
         const unsigned long long rem = rr - band * per_band;
         const unsigned long long i = rem / A.fan_bundle;
@@ -221,10 +226,11 @@ __device__ __forceinline__ void fan_ray(const CompactArgs & A, unsigned long lon
         const double2 az = __ldg(A.fan_az + i);
         const double2 el = __ldg(A.fan_el + j);
         const double r0 = el.x * az.x, r1 = el.x * az.y, r2 = el.y;
+        const double * f = A.fan_station + 12ull * s;
 #pragma unroll
         for (int c = 0; c < 3; c++) {
-                pos[c] = A.fan_origin[c];
-                dir[c] = r0 * A.fan_e[c] + r1 * A.fan_n[c] + r2 * A.fan_u[c];
+                pos[c] = __ldg(f + c);
+                dir[c] = r0 * __ldg(f + 3 + c) + r1 * __ldg(f + 6 + c) + r2 * __ldg(f + 9 + c);
         }
 }
 
@@ -801,8 +807,10 @@ __global__ void __launch_bounds__(128, MINB)
  * members added to TraceArgs cost every trace kernel registers (see CompactArgs). */
 struct HorizonArgs {
         const double2 * az; /* { sin az, cos az } per azimuth, taken on the host (fan_upload) */
-        unsigned long long n;
-        double origin[3], e[3], north[3], up[3]; /* the station and its East / North / Up frame */
+        /* station[12 s ...]: origin, East, North, Up of station s (fan_upload) */
+        const double * station;
+        unsigned long long n;         /* work items: n_station x n_azimuth */
+        unsigned long long n_azimuth; /* item a is azimuth a % n_azimuth of station a / n_azimuth */
         double elevation_min, elevation_max, tolerance;
         double altitude_min, altitude_max, length_max;
         int max_steps;
@@ -833,10 +841,12 @@ __global__ void __launch_bounds__(128, MINB)
         constexpr int NF = LLA ? N_F_LLA : N_F_BASE, NI = LLA ? N_I : N_I_BASE;
         __shared__ LaneStoreT<NF, NI> store;
         __shared__ turtle_horizon record[4]; /* one per warp: the azimuth being searched */
+        __shared__ double frame[4][12];      /* ... and the frame of its station */
         const unsigned tid = threadIdx.x;
         const unsigned lane = tid & 31u;
         const unsigned FULL = 0xffffffffu;
         turtle_horizon & R = record[tid >> 5];
+        const double * F = frame[tid >> 5];
 #define SF(k) store.f[((k) < NF) ? (k) : 0][tid]
 #define SI(k) store.i[((k) < NI) ? (k) : 0][tid]
         extern __shared__ double lla_store[];
@@ -920,7 +930,9 @@ __global__ void __launch_bounds__(128, MINB)
                                 if (azimuth >= A.n) break;
                                 active = true;
                                 round = 0;
-                                sc = __ldg(A.az + azimuth);
+                                const unsigned long long s = azimuth / A.n_azimuth;
+                                sc = __ldg(A.az + (azimuth - s * A.n_azimuth));
+                                if (lane < 12u) frame[tid >> 5][lane] = __ldg(A.station + 12ull * s + lane);
                                 if (lane == 0u) {
                                         const double nan = __longlong_as_double(0x7ff8000000000000ll);
                                         R.elevation[0] = R.elevation[1] = R.length = nan;
@@ -951,8 +963,8 @@ __global__ void __launch_bounds__(128, MINB)
                         const double r0 = c_el * sc.x, r1 = c_el * sc.y, r2 = s_el;
                         double dir[3];
                         for (int c = 0; c < 3; c++) {
-                                SF(F_POS + c) = A.origin[c];
-                                dir[c] = r0 * A.e[c] + r1 * A.north[c] + r2 * A.up[c];
+                                SF(F_POS + c) = F[c];
+                                dir[c] = r0 * F[3 + c] + r1 * F[6 + c] + r2 * F[9 + c];
                                 SF(F_DIR + c) = dir[c];
                         }
                         SF(F_PROBE) = el;
@@ -965,7 +977,7 @@ __global__ void __launch_bounds__(128, MINB)
                                 SF(F_LASTPOS) = SF(F_LASTPOS + 1) = SF(F_LASTPOS + 2) = DBL_MAX;
                                 tb::lla_reset(G, V);
                         }
-                        const double origin[3] = { A.origin[0], A.origin[1], A.origin[2] };
+                        const double origin[3] = { F[0], F[1], F[2] };
                         if (!finite3(origin) || !finite3(dir)) {
                                 SI(I_OUTCOME) = TURTLE_TRACE_INVALID;
                                 SI(I_STATION) = -1;
@@ -2074,10 +2086,11 @@ struct turtle_plan {
         size_t stream_chunks;
         cudaEvent_t ev_reset;
         cudaStream_t drain[4]; /* N_DRAINS result streams */
-        /* fan tables (turtle_stepper_trace_fan), per slot: pinned host copy + device copy */
+        /* fan tables (turtle_stepper_trace_fan[s], _horizon[s]), per slot: pinned host copy +
+         * device copy of the angles' sines / cosines and the stations' frames (fan_upload) */
         double2 * h_fan[ALL_SLOTS];
         double2 * d_fan[ALL_SLOTS];
-        size_t fan_angles[ALL_SLOTS];
+        size_t fan_entries[ALL_SLOTS]; /* double2 entries allocated */
         /* device staging of the field arrays of a host-pointer call */
         void * d_field_pool;
         size_t field_pool_bytes;
@@ -2272,7 +2285,7 @@ static enum turtle_return freeze_plan(turtle_function_t * fn, struct turtle_step
         for (int k = 0; k < ALL_SLOTS; k++) {
                 plan->h_fan[k] = NULL;
                 plan->d_fan[k] = NULL;
-                plan->fan_angles[k] = 0;
+                plan->fan_entries[k] = 0;
         }
         plan->d_field_pool = NULL;
         plan->field_pool_bytes = 0;
@@ -2788,12 +2801,12 @@ struct StreamState {
         unsigned * chunk_flags;
 };
 
-/* Device tables of a fan: sines / cosines of its angles and the frame of its station. */
+/* Device tables of a fan: sines / cosines of its angles and the frames of its stations. */
 struct FanTables {
         const double2 * az;
         const double2 * el;
-        double origin[3], e[3], n[3], u[3];
-        unsigned long long naz, bundle, ray0;
+        const double * station; /* [n_station][12]: origin, East, North, Up */
+        unsigned long long naz, bundle, per_station, ray0;
 };
 
 /* What one launch reads and writes: DEVICE memory throughout. */
@@ -2834,14 +2847,10 @@ static cudaError_t launch_trace(struct turtle_plan * plan, int slot, size_t n,
                 A.position = A.direction = NULL;
                 C.fan_az = io.fan->az;
                 C.fan_el = io.fan->el;
-                for (int c = 0; c < 3; c++) {
-                        C.fan_origin[c] = io.fan->origin[c];
-                        C.fan_e[c] = io.fan->e[c];
-                        C.fan_n[c] = io.fan->n[c];
-                        C.fan_u[c] = io.fan->u[c];
-                }
+                C.fan_station = io.fan->station;
                 C.fan_naz = io.fan->naz;
                 C.fan_bundle = io.fan->bundle;
+                C.fan_per_station = io.fan->per_station;
                 C.fan_ray0 = io.fan->ray0;
         }
         A.results = io.results;
@@ -3054,54 +3063,98 @@ static enum turtle_return check_fan(turtle_function_t * fn, const struct turtle_
         return TURTLE_RETURN_SUCCESS;
 }
 
-/* Sines and cosines of the angles of a fan, taken on the host by the calls of
- * turtle_ecef_from_horizontal (ecef.c:139-144,170-173), and the East / North / Up frame of
- * its station (compute_enu, ecef.c:136-158); queued for upload on `stream`. */
-static cudaError_t fan_upload(struct turtle_plan * plan, int slot, const struct turtle_fan * fan,
+static enum turtle_return check_fans(turtle_function_t * fn, const struct turtle_fans * fans,
+    size_t * n, size_t * bundle)
+{
+        if ((fans == NULL) || ((fans->n_azimuth > 0) && (fans->azimuth == NULL)) ||
+            ((fans->n_elevation > 0) && (fans->elevation == NULL)))
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
+                    "missing fan angles");
+        if ((fans->n_station > 0) && ((fans->latitude == NULL) || (fans->longitude == NULL) ||
+                                         (fans->position == NULL)))
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
+                    "missing station latitudes, longitudes or positions");
+        *bundle = (fans->bundle > 0) ? fans->bundle : 1;
+        if ((fans->n_elevation % *bundle) != 0)
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "the number of elevations of a fan (%zu) must be a multiple of its bundle (%zu)",
+                    fans->n_elevation, *bundle);
+        *n = fans->n_station * fans->n_azimuth * fans->n_elevation;
+        return TURTLE_RETURN_SUCCESS;
+}
+
+/* A fan as the one-station case of struct turtle_fans. */
+static struct turtle_fans one_station(const struct turtle_fan * fan)
+{
+        struct turtle_fans fans;
+        fans.n_station = 1;
+        fans.latitude = &fan->latitude;
+        fans.longitude = &fan->longitude;
+        fans.position = fan->position;
+        fans.n_azimuth = fan->n_azimuth;
+        fans.n_elevation = fan->n_elevation;
+        fans.azimuth = fan->azimuth;
+        fans.elevation = fan->elevation;
+        fans.bundle = fan->bundle;
+        return fans;
+}
+
+/* Sines and cosines of the angles of the fans, taken on the host by the calls of
+ * turtle_ecef_from_horizontal (ecef.c:139-144,170-173), then the origin and the East / North
+ * / Up frame of every station (compute_enu, ecef.c:136-158), 12 doubles each; ONE table per
+ * slot, queued for upload on `stream`. */
+static cudaError_t fan_upload(struct turtle_plan * plan, int slot, const struct turtle_fans * fans,
     size_t bundle, size_t ray0, cudaStream_t stream, FanTables * T)
 {
-        const size_t angles = fan->n_azimuth + fan->n_elevation;
-        if (plan->fan_angles[slot] < angles) {
+        const size_t angles = fans->n_azimuth + fans->n_elevation;
+        const size_t entries = angles + 6 * fans->n_station; /* in double2 */
+        if (plan->fan_entries[slot] < entries) {
                 if (plan->h_fan[slot] != NULL) cudaFreeHost(plan->h_fan[slot]);
                 cudaFree(plan->d_fan[slot]);
                 plan->h_fan[slot] = NULL;
                 plan->d_fan[slot] = NULL;
-                plan->fan_angles[slot] = 0;
-                cudaError_t err = cudaHostAlloc((void **)&plan->h_fan[slot], angles * sizeof(double2),
+                plan->fan_entries[slot] = 0;
+                cudaError_t err = cudaHostAlloc((void **)&plan->h_fan[slot], entries * sizeof(double2),
                     cudaHostAllocDefault);
                 if (err == cudaSuccess)
-                        err = cudaMalloc((void **)&plan->d_fan[slot], angles * sizeof(double2));
+                        err = cudaMalloc((void **)&plan->d_fan[slot], entries * sizeof(double2));
                 if (err != cudaSuccess) return err;
-                plan->fan_angles[slot] = angles;
+                plan->fan_entries[slot] = entries;
         }
         double2 * h = plan->h_fan[slot];
-        for (size_t i = 0; i < fan->n_azimuth; i++) {
-                const double az = fan->azimuth[i] * M_PI / 180.;
+        for (size_t i = 0; i < fans->n_azimuth; i++) {
+                const double az = fans->azimuth[i] * M_PI / 180.;
                 h[i].x = sin(az);
                 h[i].y = cos(az);
         }
-        for (size_t j = 0; j < fan->n_elevation; j++) {
-                const double el = fan->elevation[j] * M_PI / 180.;
-                h[fan->n_azimuth + j].x = cos(el);
-                h[fan->n_azimuth + j].y = sin(el);
+        for (size_t j = 0; j < fans->n_elevation; j++) {
+                const double el = fans->elevation[j] * M_PI / 180.;
+                h[fans->n_azimuth + j].x = cos(el);
+                h[fans->n_azimuth + j].y = sin(el);
         }
-        const double lambda = fan->longitude * M_PI / 180.;
-        const double phi = fan->latitude * M_PI / 180.;
-        const double sl = sin(lambda), cl = cos(lambda), sp = sin(phi), cp = cos(phi);
-        const double e[3] = { -sl, cl, 0. }, nn[3] = { -cl * sp, -sl * sp, cp };
-        const double u[3] = { cl * cp, sl * cp, sp };
-        for (int c = 0; c < 3; c++) {
-                T->origin[c] = fan->position[c];
-                T->e[c] = e[c];
-                T->n[c] = nn[c];
-                T->u[c] = u[c];
+        double * station = (double *)(h + angles);
+        for (size_t s = 0; s < fans->n_station; s++) {
+                const double lambda = fans->longitude[s] * M_PI / 180.;
+                const double phi = fans->latitude[s] * M_PI / 180.;
+                const double sl = sin(lambda), cl = cos(lambda), sp = sin(phi), cp = cos(phi);
+                const double e[3] = { -sl, cl, 0. }, nn[3] = { -cl * sp, -sl * sp, cp };
+                const double u[3] = { cl * cp, sl * cp, sp };
+                double * f = station + 12 * s;
+                for (int c = 0; c < 3; c++) {
+                        f[c] = fans->position[3 * s + c];
+                        f[3 + c] = e[c];
+                        f[6 + c] = nn[c];
+                        f[9 + c] = u[c];
+                }
         }
         T->az = plan->d_fan[slot];
-        T->el = plan->d_fan[slot] + fan->n_azimuth;
-        T->naz = fan->n_azimuth;
+        T->el = plan->d_fan[slot] + fans->n_azimuth;
+        T->station = (const double *)(plan->d_fan[slot] + angles);
+        T->naz = fans->n_azimuth;
         T->bundle = bundle;
+        T->per_station = fans->n_azimuth * fans->n_elevation;
         T->ray0 = ray0;
-        return cudaMemcpyAsync(plan->d_fan[slot], h, angles * sizeof(double2),
+        return cudaMemcpyAsync(plan->d_fan[slot], h, entries * sizeof(double2),
             cudaMemcpyHostToDevice, stream);
 }
 
@@ -3144,7 +3197,7 @@ static int field_specs(const struct turtle_trace_fields * f, FieldSpec specs[12]
  * chunk, and no lane ever idles between chunks. */
 static enum turtle_return trace_streamed(turtle_function_t * fn, struct turtle_plan * plan,
     size_t n, size_t ray0, const double * position, const double * direction,
-    const struct turtle_fan * fan, size_t bundle, const struct turtle_trace_rule * rule,
+    const struct turtle_fans * fan, size_t bundle, const struct turtle_trace_rule * rule,
     struct turtle_trace_result * results, const struct turtle_trace_fields * fields,
     int chunk_shift)
 {
@@ -3329,7 +3382,7 @@ static enum turtle_return trace_streamed(turtle_function_t * fn, struct turtle_p
 /* A host-pointer call in rounds of at most STREAM_MAX_RAYS rays, which bounds the device
  * staging of a call whatever the size of the batch. */
 static enum turtle_return trace_rounds(turtle_function_t * fn, struct turtle_plan * plan,
-    size_t n, const double * position, const double * direction, const struct turtle_fan * fan,
+    size_t n, const double * position, const double * direction, const struct turtle_fans * fan,
     size_t bundle, const struct turtle_trace_rule * rule, struct turtle_trace_result * results,
     const struct turtle_trace_fields * fields)
 {
@@ -3367,8 +3420,9 @@ static enum turtle_return trace_rounds(turtle_function_t * fn, struct turtle_pla
 }
 
 /* Host-pointer fan: nothing per ray goes in, so there is nothing to stream IN -- the fan is
- * cut in up to 8 slices of consecutive rays (the lowest elevation bands, i.e. the longest
- * rays, first), each a RESIDENT compact kernel followed by the copy of its records / field
+ * cut in up to 8 slices of consecutive rays (in ray order: station by station, the lowest
+ * elevation bands, i.e. the longest rays, first; a slice is made of whole bands and may
+ * begin within a station), each a RESIDENT compact kernel followed by the copy of its records / field
  * slices to the host, alternating on two streams: the copy of a slice runs under the
  * kernel of the next, and the SMs that the tail of one slice leaves idle are taken by the
  * head of the next (concurrent launches on one plan). Only the copy
@@ -3376,7 +3430,7 @@ static enum turtle_return trace_rounds(turtle_function_t * fn, struct turtle_pla
  * watermark -- does the same at 5 % more kernel time; it stays the path of calls that
  * must stream rays in.) */
 static enum turtle_return trace_fan_sliced(turtle_function_t * fn, struct turtle_plan * plan,
-    size_t n, const struct turtle_fan * fan, size_t bundle, const struct turtle_trace_rule * rule,
+    size_t n, const struct turtle_fans * fan, size_t bundle, const struct turtle_trace_rule * rule,
     struct turtle_trace_result * results, const struct turtle_trace_fields * fields)
 {
         CUDA_TRY(fn, plan_pipeline(plan, 1)); /* the streams and their events */
@@ -3471,6 +3525,47 @@ static enum turtle_return trace_fan_sliced(turtle_function_t * fn, struct turtle
         return TURTLE_RETURN_SUCCESS;
 }
 
+/* A device and a plan, for entry points that check their arguments before either is used. */
+static enum turtle_return check_plan(turtle_function_t * fn, const struct turtle_plan * plan)
+{
+        const enum turtle_return rc = require_device(fn, (plan != NULL) ? plan->device : 0);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        if (plan == NULL)
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__, "missing plan");
+        return TURTLE_RETURN_SUCCESS;
+}
+
+/* The n > 0 rays of checked fans, host-pointer results. */
+static enum turtle_return trace_fans_host(turtle_function_t * fn, struct turtle_plan * plan,
+    const struct turtle_fans * fans, size_t n, size_t bundle, const struct turtle_trace_rule * rule,
+    struct turtle_trace_result * results, const struct turtle_trace_fields * fields)
+{
+        CUDA_TRY(fn, cudaSetDevice(plan->device));
+        if (getenv("TURTLE_B200_FAN_STREAMED") != NULL) /* development: the streamed kernel */
+                return trace_rounds(fn, plan, n, NULL, NULL, fans, bundle, rule, results, fields);
+        return trace_fan_sliced(fn, plan, n, fans, bundle, rule, results, fields);
+}
+
+/* The n > 0 rays of checked fans, device-pointer results: ONE launch, asynchronous. */
+static enum turtle_return trace_fans_device(turtle_function_t * fn, struct turtle_plan * plan,
+    const struct turtle_fans * fans, size_t n, size_t bundle, const struct turtle_trace_rule * rule,
+    struct turtle_trace_result * results, const struct turtle_trace_fields * fields, void * stream)
+{
+        CUDA_TRY(fn, cudaSetDevice(plan->device));
+        memset(&plan->counters, 0x0, sizeof(plan->counters));
+        plan->counters.rays = n;
+        int slot;
+        CUDA_TRY(fn, next_device_slot(plan, &slot));
+        FanTables tables;
+        cudaError_t err = fan_upload(plan, slot, fans, bundle, 0, (cudaStream_t)stream, &tables);
+        const DeviceIo io = { NULL, NULL, &tables, results, fields };
+        if (err == cudaSuccess)
+                err = launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
+                    (cudaStream_t)stream);
+        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
+        return TURTLE_RETURN_SUCCESS;
+}
+
 extern "C" enum turtle_return turtle_stepper_trace_fan(struct turtle_plan * plan,
     const struct turtle_fan * fan, const struct turtle_trace_rule * rule,
     struct turtle_trace_result * results, const struct turtle_trace_fields * fields)
@@ -3483,10 +3578,8 @@ extern "C" enum turtle_return turtle_stepper_trace_fan(struct turtle_plan * plan
         if (rc != TURTLE_RETURN_SUCCESS) return rc;
         memset(&plan->counters, 0x0, sizeof(plan->counters));
         if (n == 0) return TURTLE_RETURN_SUCCESS;
-        CUDA_TRY(fn, cudaSetDevice(plan->device));
-        if (getenv("TURTLE_B200_FAN_STREAMED") != NULL) /* development: the streamed kernel */
-                return trace_rounds(fn, plan, n, NULL, NULL, fan, bundle, rule, results, fields);
-        return trace_fan_sliced(fn, plan, n, fan, bundle, rule, results, fields);
+        const struct turtle_fans fans = one_station(fan);
+        return trace_fans_host(fn, plan, &fans, n, bundle, rule, results, fields);
 }
 
 extern "C" enum turtle_return turtle_stepper_trace_fan_device(struct turtle_plan * plan,
@@ -3501,19 +3594,40 @@ extern "C" enum turtle_return turtle_stepper_trace_fan_device(struct turtle_plan
         rc = check_fan(fn, fan, &n, &bundle);
         if (rc != TURTLE_RETURN_SUCCESS) return rc;
         if (n == 0) return TURTLE_RETURN_SUCCESS;
-        CUDA_TRY(fn, cudaSetDevice(plan->device));
+        const struct turtle_fans fans = one_station(fan);
+        return trace_fans_device(fn, plan, &fans, n, bundle, rule, results, fields, stream);
+}
+
+extern "C" enum turtle_return turtle_stepper_trace_fans(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    struct turtle_trace_result * results, const struct turtle_trace_fields * fields)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_trace_fans);
+        enum turtle_return rc = check_rule(fn, rule);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        size_t n, bundle;
+        rc = check_fans(fn, fans, &n, &bundle);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        rc = check_plan(fn, plan);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
         memset(&plan->counters, 0x0, sizeof(plan->counters));
-        plan->counters.rays = n;
-        int slot;
-        CUDA_TRY(fn, next_device_slot(plan, &slot));
-        FanTables tables;
-        cudaError_t err = fan_upload(plan, slot, fan, bundle, 0, (cudaStream_t)stream, &tables);
-        const DeviceIo io = { NULL, NULL, &tables, results, fields };
-        if (err == cudaSuccess)
-                err = launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
-                    (cudaStream_t)stream);
-        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
-        return TURTLE_RETURN_SUCCESS;
+        return trace_fans_host(fn, plan, fans, n, bundle, rule, results, fields);
+}
+
+extern "C" enum turtle_return turtle_stepper_trace_fans_device(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    struct turtle_trace_result * results, const struct turtle_trace_fields * fields,
+    void * stream)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_trace_fans_device);
+        enum turtle_return rc = check_rule(fn, rule);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        size_t n, bundle;
+        rc = check_fans(fn, fans, &n, &bundle);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        rc = check_plan(fn, plan);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        return trace_fans_device(fn, plan, fans, n, bundle, rule, results, fields, stream);
 }
 
 extern "C" enum turtle_return turtle_stepper_trace_fields(struct turtle_plan * plan, size_t n,
@@ -3554,11 +3668,12 @@ extern "C" enum turtle_return turtle_stepper_trace_fields_device(struct turtle_p
 
 /* Arguments first (no plan, no device needed), then the device, then the plan. */
 static enum turtle_return check_horizon(turtle_function_t * fn, const struct turtle_plan * plan,
-    const double * position, size_t n_azimuth, const double * azimuth, double elevation_min,
-    double elevation_max, double tolerance, const struct turtle_trace_rule * rule,
-    const struct turtle_horizon * results)
+    size_t n_station, const double * latitude, const double * longitude, const double * position,
+    size_t n_azimuth, const double * azimuth, double elevation_min, double elevation_max,
+    double tolerance, const struct turtle_trace_rule * rule, const struct turtle_horizon * results)
 {
-        if ((position == NULL) || ((n_azimuth > 0) && ((azimuth == NULL) || (results == NULL))))
+        if ((n_station > 0) && ((latitude == NULL) || (longitude == NULL) || (position == NULL) ||
+                                   ((n_azimuth > 0) && ((azimuth == NULL) || (results == NULL)))))
                 return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
                     "missing station position, azimuths or results");
         if (!(tolerance > 0.))
@@ -3569,46 +3684,39 @@ static enum turtle_return check_horizon(turtle_function_t * fn, const struct tur
                     "invalid elevation window [%g, %g] (must be an interval of [-90, 90])",
                     elevation_min, elevation_max);
         enum turtle_return rc = check_rule(fn, rule);
-        if ((rc != TURTLE_RETURN_SUCCESS) || (n_azimuth == 0)) return rc;
-        rc = require_device(fn, (plan != NULL) ? plan->device : 0);
-        if (rc != TURTLE_RETURN_SUCCESS) return rc;
-        if (plan == NULL)
-                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__, "missing plan");
-        return TURTLE_RETURN_SUCCESS;
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n_station * n_azimuth == 0)) return rc;
+        return check_plan(fn, plan);
 }
 
-/* Queue the search on `stream`: azimuth table (fan_upload), counters, kernel; with the
- * counter block and tables of `slot`. */
-static cudaError_t launch_horizon(struct turtle_plan * plan, int slot, double latitude,
-    double longitude,
-    const double position[3], size_t n_azimuth, const double * azimuth, double elevation_min,
-    double elevation_max, double tolerance, const struct turtle_trace_rule * rule,
-    struct turtle_horizon * results, cudaStream_t stream)
+/* Queue the search on `stream`: azimuth and station tables (fan_upload), counters, kernel;
+ * with the counter block and tables of `slot`. One work item per station and azimuth. */
+static cudaError_t launch_horizon(struct turtle_plan * plan, int slot, size_t n_station,
+    const double * latitude, const double * longitude, const double * position, size_t n_azimuth,
+    const double * azimuth, double elevation_min, double elevation_max, double tolerance,
+    const struct turtle_trace_rule * rule, struct turtle_horizon * results, cudaStream_t stream)
 {
         memset(&plan->counters, 0x0, sizeof(plan->counters));
         unsigned long long * d_counters = plan->d_counters + CTR * slot;
-        struct turtle_fan fan;
-        memset(&fan, 0x0, sizeof fan);
-        fan.latitude = latitude;
-        fan.longitude = longitude;
-        for (int c = 0; c < 3; c++) fan.position[c] = position[c];
-        fan.n_azimuth = n_azimuth;
-        fan.azimuth = azimuth;
+        struct turtle_fans fans;
+        memset(&fans, 0x0, sizeof fans);
+        fans.n_station = n_station;
+        fans.latitude = latitude;
+        fans.longitude = longitude;
+        fans.position = position;
+        fans.n_azimuth = n_azimuth;
+        fans.azimuth = azimuth;
         FanTables T;
-        cudaError_t err = fan_upload(plan, slot, &fan, 1, 0, stream, &T);
+        cudaError_t err = fan_upload(plan, slot, &fans, 1, 0, stream, &T);
         if (err == cudaSuccess)
                 err = cudaMemsetAsync(d_counters, 0x0, CTR * sizeof(unsigned long long), stream);
         if (err != cudaSuccess) return err;
+        const size_t items = n_station * n_azimuth;
         HorizonArgs A;
         memset(&A, 0x0, sizeof A);
         A.az = T.az;
-        A.n = n_azimuth;
-        for (int c = 0; c < 3; c++) {
-                A.origin[c] = T.origin[c];
-                A.e[c] = T.e[c];
-                A.north[c] = T.n[c];
-                A.up[c] = T.u[c];
-        }
+        A.station = T.station;
+        A.n = items;
+        A.n_azimuth = n_azimuth;
         A.elevation_min = elevation_min;
         A.elevation_max = elevation_max;
         A.tolerance = tolerance;
@@ -3623,7 +3731,7 @@ static cudaError_t launch_horizon(struct turtle_plan * plan, int slot, double la
         int blocks, threads;
         const int per_sm = trace_grid(plan, 0, &blocks, &threads);
         const size_t warps = (size_t)threads / 32;
-        blocks = (int)std::min<size_t>((size_t)plan->sm_count * per_sm, (n_azimuth + warps - 1) / warps);
+        blocks = (int)std::min<size_t>((size_t)plan->sm_count * per_sm, (items + warps - 1) / warps);
         const bool lla = plan->G.range > 0.;
         bool proj = false;
         for (int t = 0; t < plan->G.n_transforms; t++)
@@ -3643,23 +3751,54 @@ static cudaError_t launch_horizon(struct turtle_plan * plan, int slot, double la
         return cudaGetLastError();
 }
 
+/* Checked arguments, items > 0: device-pointer results, asynchronous. */
+static enum turtle_return horizons_device(turtle_function_t * fn, struct turtle_plan * plan,
+    size_t n_station, const double * latitude, const double * longitude, const double * position,
+    size_t n_azimuth, const double * azimuth, double elevation_min, double elevation_max,
+    double tolerance, const struct turtle_trace_rule * rule, struct turtle_horizon * results,
+    void * stream)
+{
+        CUDA_TRY(fn, cudaSetDevice(plan->device));
+        int slot;
+        CUDA_TRY(fn, next_device_slot(plan, &slot));
+        const cudaError_t err = launch_horizon(plan, slot, n_station, latitude, longitude, position,
+            n_azimuth, azimuth, elevation_min, elevation_max, tolerance, rule, results,
+            (cudaStream_t)stream);
+        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
+        return TURTLE_RETURN_SUCCESS;
+}
+
+/* Checked arguments, items > 0: host-pointer results. */
+static enum turtle_return horizons_host(turtle_function_t * fn, struct turtle_plan * plan,
+    size_t n_station, const double * latitude, const double * longitude, const double * position,
+    size_t n_azimuth, const double * azimuth, double elevation_min, double elevation_max,
+    double tolerance, const struct turtle_trace_rule * rule, struct turtle_horizon * results)
+{
+        CUDA_TRY(fn, cudaSetDevice(plan->device));
+        struct turtle_horizon * d_results = NULL;
+        const size_t bytes = n_station * n_azimuth * sizeof(*d_results);
+        CUDA_TRY(fn, cudaMalloc((void **)&d_results, bytes));
+        /* a host-pointer call: the counter block and tables of the host pipeline's slot 0 */
+        cudaError_t err = launch_horizon(plan, 0, n_station, latitude, longitude, position,
+            n_azimuth, azimuth, elevation_min, elevation_max, tolerance, rule, d_results, NULL);
+        if (err == cudaSuccess) err = cudaMemcpy(results, d_results, bytes, cudaMemcpyDeviceToHost);
+        cudaFree(d_results);
+        CUDA_TRY(fn, err);
+        read_counters(plan, 0);
+        return TURTLE_RETURN_SUCCESS;
+}
+
 extern "C" enum turtle_return turtle_stepper_horizon_device(struct turtle_plan * plan,
     double latitude, double longitude, const double position[3], size_t n_azimuth,
     const double * azimuth, double elevation_min, double elevation_max, double tolerance,
     const struct turtle_trace_rule * rule, struct turtle_horizon * results, void * stream)
 {
         turtle_function_t * fn = FN(&turtle_stepper_horizon_device);
-        enum turtle_return rc = check_horizon(fn, plan, position, n_azimuth, azimuth,
-            elevation_min, elevation_max, tolerance, rule, results);
+        enum turtle_return rc = check_horizon(fn, plan, 1, &latitude, &longitude, position,
+            n_azimuth, azimuth, elevation_min, elevation_max, tolerance, rule, results);
         if ((rc != TURTLE_RETURN_SUCCESS) || (n_azimuth == 0)) return rc;
-        CUDA_TRY(fn, cudaSetDevice(plan->device));
-        int slot;
-        CUDA_TRY(fn, next_device_slot(plan, &slot));
-        const cudaError_t err = launch_horizon(plan, slot, latitude, longitude, position,
-            n_azimuth, azimuth, elevation_min, elevation_max, tolerance, rule, results,
-            (cudaStream_t)stream);
-        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
-        return TURTLE_RETURN_SUCCESS;
+        return horizons_device(fn, plan, 1, &latitude, &longitude, position, n_azimuth, azimuth,
+            elevation_min, elevation_max, tolerance, rule, results, stream);
 }
 
 extern "C" enum turtle_return turtle_stepper_horizon(struct turtle_plan * plan,
@@ -3668,23 +3807,39 @@ extern "C" enum turtle_return turtle_stepper_horizon(struct turtle_plan * plan,
     const struct turtle_trace_rule * rule, struct turtle_horizon * results)
 {
         turtle_function_t * fn = FN(&turtle_stepper_horizon);
-        enum turtle_return rc = check_horizon(fn, plan, position, n_azimuth, azimuth,
-            elevation_min, elevation_max, tolerance, rule, results);
+        enum turtle_return rc = check_horizon(fn, plan, 1, &latitude, &longitude, position,
+            n_azimuth, azimuth, elevation_min, elevation_max, tolerance, rule, results);
         if ((rc != TURTLE_RETURN_SUCCESS) || (n_azimuth == 0)) return rc;
-        CUDA_TRY(fn, cudaSetDevice(plan->device));
-        struct turtle_horizon * d_results = NULL;
-        const size_t bytes = n_azimuth * sizeof(*d_results);
-        CUDA_TRY(fn, cudaMalloc((void **)&d_results, bytes));
-        /* a host-pointer call: the counter block and tables of the host pipeline's slot 0 */
-        cudaError_t err = launch_horizon(plan, 0, latitude, longitude, position, n_azimuth,
-            azimuth, elevation_min, elevation_max, tolerance, rule, d_results, NULL);
-        if (err == cudaSuccess) err = cudaMemcpy(results, d_results, bytes, cudaMemcpyDeviceToHost);
-        cudaFree(d_results);
-        CUDA_TRY(fn, err);
-        read_counters(plan, 0);
-        return TURTLE_RETURN_SUCCESS;
+        return horizons_host(fn, plan, 1, &latitude, &longitude, position, n_azimuth, azimuth,
+            elevation_min, elevation_max, tolerance, rule, results);
 }
 
+extern "C" enum turtle_return turtle_stepper_horizons_device(struct turtle_plan * plan,
+    size_t n_station, const double * latitude, const double * longitude, const double * position,
+    size_t n_azimuth, const double * azimuth, double elevation_min, double elevation_max,
+    double tolerance, const struct turtle_trace_rule * rule, struct turtle_horizon * results,
+    void * stream)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_horizons_device);
+        enum turtle_return rc = check_horizon(fn, plan, n_station, latitude, longitude, position,
+            n_azimuth, azimuth, elevation_min, elevation_max, tolerance, rule, results);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n_station * n_azimuth == 0)) return rc;
+        return horizons_device(fn, plan, n_station, latitude, longitude, position, n_azimuth,
+            azimuth, elevation_min, elevation_max, tolerance, rule, results, stream);
+}
+
+extern "C" enum turtle_return turtle_stepper_horizons(struct turtle_plan * plan,
+    size_t n_station, const double * latitude, const double * longitude, const double * position,
+    size_t n_azimuth, const double * azimuth, double elevation_min, double elevation_max,
+    double tolerance, const struct turtle_trace_rule * rule, struct turtle_horizon * results)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_horizons);
+        enum turtle_return rc = check_horizon(fn, plan, n_station, latitude, longitude, position,
+            n_azimuth, azimuth, elevation_min, elevation_max, tolerance, rule, results);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n_station * n_azimuth == 0)) return rc;
+        return horizons_host(fn, plan, n_station, latitude, longitude, position, n_azimuth,
+            azimuth, elevation_min, elevation_max, tolerance, rule, results);
+}
 extern "C" enum turtle_return turtle_stepper_trace_batch(
     struct turtle_plan * plan, size_t n, const double * position,
     const double * direction, const struct turtle_trace_rule * rule,
@@ -4748,6 +4903,8 @@ extern "C" const char * tb_batch_function_name(turtle_function_t * caller)
         NAME(turtle_residency_from_rays);
         NAME(turtle_stepper_trace_fan);
         NAME(turtle_stepper_trace_fan_device);
+        NAME(turtle_stepper_trace_fans);
+        NAME(turtle_stepper_trace_fans_device);
         NAME(turtle_stepper_trace_fields);
         NAME(turtle_stepper_trace_fields_device);
         NAME(turtle_plan_gather_set);
@@ -4759,6 +4916,8 @@ extern "C" const char * tb_batch_function_name(turtle_function_t * caller)
         NAME(turtle_stepper_trace_crossings_device);
         NAME(turtle_stepper_horizon);
         NAME(turtle_stepper_horizon_device);
+        NAME(turtle_stepper_horizons);
+        NAME(turtle_stepper_horizons_device);
         NAME(turtle_b200_peer_alloc);
         NAME(turtle_b200_peer_free);
         NAME(turtle_b200_peer_export);
