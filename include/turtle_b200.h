@@ -99,8 +99,8 @@ struct turtle_plan_counters {
 
 /* Threading: a plan carries the streams, staging buffers and counters of the calls made
  * through it, and is used from one host thread at a time. HOST-pointer calls (`*_batch`,
- * `_trace_fan[s]`, `_trace_fields`, `_trace_crossings`, `_horizon[s]`) return when their results are
- * in place: ONE at a time per plan. DEVICE-pointer calls (`*_device`) are asynchronous on the
+ * `_trace_fan[s]`, `_trace_fields`, `_trace_crossings`, `_horizon[s]`, `_trace_[fans_]voxels`)
+ * return when their results are in place: ONE at a time per plan. DEVICE-pointer calls (`*_device`) are asynchronous on the
  * caller's stream: that is how a caller with several batches hides the tail of one (a launch
  * ends when its slowest ray does) behind the head of the next. A device-pointer call is IN
  * FLIGHT from its return until its stream has done all it queued; up to 8 may be in flight on
@@ -109,8 +109,8 @@ struct turtle_plan_counters {
  * fan / azimuth / station tables) until it completes; a ninth call waits on the host until the call
  * that took its slot first is over. Host-pointer calls have slots of their own and may be
  * made while device-pointer calls are in flight; those that stage their arrays in device
- * memory of their own (turtle_stepper_step_batch, _walk_batch, _trace_crossings, _horizon[s])
- * free it before they return, which waits for the device to be idle. After the caller has
+ * memory of their own (turtle_stepper_step_batch, _walk_batch, _trace_crossings, _horizon[s],
+ * _trace_[fans_]voxels) free it before they return, which waits for the device to be idle. After the caller has
  * synchronised, turtle_plan_counters_sync reports the device-pointer call issued last.
  * Several plans (one per host thread or per device) are independent; they share nothing but
  * read-only tiles of their own. This is the batched form of the reference's rule "one
@@ -395,6 +395,76 @@ TURTLE_API enum turtle_return turtle_stepper_trace_crossings_device(
     const double * direction, const struct turtle_trace_rule * rule,
     struct turtle_trace_result * results, struct turtle_trace_crossing * crossings,
     int max_crossings, void * stream);
+
+/* ---- the length of every ray in every cell of a voxel grid: the matrix of a density
+ * inversion ----------------------------------------------------------------------------------
+ * A density inversion solves opacity_i = sum_j L_ij rho_j, where rho_j is the density of cell j
+ * of a grid around the mountain and L_ij the length of ray i inside cell j AND inside the rock.
+ * These calls build L on the device, one sparse row per ray.
+ *
+ * Rays. Ray i is traced exactly as turtle_stepper_trace_batch (or, for the fans form,
+ * turtle_stepper_trace_fans, same ray order and directions) traces it: same steps, same bits.
+ * `results` (may be NULL) receives the very records of the plain call.
+ * Segments. Step k of a ray covers the path lengths [s_{k-1}, s_k] of the ray line
+ * origin + s * direction, where s is the running `total` before and after the step (the
+ * doubles turtle_stepper_trace_crossings reports). A step counts when bit medium0 of
+ * grid->media is set, medium0 being the medium its start sample was in (the rule of
+ * length[m], by true layer index, not folded to TURTLE_TRACE_MEDIA). Its segment is clipped to
+ * the cells of the grid.
+ * Cells. The grid frame has its origin at turtle_ecef_from_geodetic(latitude, longitude, height)
+ * and the East / North / Up vectors of turtle_ecef_from_horizontal at (latitude, longitude).
+ * Cell (ix, iy, iz) is the half-open box [corner + i * size, corner + (i + 1) * size) on each
+ * axis. Cell planes are met at absolute path lengths along the ray line, so the steps do not
+ * move a cell boundary.
+ * Entries. The entries of ray i are entries[i * capacity + k], in order along the ray. A new
+ * entry starts whenever the cell or the medium changes; consecutive pieces in the same (cell,
+ * medium) are summed into one entry, across step boundaries and across stretches in media
+ * that are not selected. No entry has length 0: a (cell, medium) pair appears twice in one ray
+ * only with something else between its appearances.
+ * Count and capacity. count[i] is the number of entries of ray i in all, which may exceed
+ * `capacity`; only the first min(count[i], capacity) are written, the slots after them are
+ * left untouched. With capacity = 0, `entries` may be NULL and the call only counts: a first
+ * pass that sizes an exact buffer. Invalid rays (TURTLE_TRACE_INVALID) and rays without a
+ * selected step in the grid have count 0.
+ * Checks. The arguments are checked before the plan or the device is used. A missing grid or
+ * fans struct, missing positions, directions or counts (n > 0), or entries NULL with
+ * capacity > 0 are TURTLE_RETURN_BAD_ADDRESS. capacity < 0, cell counts <= 0 or of more than
+ * INT32_MAX cells in all, sizes that are not finite and > 0, a non-finite origin or corner, or
+ * media == 0 are TURTLE_RETURN_DOMAIN_ERROR. n = 0 or an empty fan grid does nothing.
+ * Memory. turtle_stepper_trace_voxels and _fans_voxels take HOST memory and return when the
+ * results are in place (the entries are staged in device memory of their own, freed before
+ * the return). The _device variants take DEVICE memory (the fans' arrays stay on the host, as
+ * for turtle_stepper_trace_fans_device), are one asynchronous launch on `stream` and hold one
+ * of the plan's 8 slots. The plan counters report rays, steps and samples as a trace does. */
+struct turtle_voxel_grid {
+        double latitude, longitude, height; /* frame origin, turtle_ecef_from_geodetic(...) */
+        double corner[3];  /* E, N, U coordinates (m) of the lowest corner of the grid */
+        double size[3];    /* cell edges along E, N, U (m), finite and > 0 */
+        int32_t n[3];      /* cells along E, N, U, > 0, n[0] * n[1] * n[2] <= INT32_MAX */
+        uint32_t media;    /* bit m set: steps that START in medium m are split (m < 32), != 0 */
+};
+struct turtle_voxel_entry {        /* 16 bytes */
+        double length;             /* metres of the ray in this cell and medium */
+        int32_t voxel;             /* ix + n[0] * (iy + n[1] * iz) */
+        int32_t medium;            /* medium the steps started in */
+};
+TURTLE_API enum turtle_return turtle_stepper_trace_voxels(struct turtle_plan * plan, size_t n,
+    const double * position, const double * direction, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, struct turtle_trace_result * results,
+    struct turtle_voxel_entry * entries, int capacity, int32_t * count);
+TURTLE_API enum turtle_return turtle_stepper_trace_voxels_device(struct turtle_plan * plan,
+    size_t n, const double * position, const double * direction,
+    const struct turtle_trace_rule * rule, const struct turtle_voxel_grid * grid,
+    struct turtle_trace_result * results, struct turtle_voxel_entry * entries, int capacity,
+    int32_t * count, void * stream);
+TURTLE_API enum turtle_return turtle_stepper_trace_fans_voxels(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, struct turtle_trace_result * results,
+    struct turtle_voxel_entry * entries, int capacity, int32_t * count);
+TURTLE_API enum turtle_return turtle_stepper_trace_fans_voxels_device(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, struct turtle_trace_result * results,
+    struct turtle_voxel_entry * entries, int capacity, int32_t * count, void * stream);
 
 /* ---- one turtle_stepper_step for n independent particles -------------------
  * Same outputs as the scalar call (any output pointer may be NULL; direction

@@ -67,6 +67,19 @@ class Fans(C.Structure):
                 ("elevation", C.c_void_p), ("bundle", C.c_size_t)]
 
 
+class VoxelGrid(C.Structure):
+    """struct turtle_voxel_grid (include/turtle_b200.h): cells in the East / North / Up frame
+    of a point."""
+    _fields_ = [("latitude", C.c_double), ("longitude", C.c_double), ("height", C.c_double),
+                ("corner", C.c_double * 3), ("size", C.c_double * 3), ("n", C.c_int32 * 3),
+                ("media", C.c_uint32)]
+
+
+class VoxelEntry(C.Structure):
+    """struct turtle_voxel_entry (include/turtle_b200.h)."""
+    _fields_ = [("length", C.c_double), ("voxel", C.c_int32), ("medium", C.c_int32)]
+
+
 class PlanCounters(C.Structure):
     """struct turtle_plan_counters (include/turtle_b200.h)."""
     _fields_ = [("rays", C.c_uint64), ("steps", C.c_uint64),
@@ -184,6 +197,14 @@ SIGNATURES = {
     "turtle_stepper_trace_crossings": (_I, [_P, _N, _P, _P, C.POINTER(TraceRule), _P, _P, _I]),
     "turtle_stepper_trace_crossings_device": (_I, [_P, _N, _P, _P, C.POINTER(TraceRule), _P, _P,
                                                    _I, _P]),
+    "turtle_stepper_trace_voxels": (_I, [_P, _N, _P, _P, C.POINTER(TraceRule),
+                                         C.POINTER(VoxelGrid), _P, _P, _I, _P]),
+    "turtle_stepper_trace_voxels_device": (_I, [_P, _N, _P, _P, C.POINTER(TraceRule),
+                                                C.POINTER(VoxelGrid), _P, _P, _I, _P, _P]),
+    "turtle_stepper_trace_fans_voxels": (_I, [_P, C.POINTER(Fans), C.POINTER(TraceRule),
+                                              C.POINTER(VoxelGrid), _P, _P, _I, _P]),
+    "turtle_stepper_trace_fans_voxels_device": (_I, [_P, C.POINTER(Fans), C.POINTER(TraceRule),
+                                                     C.POINTER(VoxelGrid), _P, _P, _I, _P, _P]),
     "turtle_stepper_horizon": (_I, [_P, _D, _D, _P, _N, _P, _D, _D, _D, C.POINTER(TraceRule), _P]),
     "turtle_stepper_horizon_device": (_I, [_P, _D, _D, _P, _N, _P, _D, _D, _D,
                                            C.POINTER(TraceRule), _P, _P]),

@@ -10,7 +10,7 @@ import ctypes as C
 import numpy as np
 
 from ._lib import (ERROR_HANDLER, Fan, Fans, MapInfo, PlanCounters, TraceFields, Residency, ResidencyReport, TraceRule,
-                   lib)
+                   VoxelGrid, lib)
 
 TRACE_RESULT = np.dtype([
     ("position", "<f8", (3,)), ("altitude", "<f8"), ("length", "<f8", (4,)),
@@ -30,6 +30,9 @@ HORIZON_RESULT = np.dtype([
 assert HORIZON_RESULT.itemsize == 96
 
 HORIZON_FOUND, HORIZON_BELOW, HORIZON_ABOVE, HORIZON_INVALID = range(4)
+
+VOXEL_ENTRY = np.dtype([("length", "<f8"), ("voxel", "<i4"), ("medium", "<i4")])
+assert VOXEL_ENTRY.itemsize == 16
 
 
 class TurtleError(RuntimeError):
@@ -369,6 +372,15 @@ def trace_rule(altitude_max, altitude_min=-1.7976931348623157e308,
     return TraceRule(altitude_min, altitude_max, length_max, max_steps, 0)
 
 
+def voxel_grid(latitude, longitude, height, corner, size, n, media):
+    """struct turtle_voxel_grid: n[0] x n[1] x n[2] cells of `size` metres (East, North, Up)
+    from `corner`, in the East / North / Up frame of (latitude, longitude, height). `media`:
+    bit m selects the steps that start in medium m (layer index)."""
+    return VoxelGrid(latitude, longitude, height, (C.c_double * 3)(*map(float, corner)),
+                     (C.c_double * 3)(*map(float, size)), (C.c_int32 * 3)(*map(int, n)),
+                     int(media))
+
+
 class Plan:
     """turtle_plan: a stepper geometry resident on one GPU."""
 
@@ -544,6 +556,51 @@ class Plan:
         _check(lib.turtle_stepper_trace_batch_device(
             self._p, n, _ptr(position), _ptr(direction), C.byref(rule), _ptr(results),
             C.c_void_p(stream) if stream else None))
+
+    # ---- rock length per cell of a voxel grid (turtle_stepper_trace_voxels) ---------------
+    @staticmethod
+    def _voxel_out(n, capacity):
+        return (np.zeros(n, dtype=TRACE_RESULT), np.zeros((n, capacity), dtype=VOXEL_ENTRY),
+                np.zeros(n, dtype=np.int32))
+
+    def trace_voxels(self, position, direction, rule, grid, capacity):
+        """turtle_stepper_trace_voxels: host rays in -> (records, entries [n, capacity]
+        (VOXEL_ENTRY), count [n]). count[i] may exceed capacity: only the first `capacity`
+        entries of such a ray are kept."""
+        position, direction = _f8(position, (-1, 3)), _f8(direction, (-1, 3))
+        n = len(position)
+        results, entries, count = self._voxel_out(n, capacity)
+        _check(lib.turtle_stepper_trace_voxels(
+            self._p, n, _ptr(position), _ptr(direction), C.byref(rule), C.byref(grid),
+            _ptr(results), _ptr(entries) if capacity else None, capacity, _ptr(count)))
+        return results, entries, count
+
+    def trace_voxels_device(self, n, position, direction, rule, grid, capacity, entries, count,
+                            results=None, stream=None):
+        """turtle_stepper_trace_voxels_device: device tensors in / out, asynchronous."""
+        _check(lib.turtle_stepper_trace_voxels_device(
+            self._p, n, _ptr(position), _ptr(direction), C.byref(rule), C.byref(grid),
+            _ptr(results), _ptr(entries), capacity, _ptr(count),
+            C.c_void_p(stream) if stream else None))
+
+    def trace_fans_voxels(self, fans, rule, grid, capacity):
+        """turtle_stepper_trace_fans_voxels: the rays of make_fans(...) -> (records, entries
+        [n, capacity], count [n]), ray order of trace_fans."""
+        f = fans[0]
+        n = f.n_station * f.n_azimuth * f.n_elevation
+        results, entries, count = self._voxel_out(n, capacity)
+        _check(lib.turtle_stepper_trace_fans_voxels(
+            self._p, C.byref(f), C.byref(rule), C.byref(grid), _ptr(results),
+            _ptr(entries) if capacity else None, capacity, _ptr(count)))
+        return results, entries, count
+
+    def trace_fans_voxels_device(self, fans, rule, grid, capacity, entries, count, results=None,
+                                 stream=None):
+        """turtle_stepper_trace_fans_voxels_device: device entries / count / records, one
+        launch, asynchronous."""
+        _check(lib.turtle_stepper_trace_fans_voxels_device(
+            self._p, C.byref(fans[0]), C.byref(rule), C.byref(grid), _ptr(results),
+            _ptr(entries), capacity, _ptr(count), C.c_void_p(stream) if stream else None))
 
     # ---- the horizon of a station (turtle_stepper_horizon) -------------------------------
     def horizon(self, latitude, longitude, position, azimuth, rule, elevation=(-90., 90.),

@@ -1205,6 +1205,478 @@ __global__ void __launch_bounds__(128, MINB)
         }
 }
 
+/* ---- rock length per cell of a voxel grid (turtle_stepper_trace_voxels) --------------------- */
+
+/* Arguments of the voxel kernel: a kernel of its own, like the horizon kernel (members added to
+ * TraceArgs cost every trace kernel registers). */
+struct VoxelArgs {
+        unsigned long long n;
+        const double * position; /* [n][3] with `direction`, or NULL: the rays of `fan` */
+        const double * direction;
+        CompactArgs fan;         /* fan tables (fan_upload), when position == NULL */
+        turtle_trace_result * results; /* or NULL */
+        turtle_voxel_entry * entries;  /* [n][capacity], or NULL when capacity == 0 */
+        int32_t * count;
+        int capacity;
+        unsigned media;
+        double altitude_min, altitude_max, length_max;
+        int max_steps;
+        unsigned long long * cursor; /* [0] next ray, [1] steps, [2] samples, [4] Jacobian columns */
+        double frame[12];            /* origin, East, North, Up of the grid (fan_upload's frame) */
+        double corner[3], size[3];
+        int cells[3];
+};
+
+/* Per-ray rows of the voxel walk, next to the lane store: the ray in grid coordinates, the
+ * path lengths where its line enters and leaves the grid, and the open entry. */
+enum { VF_U0 = 0, VF_V = 3, VF_TIN = 6, VF_TOUT, VF_OPEN, N_VF };
+enum { VI_CELL = 0, VI_MEDIUM, VI_COUNT, N_VI };
+
+/* Path length at which the ray line u0 + s v meets plane k of axis a of the grid. */
+__device__ __forceinline__ double voxel_plane(const VoxelArgs & A, int a, int k, double u0, double v)
+{
+        return (A.corner[a] + (double)k * A.size[a] - u0) / v;
+}
+
+/* Close the open entry of a lane: store it if it fits, count it. */
+__device__ __forceinline__ void voxel_close(const VoxelArgs & A, unsigned long long ray, int cell,
+    int medium, double length, int & count)
+{
+        if (cell < 0) return;
+        if (count < A.capacity) {
+                turtle_voxel_entry * e = A.entries + ray * (unsigned long long)A.capacity + count;
+                e->length = length;
+                e->voxel = cell;
+                e->medium = medium;
+        }
+        count++;
+}
+
+/* trace_kernel's rays (same samples, steps and bits, same queue and settle point), where the
+ * length of every step that starts in a selected medium is split over the cells of the grid
+ * by a 3-D DDA along the ray line, with cell planes at absolute path lengths. */
+template <bool LLA, bool PROJ, int MINB, int SHAPE>
+__global__ void __launch_bounds__(128, MINB)
+    voxel_kernel(const __grid_constant__ tb::Geometry G, const __grid_constant__ VoxelArgs A)
+{
+        constexpr int NF = LLA ? N_F_LLA : N_F_BASE, NI = LLA ? N_I : N_I_BASE;
+        __shared__ LaneStoreT<NF, NI> store;
+        __shared__ double vf[N_VF][128];
+        __shared__ int vi[N_VI][128];
+        const unsigned tid = threadIdx.x;
+        const unsigned lane = tid & 31u;
+        const unsigned FULL = 0xffffffffu;
+#define SF(k) store.f[((k) < NF) ? (k) : 0][tid]
+#define SI(k) store.i[((k) < NI) ? (k) : 0][tid]
+        extern __shared__ double lla_store[];
+        const tb::LlaShared V = { lla_store + tid };
+        unsigned my_steps = 0u, my_samples = 0u, my_rebuilds = 0u;
+        int mode = MODE_IDLE;
+        bool exhausted = false;
+
+        for (;;) {
+                /* ---- write out finished records, twelve lanes side by side (trace_kernel) ---- */
+                unsigned done_mask = __ballot_sync(FULL, mode == MODE_DONE);
+                if (done_mask != 0u) __syncwarp();
+                const bool wrote = done_mask != 0u;
+                while (done_mask != 0u) {
+                        const unsigned src = (unsigned)__ffs((int)done_mask) - 1u;
+                        done_mask &= done_mask - 1u;
+                        const unsigned t = (tid & ~31u) + src;
+                        const unsigned long long ray =
+                            ((unsigned long long)(unsigned)store.i[I_RAYHI][t] << 32) |
+                            (unsigned long long)(unsigned)store.i[I_RAYLO][t];
+                        if ((lane < 12u) && (A.results != NULL)) {
+                                unsigned long long bits;
+                                if (lane < 9u) {
+                                        const int row = (lane < 3u) ? (int)(F_POS + lane) :
+                                            ((lane == 3u) ? (int)F_ALT :
+                                                ((lane < 8u) ? (int)(F_LEN + lane - 4u) : (int)F_TOTAL));
+                                        bits = (unsigned long long)__double_as_longlong(store.f[row][t]);
+                                } else {
+                                        const int lo = (lane == 9u) ? I_NSTEPS : ((lane == 10u) ? I_IDX0 : I_HASH);
+                                        const int hi = (lane == 9u) ? I_MEDIUM0 : ((lane == 10u) ? I_IDX1 : I_NCHANGES);
+                                        bits = ((unsigned long long)(unsigned)store.i[hi][t] << 32) |
+                                            (unsigned long long)(unsigned)store.i[lo][t];
+                                }
+                                reinterpret_cast<unsigned long long *>(A.results + ray)[lane] = bits;
+                        }
+                        if (lane == src) {
+                                A.count[ray] = vi[VI_COUNT][tid];
+                                mode = MODE_IDLE;
+                        }
+                }
+                if (wrote) __syncwarp();
+                /* ---- refill idle lanes from the ray queue (every ray is resident) ---- */
+                const unsigned idle = __ballot_sync(FULL, mode == MODE_IDLE);
+                if (idle != 0u) {
+                        if (!exhausted) {
+                                const int need = __popc(idle);
+                                unsigned long long base = 0ull;
+                                if (lane == 0u) base = atomicAdd(A.cursor, (unsigned long long)need);
+                                base = __shfl_sync(FULL, base, 0);
+                                if (mode == MODE_IDLE) {
+                                        const unsigned long long r =
+                                            base + __popc(idle & ((1u << lane) - 1u));
+                                        if (r < A.n) {
+                                                double pos[3], dir[3];
+                                                if (A.position == NULL) {
+                                                        fan_ray(A.fan, r, pos, dir);
+                                                } else {
+#pragma unroll
+                                                        for (int c = 0; c < 3; c++) {
+                                                                pos[c] = __ldg(A.position + 3ull * r + c);
+                                                                dir[c] = __ldg(A.direction + 3ull * r + c);
+                                                        }
+                                                }
+                                                for (int c = 0; c < 3; c++) {
+                                                        SF(F_POS + c) = pos[c];
+                                                        SF(F_DIR + c) = dir[c];
+                                                }
+#pragma unroll
+                                                for (int m = 0; m < TURTLE_TRACE_MEDIA; m++)
+                                                        SF(F_LEN + m) = 0.;
+                                                SF(F_TOTAL) = 0.;
+                                                SI(I_NSTEPS) = 0;
+                                                SI(I_NCHANGES) = 0;
+                                                SI(I_RAYLO) = (int)(unsigned)(r & 0xffffffffull);
+                                                SI(I_RAYHI) = (int)(unsigned)(r >> 32);
+                                                vi[VI_CELL][tid] = -1;
+                                                vi[VI_COUNT][tid] = 0;
+                                                /* the ray in grid coordinates, and where its line
+                                                 * enters and leaves the grid (+inf: never) */
+                                                double t_in = -DBL_MAX, t_out = DBL_MAX;
+                                                for (int a = 0; a < 3; a++) {
+                                                        const double * e = A.frame + 3 + 3 * a;
+                                                        const double u0 = e[0] * (pos[0] - A.frame[0]) +
+                                                            e[1] * (pos[1] - A.frame[1]) + e[2] * (pos[2] - A.frame[2]);
+                                                        const double v = e[0] * dir[0] + e[1] * dir[1] + e[2] * dir[2];
+                                                        vf[VF_U0 + a][tid] = u0;
+                                                        vf[VF_V + a][tid] = v;
+                                                        if (v != 0.) {
+                                                                const double t0 = voxel_plane(A, a, 0, u0, v);
+                                                                const double t1 = voxel_plane(A, a, A.cells[a], u0, v);
+                                                                t_in = fmax(t_in, fmin(t0, t1));
+                                                                t_out = fmin(t_out, fmax(t0, t1));
+                                                        } else {
+                                                                const double i = floor((u0 - A.corner[a]) / A.size[a]);
+                                                                if (!((i >= 0.) && (i < (double)A.cells[a]))) t_in = DBL_MAX;
+                                                        }
+                                                }
+                                                vf[VF_TIN][tid] = t_in;
+                                                vf[VF_TOUT][tid] = t_out;
+                                                mode = MODE_INIT;
+                                                if (LLA) { /* a reset stepper (stepper.c:647-651) */
+                                                        SI(I_PEND) = 0;
+                                                        SF(F_LASTPOS) = SF(F_LASTPOS + 1) =
+                                                            SF(F_LASTPOS + 2) = DBL_MAX;
+                                                        tb::lla_reset(G, V);
+                                                }
+                                                if (!finite3(pos) || !finite3(dir)) {
+                                                        SF(F_ALT) = 0.;
+                                                        SI(I_IDX0) = -1;
+                                                        SI(I_IDX1) = -1;
+                                                        SI(I_HASH) = 0;
+                                                        SI(I_MEDIUM0) = TURTLE_TRACE_INVALID;
+                                                        mode = MODE_DONE;
+                                                }
+                                        }
+                                }
+                                if (base + (unsigned long long)need >= A.n) exhausted = true;
+                        }
+                        if (__all_sync(FULL, mode == MODE_IDLE)) {
+                                if (exhausted) break;
+                                continue;
+                        }
+                }
+                if ((mode == MODE_IDLE) || (mode == MODE_DONE)) continue;
+
+                /* ---- one sample per lane: as in trace_kernel ---- */
+                tb::Sample S;
+                double moved[3] = { 0., 0., 0. };
+                if (SHAPE == tb::SHAPE_STACK) {
+                        double p[3] = { SF(F_POS), SF(F_POS + 1), SF(F_POS + 2) };
+                        if (mode != MODE_INIT) {
+                                const double step = (mode == MODE_TENT) ?
+                                    SF(F_DS) : 0.5 * (SF(F_DS0) + SF(F_DS1));
+                                p[0] += SF(F_DIR) * step;
+                                p[1] += SF(F_DIR + 1) * step;
+                                p[2] += SF(F_DIR + 2) * step;
+                        }
+                        tb::sample_single_stack(tb::NodesGlobal(), G, p, S);
+                        moved[0] = p[0];
+                        moved[1] = p[1];
+                        moved[2] = p[2];
+                } else {
+                        double p[3];
+                        int rb_t = 0, rb_axis = 0;
+                        bool heavy = true;
+                        unsigned in_range = 0u;
+                        if (!LLA || (mode != MODE_REBUILD)) {
+                                double step = 0.;
+                                if (mode == MODE_TENT)
+                                        step = SF(F_DS);
+                                else if (mode == MODE_BISECT)
+                                        step = 0.5 * (SF(F_DS0) + SF(F_DS1));
+                                p[0] = SF(F_POS);
+                                p[1] = SF(F_POS + 1);
+                                p[2] = SF(F_POS + 2);
+                                if (mode != MODE_INIT) {
+                                        p[0] += SF(F_DIR) * step;
+                                        p[1] += SF(F_DIR + 1) * step;
+                                        p[2] += SF(F_DIR + 2) * step;
+                                }
+                                if (LLA) {
+                                        in_range = tb::lla_range_mask(G, V, p);
+                                        const unsigned due = in_range & (unsigned)SI(I_PEND);
+                                        if (due != 0u) {
+                                                SI(I_RESUME) = mode;
+                                                SI(I_RB_MASK) = (int)due;
+                                                SI(I_RB_AXIS) = 0;
+                                                mode = MODE_REBUILD;
+                                        }
+                                }
+                        }
+                        if (LLA && (mode == MODE_REBUILD)) {
+                                rb_t = __ffs(SI(I_RB_MASK)) - 1;
+                                rb_axis = SI(I_RB_AXIS);
+                                const int row0 = G.lla_row[rb_t];
+                                p[0] = tb::lla_at(V, row0);
+                                p[1] = tb::lla_at(V, row0 + 1);
+                                p[2] = tb::lla_at(V, row0 + 2);
+                                if (rb_axis == 0) p[0] += 10.;
+                                else if (rb_axis == 1) p[1] += 10.;
+                                else p[2] += 10.;
+                        } else if (LLA) {
+                                heavy = !((in_range >> G.lla_first) & 1u);
+                        }
+                        double pre[3] = { 0., 0., 0. };
+                        if (heavy) tb::geodetic_with_geoid(G, p, pre);
+                        if (LLA && (mode == MODE_REBUILD)) {
+                                tb::rebuild_column<PROJ>(G, V, rb_t, rb_axis, pre);
+                                my_rebuilds++;
+                                if (rb_axis == 2) {
+                                        SI(I_RB_MASK) &= ~(1 << rb_t);
+                                        SI(I_PEND) &= ~(1 << rb_t);
+                                        SI(I_RB_AXIS) = 0;
+                                        if (SI(I_RB_MASK) == 0) mode = SI(I_RESUME);
+                                } else {
+                                        SI(I_RB_AXIS) = rb_axis + 1;
+                                }
+                                continue;
+                        }
+                        double last_pos[3] = { 0., 0., 0. };
+                        unsigned stale = 0u;
+                        if (LLA) {
+                                last_pos[0] = SF(F_LASTPOS);
+                                last_pos[1] = SF(F_LASTPOS + 1);
+                                last_pos[2] = SF(F_LASTPOS + 2);
+                                stale = (unsigned)SI(I_PEND);
+                        }
+                        tb::sample_geometry<LLA, PROJ, true>(G, V, stale, last_pos,
+                            mode != MODE_BISECT, p, S, heavy ? pre : NULL, in_range);
+                        if (LLA) {
+                                SI(I_PEND) = (int)stale;
+                                if (mode != MODE_BISECT) {
+                                        SF(F_LASTPOS) = last_pos[0];
+                                        SF(F_LASTPOS + 1) = last_pos[1];
+                                        SF(F_LASTPOS + 2) = last_pos[2];
+                                }
+                        }
+                }
+                compiler_fence();
+                my_samples++;
+
+                /* ---- state update: trace_kernel's ---- */
+                bool settle = false;
+                bool publish = false;
+                const int medium0 = SI(I_MEDIUM0);
+                double ds = SF(F_DS);
+                if (mode == MODE_INIT) {
+                        publish = true;
+                        SI(I_HASH) = (int)((2166136261u ^ (unsigned)(S.idx0 + 1)) * 16777619u);
+                        settle = true;
+                } else if (mode == MODE_TENT) {
+                        if (SHAPE == tb::SHAPE_STACK) {
+                                SF(F_POS) = moved[0];
+                                SF(F_POS + 1) = moved[1];
+                                SF(F_POS + 2) = moved[2];
+                        } else {
+                                SF(F_POS) += SF(F_DIR) * ds;
+                                SF(F_POS + 1) += SF(F_DIR + 1) * ds;
+                                SF(F_POS + 2) += SF(F_DIR + 2) * ds;
+                        }
+                        publish = true;
+                        if (S.idx0 != medium0) {
+                                SF(F_DS0) = -ds;
+                                SF(F_DS1) = 0.;
+                                mode = MODE_BISECT;
+                                settle = !(0. - (-ds) > 1E-08);
+                        } else {
+                                settle = true;
+                        }
+                } else {
+                        double ds0 = SF(F_DS0), ds1 = SF(F_DS1);
+                        const double ds2 = 0.5 * (ds0 + ds1);
+                        if (S.idx0 == medium0) {
+                                ds0 = ds2;
+                                SF(F_DS0) = ds0;
+                        } else {
+                                ds1 = ds2;
+                                SF(F_DS1) = ds1;
+                                publish = true;
+                                if (LLA) {
+                                        SF(F_LASTPOS) = SF(F_POS) + SF(F_DIR) * ds2;
+                                        SF(F_LASTPOS + 1) = SF(F_POS + 1) + SF(F_DIR + 1) * ds2;
+                                        SF(F_LASTPOS + 2) = SF(F_POS + 2) + SF(F_DIR + 2) * ds2;
+                                }
+                        }
+                        if (!(ds1 - ds0 > 1E-08)) {
+                                ds += ds1;
+                                SF(F_POS) += SF(F_DIR) * ds1;
+                                SF(F_POS + 1) += SF(F_DIR + 1) * ds1;
+                                SF(F_POS + 2) += SF(F_DIR + 2) * ds1;
+                                settle = true;
+                        }
+                }
+                if (publish) {
+                        SF(F_ALT) = S.alt;
+                        SF(F_ELEV0) = S.elev0;
+                        SF(F_ELEV1) = S.elev1;
+                        SI(I_IDX0) = S.idx0;
+                        SI(I_IDX1) = S.idx1;
+                }
+                if (!settle) continue;
+
+                tb::Sample last;
+                last.lat = last.lon = 0.;
+                last.alt = publish ? S.alt : SF(F_ALT);
+                last.elev0 = publish ? S.elev0 : SF(F_ELEV0);
+                last.elev1 = publish ? S.elev1 : SF(F_ELEV1);
+                last.idx0 = publish ? S.idx0 : SI(I_IDX0);
+                last.idx1 = publish ? S.idx1 : SI(I_IDX1);
+                double total = SF(F_TOTAL);
+                int n_steps = SI(I_NSTEPS);
+                const unsigned long long ray =
+                    ((unsigned long long)(unsigned)SI(I_RAYHI) << 32) | (unsigned long long)(unsigned)SI(I_RAYLO);
+                if (mode != MODE_INIT) {
+                        const int m = (medium0 < TURTLE_TRACE_MEDIA - 1) ? medium0 :
+                                                                           TURTLE_TRACE_MEDIA - 1;
+                        store.f[F_LEN + m][tid] += ds;
+                        const double s0 = total; /* the step covers [s0, total] of the ray line */
+                        total += ds;
+                        SF(F_TOTAL) = total;
+                        n_steps++;
+                        SI(I_NSTEPS) = n_steps;
+                        my_steps++;
+                        if (last.idx0 != medium0) {
+                                SI(I_NCHANGES) += 1;
+                                SI(I_HASH) = (int)(((unsigned)SI(I_HASH) ^
+                                                       (unsigned)(last.idx0 + 1)) * 16777619u);
+                        }
+                        /* ---- the step's segment through the grid ---- */
+                        double s = fmax(s0, vf[VF_TIN][tid]);
+                        const double s_end = fmin(total, vf[VF_TOUT][tid]);
+                        if (((unsigned)medium0 < 32u) && ((A.media >> medium0) & 1u) && (s < s_end)) {
+                                int i[3];
+                                double next[3];
+                                for (int a = 0; a < 3; a++) {
+                                        const double u0 = vf[VF_U0 + a][tid], v = vf[VF_V + a][tid];
+                                        const int n = A.cells[a];
+                                        /* the cell just after s, with the plane crossings as
+                                         * the truth: a first guess from the position, then
+                                         * moved until t(i) <= s < t(i + 1) (v > 0), or
+                                         * t(i + 1) <= s < t(i) (v < 0) */
+                                        const double g = floor((u0 + s * v - A.corner[a]) / A.size[a]);
+                                        int k = (g < 0.) ? 0 : ((g > (double)(n - 1)) ? n - 1 : (int)g);
+                                        if (v > 0.) {
+                                                while ((k + 1 < n) && (voxel_plane(A, a, k + 1, u0, v) <= s)) k++;
+                                                while ((k > 0) && (voxel_plane(A, a, k, u0, v) > s)) k--;
+                                                next[a] = voxel_plane(A, a, k + 1, u0, v);
+                                        } else if (v < 0.) {
+                                                while ((k > 0) && (voxel_plane(A, a, k, u0, v) <= s)) k--;
+                                                while ((k + 1 < n) && (voxel_plane(A, a, k + 1, u0, v) > s)) k++;
+                                                next[a] = voxel_plane(A, a, k, u0, v);
+                                        } else {
+                                                next[a] = DBL_MAX;
+                                        }
+                                        i[a] = k;
+                                }
+                                int open_cell = vi[VI_CELL][tid], open_medium = vi[VI_MEDIUM][tid];
+                                int count = vi[VI_COUNT][tid];
+                                double open_length = vf[VF_OPEN][tid];
+                                for (;;) {
+                                        const double t = fmin(next[0], fmin(next[1], next[2]));
+                                        const double e = fmin(t, s_end);
+                                        if (e > s) {
+                                                const int cell = i[0] + A.cells[0] * (i[1] + A.cells[1] * i[2]);
+                                                if ((cell == open_cell) && (medium0 == open_medium)) {
+                                                        open_length += e - s;
+                                                } else {
+                                                        voxel_close(A, ray, open_cell, open_medium, open_length, count);
+                                                        open_cell = cell;
+                                                        open_medium = medium0;
+                                                        open_length = e - s;
+                                                }
+                                                s = e;
+                                        }
+                                        if (!(t < s_end)) break;
+                                        /* every axis whose plane comes now: one cell on */
+                                        bool out = false;
+                                        for (int a = 0; a < 3; a++) {
+                                                if (next[a] != t) continue;
+                                                const double u0 = vf[VF_U0 + a][tid], v = vf[VF_V + a][tid];
+                                                i[a] += (v > 0.) ? 1 : -1;
+                                                if ((i[a] < 0) || (i[a] >= A.cells[a])) out = true;
+                                                else next[a] = voxel_plane(A, a, (v > 0.) ? i[a] + 1 : i[a], u0, v);
+                                        }
+                                        if (out) break;
+                                }
+                                vi[VI_CELL][tid] = open_cell;
+                                vi[VI_MEDIUM][tid] = open_medium;
+                                vi[VI_COUNT][tid] = count;
+                                vf[VF_OPEN][tid] = open_length;
+                        }
+                }
+
+                int status = -1;
+                if (last.idx0 < 0)
+                        status = TURTLE_TRACE_DOMAIN;
+                else if (!(last.alt < A.altitude_max) || !(last.alt > A.altitude_min))
+                        status = TURTLE_TRACE_ALTITUDE;
+                else if (total >= A.length_max)
+                        status = TURTLE_TRACE_LENGTH;
+                else if (n_steps >= A.max_steps)
+                        status = TURTLE_TRACE_STEPS;
+
+                if (status >= 0) {
+                        SI(I_MEDIUM0) = status;
+                        int count = vi[VI_COUNT][tid];
+                        voxel_close(A, ray, vi[VI_CELL][tid], vi[VI_MEDIUM][tid], vf[VF_OPEN][tid], count);
+                        vi[VI_COUNT][tid] = count;
+                        mode = MODE_DONE;
+                } else {
+                        SI(I_MEDIUM0) = last.idx0;
+                        SF(F_DS) = tb::step_length(G, last);
+                        mode = MODE_TENT;
+                }
+        }
+#undef SF
+#undef SI
+
+        unsigned long long steps64 = my_steps, samples64 = my_samples, rebuilds64 = my_rebuilds;
+        for (int o = 16; o > 0; o >>= 1) {
+                steps64 += __shfl_down_sync(FULL, steps64, o);
+                samples64 += __shfl_down_sync(FULL, samples64, o);
+                if (LLA) rebuilds64 += __shfl_down_sync(FULL, rebuilds64, o);
+        }
+        if (lane == 0u) {
+                atomicAdd(A.cursor + 1, steps64);
+                atomicAdd(A.cursor + 2, samples64);
+                if (LLA) atomicAdd(A.cursor + 4, rebuilds64);
+        }
+}
+
 /* Longest-expected-first scheduling: the number of steps of a ray grows as it runs
  * closer to the horizontal (it stays near the ground), and the kernel time is bounded
  * below by the LATEST-starting long ray. Key = |sin(elevation)| w.r.t. the geocentric
@@ -3099,10 +3571,26 @@ static struct turtle_fans one_station(const struct turtle_fan * fan)
         return fans;
 }
 
+/* The East / North / Up vectors at (latitude, longitude) (compute_enu, ecef.c:136-158):
+ * f[3..5], f[6..8], f[9..11]. */
+static void enu_frame(double latitude, double longitude, double f[12])
+{
+        const double lambda = longitude * M_PI / 180.;
+        const double phi = latitude * M_PI / 180.;
+        const double sl = sin(lambda), cl = cos(lambda), sp = sin(phi), cp = cos(phi);
+        const double e[3] = { -sl, cl, 0. }, nn[3] = { -cl * sp, -sl * sp, cp };
+        const double u[3] = { cl * cp, sl * cp, sp };
+        for (int c = 0; c < 3; c++) {
+                f[3 + c] = e[c];
+                f[6 + c] = nn[c];
+                f[9 + c] = u[c];
+        }
+}
+
 /* Sines and cosines of the angles of the fans, taken on the host by the calls of
  * turtle_ecef_from_horizontal (ecef.c:139-144,170-173), then the origin and the East / North
- * / Up frame of every station (compute_enu, ecef.c:136-158), 12 doubles each; ONE table per
- * slot, queued for upload on `stream`. */
+ * / Up frame of every station (enu_frame), 12 doubles each; ONE table per slot, queued for
+ * upload on `stream`. */
 static cudaError_t fan_upload(struct turtle_plan * plan, int slot, const struct turtle_fans * fans,
     size_t bundle, size_t ray0, cudaStream_t stream, FanTables * T)
 {
@@ -3134,18 +3622,9 @@ static cudaError_t fan_upload(struct turtle_plan * plan, int slot, const struct 
         }
         double * station = (double *)(h + angles);
         for (size_t s = 0; s < fans->n_station; s++) {
-                const double lambda = fans->longitude[s] * M_PI / 180.;
-                const double phi = fans->latitude[s] * M_PI / 180.;
-                const double sl = sin(lambda), cl = cos(lambda), sp = sin(phi), cp = cos(phi);
-                const double e[3] = { -sl, cl, 0. }, nn[3] = { -cl * sp, -sl * sp, cp };
-                const double u[3] = { cl * cp, sl * cp, sp };
                 double * f = station + 12 * s;
-                for (int c = 0; c < 3; c++) {
-                        f[c] = fans->position[3 * s + c];
-                        f[3 + c] = e[c];
-                        f[6 + c] = nn[c];
-                        f[9 + c] = u[c];
-                }
+                enu_frame(fans->latitude[s], fans->longitude[s], f);
+                for (int c = 0; c < 3; c++) f[c] = fans->position[3 * s + c];
         }
         T->az = plan->d_fan[slot];
         T->el = plan->d_fan[slot] + fans->n_azimuth;
@@ -4161,6 +4640,244 @@ extern "C" enum turtle_return turtle_stepper_trace_crossings(
         return TURTLE_RETURN_SUCCESS;
 }
 
+/* ---- rock length per cell of a voxel grid ------------------------------------------------ */
+
+/* Arguments first (no plan, no device needed). `rays`: the position and direction arrays of
+ * the explicit form are needed (n > 0, not a fan). */
+static enum turtle_return check_voxels(turtle_function_t * fn, size_t n, bool rays,
+    const double * position, const double * direction, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, const struct turtle_voxel_entry * entries,
+    int capacity, const int32_t * count)
+{
+        if (grid == NULL)
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
+                    "missing voxel grid");
+        if ((n > 0) && ((rays && ((position == NULL) || (direction == NULL))) || (count == NULL)))
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
+                    "missing ray positions, directions or counts");
+        if ((capacity > 0) && (entries == NULL))
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
+                    "missing voxel entries (capacity %d)", capacity);
+        if (capacity < 0)
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "invalid voxel capacity %d (must be >= 0)", capacity);
+        const int32_t * c = grid->n;
+        if ((c[0] <= 0) || (c[1] <= 0) || (c[2] <= 0) ||
+            ((long long)c[0] * (long long)c[1] * (long long)c[2] > (long long)INT32_MAX))
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "invalid voxel grid of %d x %d x %d cells (must be > 0, at most %d in all)",
+                    c[0], c[1], c[2], INT32_MAX);
+        const double * s = grid->size;
+        if (!(isfinite(s[0]) && (s[0] > 0.) && isfinite(s[1]) && (s[1] > 0.) && isfinite(s[2]) &&
+                (s[2] > 0.)))
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "invalid voxel size %g x %g x %g m (must be finite and > 0)", s[0], s[1], s[2]);
+        if (!(isfinite(grid->latitude) && isfinite(grid->longitude) && isfinite(grid->height) &&
+                isfinite(grid->corner[0]) && isfinite(grid->corner[1]) && isfinite(grid->corner[2])))
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "invalid voxel grid origin or corner (must be finite)");
+        if (grid->media == 0u)
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "invalid voxel media 0 (select at least one medium)");
+        return check_rule(fn, rule);
+}
+
+/* Queue the voxel kernel on `stream` with the counter block of `slot`: the rays of
+ * `d_position` / `d_direction` (device memory), or of the fan tables `fan`. */
+static cudaError_t launch_voxels(struct turtle_plan * plan, int slot, size_t n,
+    const double * d_position, const double * d_direction, const FanTables * fan,
+    const struct turtle_trace_rule * rule, const struct turtle_voxel_grid * grid,
+    struct turtle_trace_result * results, struct turtle_voxel_entry * entries, int capacity,
+    int32_t * count, cudaStream_t stream)
+{
+        unsigned long long * d_counters = plan->d_counters + CTR * slot;
+        cudaError_t err = cudaMemsetAsync(d_counters, 0x0, CTR * sizeof(unsigned long long), stream);
+        if (err != cudaSuccess) return err;
+        VoxelArgs A;
+        memset(&A, 0x0, sizeof A);
+        A.n = n;
+        A.position = d_position;
+        A.direction = d_direction;
+        if (fan != NULL) {
+                A.position = A.direction = NULL;
+                A.fan.fan_az = fan->az;
+                A.fan.fan_el = fan->el;
+                A.fan.fan_station = fan->station;
+                A.fan.fan_naz = fan->naz;
+                A.fan.fan_bundle = fan->bundle;
+                A.fan.fan_per_station = fan->per_station;
+                A.fan.fan_ray0 = fan->ray0;
+        }
+        A.results = results;
+        A.entries = entries;
+        A.count = count;
+        A.capacity = capacity;
+        A.media = grid->media;
+        A.altitude_min = rule->altitude_min;
+        A.altitude_max = rule->altitude_max;
+        A.length_max = rule->length_max;
+        A.max_steps = rule->max_steps;
+        A.cursor = d_counters;
+        turtle_ecef_from_geodetic(grid->latitude, grid->longitude, grid->height, A.frame);
+        enu_frame(grid->latitude, grid->longitude, A.frame);
+        for (int a = 0; a < 3; a++) {
+                A.corner[a] = grid->corner[a];
+                A.size[a] = grid->size[a];
+                A.cells[a] = grid->n[a];
+        }
+        const bool lla = plan->G.range > 0.;
+        bool proj = false;
+        for (int t = 0; t < plan->G.n_transforms; t++)
+                if (plan->G.transforms[t].type != tb::PROJ_GEODETIC) proj = true;
+        const bool stack_shape = plan->specialise && (tb::geometry_shape(plan->G) == tb::SHAPE_STACK);
+        void (*kernel)(const tb::Geometry, const VoxelArgs) =
+            stack_shape ? voxel_kernel<false, false, 6, tb::SHAPE_STACK> :
+            (lla && proj) ? voxel_kernel<true, true, 4, tb::SHAPE_GENERIC> :
+            lla ? voxel_kernel<true, false, 4, tb::SHAPE_GENERIC> :
+            proj ? voxel_kernel<false, true, 6, tb::SHAPE_GENERIC> :
+                   voxel_kernel<false, false, 6, tb::SHAPE_GENERIC>;
+        const size_t dynamic = lla ? lla_bytes(plan) : 0;
+        if (dynamic > 0)
+                cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dynamic);
+        /* the grid of the trace kernels, at most the CTAs that fit an SM with the rows of the
+         * walk next to the lane store */
+        int blocks, threads;
+        int per_sm = trace_grid(plan, n, &blocks, &threads);
+        int fit = 0;
+        err = cudaOccupancyMaxActiveBlocksPerMultiprocessor(&fit, kernel, threads, dynamic);
+        if (err != cudaSuccess) return err;
+        if (per_sm > fit) per_sm = (fit > 0) ? fit : 1;
+        blocks = std::min(blocks, plan->sm_count * per_sm);
+        kernel<<<blocks, threads, dynamic, stream>>>(plan->G, A);
+        plan->counters.launches++;
+        return cudaGetLastError();
+}
+
+/* Checked arguments, n > 0: host memory, results in place on return. `fans` NULL: the rays of
+ * position / direction. */
+static enum turtle_return voxels_host(turtle_function_t * fn, struct turtle_plan * plan, size_t n,
+    const double * position, const double * direction, const struct turtle_fans * fans,
+    size_t bundle, const struct turtle_trace_rule * rule, const struct turtle_voxel_grid * grid,
+    struct turtle_trace_result * results, struct turtle_voxel_entry * entries, int capacity,
+    int32_t * count)
+{
+        CUDA_TRY(fn, cudaSetDevice(plan->device));
+        DeviceBuffers buf;
+        double *d_pos = NULL, *d_dir = NULL;
+        turtle_trace_result * d_res;
+        turtle_voxel_entry * d_entries = NULL;
+        int32_t * d_count;
+        const size_t entry_bytes = n * (size_t)capacity * sizeof(turtle_voxel_entry);
+        if (fans == NULL) {
+                DEV_IN(fn, buf, d_pos, position, n * 3 * sizeof(double));
+                DEV_IN(fn, buf, d_dir, direction, n * 3 * sizeof(double));
+        }
+        DEV_OUT(fn, buf, d_res, results, n * sizeof(*d_res));
+        /* the caller's slots past each count stay as they are: staged in, copied back whole */
+        if (capacity > 0) DEV_IN(fn, buf, d_entries, entries, entry_bytes);
+        DEV_OUT(fn, buf, d_count, count, n * sizeof(*d_count));
+        /* a host-pointer call: the counter block and tables of the host pipeline's slot 0 */
+        memset(&plan->counters, 0x0, sizeof(plan->counters));
+        plan->counters.rays = n;
+        FanTables T;
+        if (fans != NULL) CUDA_TRY(fn, fan_upload(plan, 0, fans, bundle, 0, NULL, &T));
+        CUDA_TRY(fn, launch_voxels(plan, 0, n, d_pos, d_dir, (fans != NULL) ? &T : NULL, rule,
+                         grid, d_res, d_entries, capacity, d_count, NULL));
+        CUDA_TRY(fn, cudaDeviceSynchronize());
+        read_counters(plan, 0);
+        DEV_BACK(fn, results, d_res, n * sizeof(*d_res));
+        if (capacity > 0) DEV_BACK(fn, entries, d_entries, entry_bytes);
+        DEV_BACK(fn, count, d_count, n * sizeof(*d_count));
+        return TURTLE_RETURN_SUCCESS;
+}
+
+/* Checked arguments, n > 0: device memory, one launch, asynchronous on `stream`. */
+static enum turtle_return voxels_device(turtle_function_t * fn, struct turtle_plan * plan, size_t n,
+    const double * position, const double * direction, const struct turtle_fans * fans,
+    size_t bundle, const struct turtle_trace_rule * rule, const struct turtle_voxel_grid * grid,
+    struct turtle_trace_result * results, struct turtle_voxel_entry * entries, int capacity,
+    int32_t * count, void * stream)
+{
+        CUDA_TRY(fn, cudaSetDevice(plan->device));
+        memset(&plan->counters, 0x0, sizeof(plan->counters));
+        plan->counters.rays = n;
+        int slot;
+        CUDA_TRY(fn, next_device_slot(plan, &slot));
+        FanTables T;
+        cudaError_t err = cudaSuccess;
+        if (fans != NULL) err = fan_upload(plan, slot, fans, bundle, 0, (cudaStream_t)stream, &T);
+        if (err == cudaSuccess)
+                err = launch_voxels(plan, slot, n, position, direction, (fans != NULL) ? &T : NULL,
+                    rule, grid, results, entries, capacity, count, (cudaStream_t)stream);
+        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
+        return TURTLE_RETURN_SUCCESS;
+}
+
+extern "C" enum turtle_return turtle_stepper_trace_voxels(struct turtle_plan * plan, size_t n,
+    const double * position, const double * direction, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, struct turtle_trace_result * results,
+    struct turtle_voxel_entry * entries, int capacity, int32_t * count)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_trace_voxels);
+        enum turtle_return rc = check_voxels(fn, n, true, position, direction, rule, grid, entries,
+            capacity, count);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        rc = check_plan(fn, plan);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        return voxels_host(fn, plan, n, position, direction, NULL, 1, rule, grid, results, entries,
+            capacity, count);
+}
+
+extern "C" enum turtle_return turtle_stepper_trace_voxels_device(struct turtle_plan * plan,
+    size_t n, const double * position, const double * direction,
+    const struct turtle_trace_rule * rule, const struct turtle_voxel_grid * grid,
+    struct turtle_trace_result * results, struct turtle_voxel_entry * entries, int capacity,
+    int32_t * count, void * stream)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_trace_voxels_device);
+        enum turtle_return rc = check_voxels(fn, n, true, position, direction, rule, grid, entries,
+            capacity, count);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        rc = check_plan(fn, plan);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        return voxels_device(fn, plan, n, position, direction, NULL, 1, rule, grid, results,
+            entries, capacity, count, stream);
+}
+
+extern "C" enum turtle_return turtle_stepper_trace_fans_voxels(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, struct turtle_trace_result * results,
+    struct turtle_voxel_entry * entries, int capacity, int32_t * count)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_trace_fans_voxels);
+        size_t n, bundle;
+        enum turtle_return rc = check_fans(fn, fans, &n, &bundle);
+        if (rc == TURTLE_RETURN_SUCCESS)
+                rc = check_voxels(fn, n, false, NULL, NULL, rule, grid, entries, capacity, count);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        rc = check_plan(fn, plan);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        return voxels_host(fn, plan, n, NULL, NULL, fans, bundle, rule, grid, results, entries,
+            capacity, count);
+}
+
+extern "C" enum turtle_return turtle_stepper_trace_fans_voxels_device(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, struct turtle_trace_result * results,
+    struct turtle_voxel_entry * entries, int capacity, int32_t * count, void * stream)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_trace_fans_voxels_device);
+        size_t n, bundle;
+        enum turtle_return rc = check_fans(fn, fans, &n, &bundle);
+        if (rc == TURTLE_RETURN_SUCCESS)
+                rc = check_voxels(fn, n, false, NULL, NULL, rule, grid, entries, capacity, count);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        rc = check_plan(fn, plan);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        return voxels_device(fn, plan, n, NULL, NULL, fans, bundle, rule, grid, results, entries,
+            capacity, count, stream);
+}
+
 extern "C" enum turtle_return turtle_map_resample(struct turtle_map * map,
     struct turtle_plan * plan, int layer, size_t * outside)
 {
@@ -4918,6 +5635,10 @@ extern "C" const char * tb_batch_function_name(turtle_function_t * caller)
         NAME(turtle_stepper_horizon_device);
         NAME(turtle_stepper_horizons);
         NAME(turtle_stepper_horizons_device);
+        NAME(turtle_stepper_trace_voxels);
+        NAME(turtle_stepper_trace_voxels_device);
+        NAME(turtle_stepper_trace_fans_voxels);
+        NAME(turtle_stepper_trace_fans_voxels_device);
         NAME(turtle_b200_peer_alloc);
         NAME(turtle_b200_peer_free);
         NAME(turtle_b200_peer_export);
