@@ -206,6 +206,187 @@ typedef LaneStoreT<N_F, N_I> LaneStore;
 
 __device__ __forceinline__ void compiler_fence() { asm volatile("" ::: "memory"); }
 
+/* Row k of this lane's column of `store`, a LaneStoreT<NF, NI> (rows beyond the allocation
+ * are only named in code that is compiled out). */
+#define SF(k) store.f[((k) < NF) ? (k) : 0][tid]
+#define SI(k) store.i[((k) < NI) ? (k) : 0][tid]
+
+/* ---- pieces of the lane-store stepper that the trace, horizon, voxel and walk kernels share ---- */
+
+/* Start ray r at pos, dir in this lane's column: every ray starts from a reset stepper
+ * (turtle_stepper_reset, stepper.c:647-651). Returns MODE_INIT, or MODE_DONE for a ray that
+ * is never traced: an empty INVALID record (position as given), written out with the others. */
+template <bool LLA, int NF, int NI>
+__device__ __forceinline__ int ray_start(const tb::Geometry & G, const tb::LlaShared & V,
+    LaneStoreT<NF, NI> & store, const unsigned tid, unsigned long long r, const double pos[3],
+    const double dir[3])
+{
+        SF(F_POS) = pos[0];
+        SF(F_POS + 1) = pos[1];
+        SF(F_POS + 2) = pos[2];
+        SF(F_DIR) = dir[0];
+        SF(F_DIR + 1) = dir[1];
+        SF(F_DIR + 2) = dir[2];
+#pragma unroll
+        for (int m = 0; m < TURTLE_TRACE_MEDIA; m++)
+                SF(F_LEN + m) = 0.;
+        SF(F_TOTAL) = 0.;
+        SI(I_NSTEPS) = 0;
+        SI(I_NCHANGES) = 0;
+        SI(I_RAYLO) = (int)(unsigned)(r & 0xffffffffull);
+        SI(I_RAYHI) = (int)(unsigned)(r >> 32);
+        if (LLA) {
+                SI(I_PEND) = 0;
+                SF(F_LASTPOS) = SF(F_LASTPOS + 1) = SF(F_LASTPOS + 2) = DBL_MAX;
+                tb::lla_reset(G, V);
+        }
+        if (!finite3(pos) || !finite3(dir)) {
+                SF(F_ALT) = 0.;
+                SI(I_IDX0) = -1;
+                SI(I_IDX1) = -1;
+                SI(I_HASH) = 0;
+                SI(I_MEDIUM0) = TURTLE_TRACE_INVALID;
+                return MODE_DONE;
+        }
+        return MODE_INIT;
+}
+
+/* 8-byte field k < 12 of the 96-byte record of the finished lane t of this warp (MODE_DONE).
+ * Lane k stores field k: the twelve fields of a record go side by side, three full sectors
+ * in one request instead of twelve partial ones from one lane -- what makes the stores into
+ * a PEER's memory (multi-GPU, DESIGN.md section 7) cheap on NVLink, where every request is
+ * a packet. */
+template <int NF, int NI>
+__device__ __forceinline__ unsigned long long record_field(const LaneStoreT<NF, NI> & store,
+    unsigned t, unsigned k)
+{
+        if (k < 9u) {
+                const int row = (k < 3u) ? (int)(F_POS + k) :
+                    ((k == 3u) ? (int)F_ALT : ((k < 8u) ? (int)(F_LEN + k - 4u) : (int)F_TOTAL));
+                return (unsigned long long)__double_as_longlong(store.f[row][t]);
+        }
+        const int lo = (k == 9u) ? I_NSTEPS : ((k == 10u) ? I_IDX0 : I_HASH);
+        const int hi = (k == 9u) ? I_MEDIUM0 : ((k == 10u) ? I_IDX1 : I_NCHANGES);
+        return ((unsigned long long)(unsigned)store.i[hi][t] << 32) | (unsigned long long)(unsigned)store.i[lo][t];
+}
+
+/* Why a trace stops after a step (or the initial query) that settled on `last`, `total`
+ * metres and `n_steps` steps from its start (the limits of its turtle_trace_rule), or -1:
+ * it goes on. */
+template <class Args>
+__device__ __forceinline__ int stop_status(const Args & A, const tb::Sample & last, double total,
+    int n_steps)
+{
+        int status = -1;
+        if (last.idx0 < 0)
+                status = TURTLE_TRACE_DOMAIN;
+        else if (!(last.alt < A.altitude_max) || !(last.alt > A.altitude_min))
+                status = TURTLE_TRACE_ALTITUDE;
+        else if (total >= A.length_max)
+                status = TURTLE_TRACE_LENGTH;
+        else if (n_steps >= A.max_steps)
+                status = TURTLE_TRACE_STEPS;
+        return status;
+}
+
+/* The state update of a lane after its sample S (stepper.c:822-863): MODE_INIT's initial
+ * query, MODE_TENT's tentative step, MODE_BISECT's bisection of a medium change. S is
+ * published to the lane store when it becomes stepper->last. Returns true when a step (or
+ * the initial query) settled, with `last` = stepper->last and `ds` = the step's length;
+ * medium0 is the medium the step started in. HASH: MODE_INIT starts the FNV-1a hash of
+ * the media in I_HASH (a trace record; the horizon kernel uses that row otherwise). SHAPE_STACK: `moved` is the sampled position
+ * (lane_sample). */
+template <bool LLA, int SHAPE, bool HASH, int NF, int NI>
+__device__ __forceinline__ bool lane_advance(LaneStoreT<NF, NI> & store, const unsigned tid,
+    int & mode, const tb::Sample & S, const double moved[3], const int medium0, double & ds,
+    tb::Sample & last)
+{
+        bool settle = false;  /* a step (or the initial query) completed */
+        bool publish = false; /* S becomes stepper->last */
+        if (mode == MODE_INIT) {
+                publish = true;
+                if (HASH) SI(I_HASH) = (int)((2166136261u ^ (unsigned)(S.idx0 + 1)) * 16777619u);
+                settle = true;
+        } else if (mode == MODE_TENT) {
+                /* position += direction * ds, stepper.c:824 */
+                if (SHAPE == tb::SHAPE_STACK) {
+                        SF(F_POS) = moved[0];
+                        SF(F_POS + 1) = moved[1];
+                        SF(F_POS + 2) = moved[2];
+                } else {
+                        SF(F_POS) += SF(F_DIR) * ds;
+                        SF(F_POS + 1) += SF(F_DIR + 1) * ds;
+                        SF(F_POS + 2) += SF(F_DIR + 2) * ds;
+                }
+                publish = true;
+                if (S.idx0 != medium0) { /* stepper.c:832-838 */
+                        SF(F_DS0) = -ds;
+                        SF(F_DS1) = 0.;
+                        mode = MODE_BISECT;
+                        settle = !(0. - (-ds) > 1E-08);
+                } else {
+                        settle = true;
+                }
+        } else {
+                double ds0 = SF(F_DS0), ds1 = SF(F_DS1);
+                const double ds2 = 0.5 * (ds0 + ds1);
+                if (S.idx0 == medium0) { /* stepper.c:848-859 */
+                        ds0 = ds2;
+                        SF(F_DS0) = ds0;
+                } else {
+                        ds1 = ds2;
+                        SF(F_DS1) = ds1;
+                        publish = true;
+                        if (LLA) { /* last.position = position2 */
+                                SF(F_LASTPOS) = SF(F_POS) + SF(F_DIR) * ds2;
+                                SF(F_LASTPOS + 1) = SF(F_POS + 1) + SF(F_DIR + 1) * ds2;
+                                SF(F_LASTPOS + 2) = SF(F_POS + 2) + SF(F_DIR + 2) * ds2;
+                        }
+                }
+                if (!(ds1 - ds0 > 1E-08)) { /* stepper.c:861-863 */
+                        ds += ds1;
+                        SF(F_POS) += SF(F_DIR) * ds1;
+                        SF(F_POS + 1) += SF(F_DIR + 1) * ds1;
+                        SF(F_POS + 2) += SF(F_DIR + 2) * ds1;
+                        settle = true;
+                }
+        }
+        if (publish) { /* latitude and longitude are not part of a trace result */
+                SF(F_ALT) = S.alt;
+                SF(F_ELEV0) = S.elev0;
+                SF(F_ELEV1) = S.elev1;
+                SI(I_IDX0) = S.idx0;
+                SI(I_IDX1) = S.idx1;
+        }
+        if (!settle) return false;
+        last.lat = last.lon = 0.;
+        last.alt = publish ? S.alt : SF(F_ALT);
+        last.elev0 = publish ? S.elev0 : SF(F_ELEV0);
+        last.elev1 = publish ? S.elev1 : SF(F_ELEV1);
+        last.idx0 = publish ? S.idx0 : SI(I_IDX0);
+        last.idx1 = publish ? S.idx1 : SI(I_IDX1);
+        return true;
+}
+
+/* Add the counters of this warp's lanes to a call's: [1] steps, [2] samples, [4] Jacobian
+ * columns (local approximation only). */
+template <bool LLA>
+__device__ __forceinline__ void flush_counters(unsigned long long * cursor, unsigned lane,
+    unsigned steps, unsigned samples, unsigned rebuilds)
+{
+        unsigned long long steps64 = steps, samples64 = samples, rebuilds64 = rebuilds;
+        for (int o = 16; o > 0; o >>= 1) {
+                steps64 += __shfl_down_sync(0xffffffffu, steps64, o);
+                samples64 += __shfl_down_sync(0xffffffffu, samples64, o);
+                if (LLA) rebuilds64 += __shfl_down_sync(0xffffffffu, rebuilds64, o);
+        }
+        if (lane == 0u) {
+                atomicAdd(cursor + 1, steps64);
+                atomicAdd(cursor + 2, samples64);
+                if (LLA) atomicAdd(cursor + 4, rebuilds64);
+        }
+}
+
 /* Compact input / output of the trace kernel (COMPACT variants only: the kernels of
  * turtle_stepper_trace_fan / _fields; the others do not carry this code). */
 
@@ -356,9 +537,6 @@ __global__ void __launch_bounds__(128, MINB)
         const unsigned tid = threadIdx.x;
         const unsigned lane = tid & 31u;
         const unsigned FULL = 0xffffffffu;
-        /* (rows beyond the allocation are only named in code that is compiled out) */
-#define SF(k) store.f[((k) < NF) ? (k) : 0][tid]
-#define SI(k) store.i[((k) < NI) ? (k) : 0][tid]
 
         int mode = MODE_IDLE;
         /* local approximation: G.lla_rows columns of per-lane state in DYNAMIC shared memory
@@ -382,11 +560,7 @@ __global__ void __launch_bounds__(128, MINB)
         for (;;) {
                 if (STREAM && ((++iteration & 1023u) == 0u)) settle_done(A, owed);
                 /* ---- write out finished rays, one 96-byte record per instruction -------
-                 * A finished lane has left its record in shared memory (MODE_DONE). Twelve
-                 * lanes store its twelve 8-byte fields side by side: three full sectors in
-                 * one request instead of twelve partial ones from one lane -- what makes
-                 * the stores into a PEER's memory (multi-GPU, DESIGN.md section 7) cheap
-                 * on NVLink, where every request is a packet. */
+                 * A finished lane has left its record in shared memory (MODE_DONE). */
                 unsigned done_mask = __ballot_sync(FULL, mode == MODE_DONE);
                 if (COMPACT && (done_mask != 0u) && wants_fields(C) && (mode == MODE_DONE))
                         store_fields(C, &store.f[0][tid], &store.i[0][tid]); /* field arrays */
@@ -399,21 +573,9 @@ __global__ void __launch_bounds__(128, MINB)
                         const unsigned long long ray =
                             ((unsigned long long)(unsigned)store.i[I_RAYHI][t] << 32) |
                             (unsigned long long)(unsigned)store.i[I_RAYLO][t];
-                        if ((lane < 12u) && (!COMPACT || (A.results != NULL))) {
-                                unsigned long long bits;
-                                if (lane < 9u) {
-                                        const int row = (lane < 3u) ? (int)(F_POS + lane) :
-                                            ((lane == 3u) ? (int)F_ALT :
-                                                ((lane < 8u) ? (int)(F_LEN + lane - 4u) : (int)F_TOTAL));
-                                        bits = (unsigned long long)__double_as_longlong(store.f[row][t]);
-                                } else {
-                                        const int lo = (lane == 9u) ? I_NSTEPS : ((lane == 10u) ? I_IDX0 : I_HASH);
-                                        const int hi = (lane == 9u) ? I_MEDIUM0 : ((lane == 10u) ? I_IDX1 : I_NCHANGES);
-                                        bits = ((unsigned long long)(unsigned)store.i[hi][t] << 32) |
-                                            (unsigned long long)(unsigned)store.i[lo][t];
-                                }
-                                reinterpret_cast<unsigned long long *>(A.results + ray)[lane] = bits;
-                        }
+                        if ((lane < 12u) && (!COMPACT || (A.results != NULL)))
+                                reinterpret_cast<unsigned long long *>(A.results + ray)[lane] =
+                                    record_field(store, t, lane);
                         if (STREAM) {
                                 const int chunk = (int)(ray >> A.chunk_shift);
                                 const int o = __shfl_sync(FULL, owed, (int)src);
@@ -494,39 +656,7 @@ __global__ void __launch_bounds__(128, MINB)
                                                         dir[c] = __ldcg(d + c);
                                                 }
                                         }
-                                        SF(F_POS) = pos[0];
-                                        SF(F_POS + 1) = pos[1];
-                                        SF(F_POS + 2) = pos[2];
-                                        SF(F_DIR) = dir[0];
-                                        SF(F_DIR + 1) = dir[1];
-                                        SF(F_DIR + 2) = dir[2];
-#pragma unroll
-                                        for (int m = 0; m < TURTLE_TRACE_MEDIA; m++)
-                                                SF(F_LEN + m) = 0.;
-                                        SF(F_TOTAL) = 0.;
-                                        SI(I_NSTEPS) = 0;
-                                        SI(I_NCHANGES) = 0;
-                                        SI(I_RAYLO) = (int)(unsigned)(r & 0xffffffffull);
-                                        SI(I_RAYHI) = (int)(unsigned)(r >> 32);
-                                        if (LLA) SI(I_PEND) = 0;
-                                        mode = MODE_INIT;
-                                        /* every ray starts from a reset stepper
-                                         * (turtle_stepper_reset, stepper.c:647-651) */
-                                        if (LLA) {
-                                                SF(F_LASTPOS) = SF(F_LASTPOS + 1) =
-                                                    SF(F_LASTPOS + 2) = DBL_MAX;
-                                                tb::lla_reset(G, V);
-                                        }
-                                        if (!finite3(pos) || !finite3(dir)) {
-                                                /* never traced: an empty record (position
-                                                 * as given), written out with the others */
-                                                SF(F_ALT) = 0.;
-                                                SI(I_IDX0) = -1;
-                                                SI(I_IDX1) = -1;
-                                                SI(I_HASH) = 0;
-                                                SI(I_MEDIUM0) = TURTLE_TRACE_INVALID;
-                                                mode = MODE_DONE;
-                                        }
+                                        mode = ray_start<LLA>(G, V, store, tid, r, pos, dir);
                                 }
                         }
                         if (STREAM) {
@@ -658,75 +788,11 @@ __global__ void __launch_bounds__(128, MINB)
                 compiler_fence(); /* keep the state loads below out of the sample code */
                 my_samples++;
 
-                /* ---- state update ------------------------------------------ */
-                bool settle = false;  /* a step (or the initial query) completed */
-                bool publish = false; /* S becomes stepper->last */
+                /* ---- state update (lane_advance) ---- */
                 const int medium0 = SI(I_MEDIUM0);
                 double ds = SF(F_DS);
-                if (mode == MODE_INIT) {
-                        publish = true;
-                        SI(I_HASH) = (int)((2166136261u ^ (unsigned)(S.idx0 + 1)) * 16777619u);
-                        settle = true;
-                } else if (mode == MODE_TENT) {
-                        /* position += direction * ds, stepper.c:824 */
-                        if (SHAPE == tb::SHAPE_STACK) {
-                                SF(F_POS) = moved[0];
-                                SF(F_POS + 1) = moved[1];
-                                SF(F_POS + 2) = moved[2];
-                        } else {
-                                SF(F_POS) += SF(F_DIR) * ds;
-                                SF(F_POS + 1) += SF(F_DIR + 1) * ds;
-                                SF(F_POS + 2) += SF(F_DIR + 2) * ds;
-                        }
-                        publish = true;
-                        if (S.idx0 != medium0) { /* stepper.c:832-838 */
-                                SF(F_DS0) = -ds;
-                                SF(F_DS1) = 0.;
-                                mode = MODE_BISECT;
-                                settle = !(0. - (-ds) > 1E-08);
-                        } else {
-                                settle = true;
-                        }
-                } else {
-                        double ds0 = SF(F_DS0), ds1 = SF(F_DS1);
-                        const double ds2 = 0.5 * (ds0 + ds1);
-                        if (S.idx0 == medium0) { /* stepper.c:848-859 */
-                                ds0 = ds2;
-                                SF(F_DS0) = ds0;
-                        } else {
-                                ds1 = ds2;
-                                SF(F_DS1) = ds1;
-                                publish = true;
-                                if (LLA) { /* last.position = position2 */
-                                        SF(F_LASTPOS) = SF(F_POS) + SF(F_DIR) * ds2;
-                                        SF(F_LASTPOS + 1) = SF(F_POS + 1) + SF(F_DIR + 1) * ds2;
-                                        SF(F_LASTPOS + 2) = SF(F_POS + 2) + SF(F_DIR + 2) * ds2;
-                                }
-                        }
-                        if (!(ds1 - ds0 > 1E-08)) { /* stepper.c:861-863 */
-                                ds += ds1;
-                                SF(F_POS) += SF(F_DIR) * ds1;
-                                SF(F_POS + 1) += SF(F_DIR + 1) * ds1;
-                                SF(F_POS + 2) += SF(F_DIR + 2) * ds1;
-                                settle = true;
-                        }
-                }
-                if (publish) { /* latitude and longitude are not part of a trace result */
-                        SF(F_ALT) = S.alt;
-                        SF(F_ELEV0) = S.elev0;
-                        SF(F_ELEV1) = S.elev1;
-                        SI(I_IDX0) = S.idx0;
-                        SI(I_IDX1) = S.idx1;
-                }
-                if (!settle) continue;
-
                 tb::Sample last; /* stepper->last: this sample, or the one published before */
-                last.lat = last.lon = 0.;
-                last.alt = publish ? S.alt : SF(F_ALT);
-                last.elev0 = publish ? S.elev0 : SF(F_ELEV0);
-                last.elev1 = publish ? S.elev1 : SF(F_ELEV1);
-                last.idx0 = publish ? S.idx0 : SI(I_IDX0);
-                last.idx1 = publish ? S.idx1 : SI(I_IDX1);
+                if (!lane_advance<LLA, SHAPE, true>(store, tid, mode, S, moved, medium0, ds, last)) continue;
                 double total = SF(F_TOTAL);
                 int n_steps = SI(I_NSTEPS);
                 if (mode != MODE_INIT) {
@@ -757,16 +823,7 @@ __global__ void __launch_bounds__(128, MINB)
                         }
                 }
 
-                int status = -1;
-                if (last.idx0 < 0)
-                        status = TURTLE_TRACE_DOMAIN;
-                else if (!(last.alt < A.altitude_max) || !(last.alt > A.altitude_min))
-                        status = TURTLE_TRACE_ALTITUDE;
-                else if (total >= A.length_max)
-                        status = TURTLE_TRACE_LENGTH;
-                else if (n_steps >= A.max_steps)
-                        status = TURTLE_TRACE_STEPS;
-
+                const int status = stop_status(A, last, total, n_steps);
                 if (status >= 0) {
                         /* position, altitude, lengths, counters, index and hash are in the
                          * lane store already; the status takes the row of `medium0` */
@@ -778,22 +835,9 @@ __global__ void __launch_bounds__(128, MINB)
                         mode = MODE_TENT;
                 }
         }
-#undef SF
-#undef SI
 
-        /* per-warp counters ([3] is the time-out flag of a streamed call; Jacobian-column
-         * iterations are counted with the samples' cursor block, slot [4]) */
-        unsigned long long steps64 = my_steps, samples64 = my_samples, rebuilds64 = my_rebuilds;
-        for (int o = 16; o > 0; o >>= 1) {
-                steps64 += __shfl_down_sync(FULL, steps64, o);
-                samples64 += __shfl_down_sync(FULL, samples64, o);
-                if (LLA) rebuilds64 += __shfl_down_sync(FULL, rebuilds64, o);
-        }
-        if (lane == 0u) {
-                atomicAdd(A.cursor + 1, steps64);
-                atomicAdd(A.cursor + 2, samples64);
-                if (LLA) atomicAdd(A.cursor + 4, rebuilds64);
-        }
+        /* ([3] is the time-out flag of a streamed call, [5] the window's hits) */
+        flush_counters<LLA>(A.cursor, lane, my_steps, my_samples, my_rebuilds);
         if (GATHER == GATHER_WINDOW) {
                 unsigned long long hits64 = from_window.hits;
                 for (int o = 16; o > 0; o >>= 1) hits64 += __shfl_down_sync(FULL, hits64, o);
@@ -847,8 +891,6 @@ __global__ void __launch_bounds__(128, MINB)
         const unsigned FULL = 0xffffffffu;
         turtle_horizon & R = record[tid >> 5];
         const double * F = frame[tid >> 5];
-#define SF(k) store.f[((k) < NF) ? (k) : 0][tid]
-#define SI(k) store.i[((k) < NI) ? (k) : 0][tid]
         extern __shared__ double lla_store[];
         const tb::LlaShared V = { lla_store + tid };
         unsigned my_steps = 0u, my_samples = 0u, my_rebuilds = 0u, my_probes = 0u;
@@ -1085,73 +1127,11 @@ __global__ void __launch_bounds__(128, MINB)
                 compiler_fence();
                 my_samples++;
 
-                /* ---- state update: trace_kernel's, but for the end of a probe ---- */
-                bool settle = false;
-                bool publish = false;
+                /* ---- state update (lane_advance) ---- */
                 const int medium0 = SI(I_MEDIUM0);
                 double ds = SF(F_DS);
-                if (mode == MODE_INIT) {
-                        publish = true;
-                        settle = true;
-                } else if (mode == MODE_TENT) {
-                        if (SHAPE == tb::SHAPE_STACK) {
-                                SF(F_POS) = moved[0];
-                                SF(F_POS + 1) = moved[1];
-                                SF(F_POS + 2) = moved[2];
-                        } else {
-                                SF(F_POS) += SF(F_DIR) * ds;
-                                SF(F_POS + 1) += SF(F_DIR + 1) * ds;
-                                SF(F_POS + 2) += SF(F_DIR + 2) * ds;
-                        }
-                        publish = true;
-                        if (S.idx0 != medium0) {
-                                SF(F_DS0) = -ds;
-                                SF(F_DS1) = 0.;
-                                mode = MODE_BISECT;
-                                settle = !(0. - (-ds) > 1E-08);
-                        } else {
-                                settle = true;
-                        }
-                } else {
-                        double ds0 = SF(F_DS0), ds1 = SF(F_DS1);
-                        const double ds2 = 0.5 * (ds0 + ds1);
-                        if (S.idx0 == medium0) {
-                                ds0 = ds2;
-                                SF(F_DS0) = ds0;
-                        } else {
-                                ds1 = ds2;
-                                SF(F_DS1) = ds1;
-                                publish = true;
-                                if (LLA) {
-                                        SF(F_LASTPOS) = SF(F_POS) + SF(F_DIR) * ds2;
-                                        SF(F_LASTPOS + 1) = SF(F_POS + 1) + SF(F_DIR + 1) * ds2;
-                                        SF(F_LASTPOS + 2) = SF(F_POS + 2) + SF(F_DIR + 2) * ds2;
-                                }
-                        }
-                        if (!(ds1 - ds0 > 1E-08)) {
-                                ds += ds1;
-                                SF(F_POS) += SF(F_DIR) * ds1;
-                                SF(F_POS + 1) += SF(F_DIR + 1) * ds1;
-                                SF(F_POS + 2) += SF(F_DIR + 2) * ds1;
-                                settle = true;
-                        }
-                }
-                if (publish) {
-                        SF(F_ALT) = S.alt;
-                        SF(F_ELEV0) = S.elev0;
-                        SF(F_ELEV1) = S.elev1;
-                        SI(I_IDX0) = S.idx0;
-                        SI(I_IDX1) = S.idx1;
-                }
-                if (!settle) continue;
-
-                tb::Sample last;
-                last.lat = last.lon = 0.;
-                last.alt = publish ? S.alt : SF(F_ALT);
-                last.elev0 = publish ? S.elev0 : SF(F_ELEV0);
-                last.elev1 = publish ? S.elev1 : SF(F_ELEV1);
-                last.idx0 = publish ? S.idx0 : SI(I_IDX0);
-                last.idx1 = publish ? S.idx1 : SI(I_IDX1);
+                tb::Sample last; /* stepper->last: this sample, or the one published before */
+                if (!lane_advance<LLA, SHAPE, false>(store, tid, mode, S, moved, medium0, ds, last)) continue;
                 double total = SF(F_TOTAL);
                 int n_steps = SI(I_NSTEPS);
                 int outcome = TURTLE_TRACE_INVALID + 1; /* none yet */
@@ -1170,14 +1150,8 @@ __global__ void __launch_bounds__(128, MINB)
                                 outcome = HORIZON_OBSTRUCTED;
                 }
                 if (outcome > TURTLE_TRACE_INVALID) {
-                        if (last.idx0 < 0)
-                                outcome = TURTLE_TRACE_DOMAIN;
-                        else if (!(last.alt < A.altitude_max) || !(last.alt > A.altitude_min))
-                                outcome = TURTLE_TRACE_ALTITUDE;
-                        else if (total >= A.length_max)
-                                outcome = TURTLE_TRACE_LENGTH;
-                        else if (n_steps >= A.max_steps)
-                                outcome = TURTLE_TRACE_STEPS;
+                        const int status = stop_status(A, last, total, n_steps);
+                        if (status >= 0) outcome = status;
                 }
                 if (outcome <= TURTLE_TRACE_INVALID) {
                         SI(I_OUTCOME) = outcome;
@@ -1188,21 +1162,9 @@ __global__ void __launch_bounds__(128, MINB)
                         mode = MODE_TENT;
                 }
         }
-#undef SF
-#undef SI
 
-        unsigned long long steps64 = my_steps, samples64 = my_samples, rebuilds64 = my_rebuilds;
-        for (int o = 16; o > 0; o >>= 1) {
-                steps64 += __shfl_down_sync(FULL, steps64, o);
-                samples64 += __shfl_down_sync(FULL, samples64, o);
-                if (LLA) rebuilds64 += __shfl_down_sync(FULL, rebuilds64, o);
-        }
-        if (lane == 0u) {
-                atomicAdd(A.cursor + 1, steps64);
-                atomicAdd(A.cursor + 2, samples64);
-                if (LLA) atomicAdd(A.cursor + 4, rebuilds64);
-                atomicAdd(A.cursor + 6, (unsigned long long)my_probes);
-        }
+        flush_counters<LLA>(A.cursor, lane, my_steps, my_samples, my_rebuilds);
+        if (lane == 0u) atomicAdd(A.cursor + 6, (unsigned long long)my_probes);
 }
 
 /* ---- rock length per cell of a voxel grid (turtle_stepper_trace_voxels) --------------------- */
@@ -1266,8 +1228,6 @@ __global__ void __launch_bounds__(128, MINB)
         const unsigned tid = threadIdx.x;
         const unsigned lane = tid & 31u;
         const unsigned FULL = 0xffffffffu;
-#define SF(k) store.f[((k) < NF) ? (k) : 0][tid]
-#define SI(k) store.i[((k) < NI) ? (k) : 0][tid]
         extern __shared__ double lla_store[];
         const tb::LlaShared V = { lla_store + tid };
         unsigned my_steps = 0u, my_samples = 0u, my_rebuilds = 0u;
@@ -1275,7 +1235,7 @@ __global__ void __launch_bounds__(128, MINB)
         bool exhausted = false;
 
         for (;;) {
-                /* ---- write out finished records, twelve lanes side by side (trace_kernel) ---- */
+                /* ---- write out finished records (record_field) ---- */
                 unsigned done_mask = __ballot_sync(FULL, mode == MODE_DONE);
                 if (done_mask != 0u) __syncwarp();
                 const bool wrote = done_mask != 0u;
@@ -1286,21 +1246,9 @@ __global__ void __launch_bounds__(128, MINB)
                         const unsigned long long ray =
                             ((unsigned long long)(unsigned)store.i[I_RAYHI][t] << 32) |
                             (unsigned long long)(unsigned)store.i[I_RAYLO][t];
-                        if ((lane < 12u) && (A.results != NULL)) {
-                                unsigned long long bits;
-                                if (lane < 9u) {
-                                        const int row = (lane < 3u) ? (int)(F_POS + lane) :
-                                            ((lane == 3u) ? (int)F_ALT :
-                                                ((lane < 8u) ? (int)(F_LEN + lane - 4u) : (int)F_TOTAL));
-                                        bits = (unsigned long long)__double_as_longlong(store.f[row][t]);
-                                } else {
-                                        const int lo = (lane == 9u) ? I_NSTEPS : ((lane == 10u) ? I_IDX0 : I_HASH);
-                                        const int hi = (lane == 9u) ? I_MEDIUM0 : ((lane == 10u) ? I_IDX1 : I_NCHANGES);
-                                        bits = ((unsigned long long)(unsigned)store.i[hi][t] << 32) |
-                                            (unsigned long long)(unsigned)store.i[lo][t];
-                                }
-                                reinterpret_cast<unsigned long long *>(A.results + ray)[lane] = bits;
-                        }
+                        if ((lane < 12u) && (A.results != NULL))
+                                reinterpret_cast<unsigned long long *>(A.results + ray)[lane] =
+                                    record_field(store, t, lane);
                         if (lane == src) {
                                 A.count[ray] = vi[VI_COUNT][tid];
                                 mode = MODE_IDLE;
@@ -1329,18 +1277,7 @@ __global__ void __launch_bounds__(128, MINB)
                                                                 dir[c] = __ldg(A.direction + 3ull * r + c);
                                                         }
                                                 }
-                                                for (int c = 0; c < 3; c++) {
-                                                        SF(F_POS + c) = pos[c];
-                                                        SF(F_DIR + c) = dir[c];
-                                                }
-#pragma unroll
-                                                for (int m = 0; m < TURTLE_TRACE_MEDIA; m++)
-                                                        SF(F_LEN + m) = 0.;
-                                                SF(F_TOTAL) = 0.;
-                                                SI(I_NSTEPS) = 0;
-                                                SI(I_NCHANGES) = 0;
-                                                SI(I_RAYLO) = (int)(unsigned)(r & 0xffffffffull);
-                                                SI(I_RAYHI) = (int)(unsigned)(r >> 32);
+                                                mode = ray_start<LLA>(G, V, store, tid, r, pos, dir);
                                                 vi[VI_CELL][tid] = -1;
                                                 vi[VI_COUNT][tid] = 0;
                                                 /* the ray in grid coordinates, and where its line
@@ -1365,21 +1302,6 @@ __global__ void __launch_bounds__(128, MINB)
                                                 }
                                                 vf[VF_TIN][tid] = t_in;
                                                 vf[VF_TOUT][tid] = t_out;
-                                                mode = MODE_INIT;
-                                                if (LLA) { /* a reset stepper (stepper.c:647-651) */
-                                                        SI(I_PEND) = 0;
-                                                        SF(F_LASTPOS) = SF(F_LASTPOS + 1) =
-                                                            SF(F_LASTPOS + 2) = DBL_MAX;
-                                                        tb::lla_reset(G, V);
-                                                }
-                                                if (!finite3(pos) || !finite3(dir)) {
-                                                        SF(F_ALT) = 0.;
-                                                        SI(I_IDX0) = -1;
-                                                        SI(I_IDX1) = -1;
-                                                        SI(I_HASH) = 0;
-                                                        SI(I_MEDIUM0) = TURTLE_TRACE_INVALID;
-                                                        mode = MODE_DONE;
-                                                }
                                         }
                                 }
                                 if (base + (unsigned long long)need >= A.n) exhausted = true;
@@ -1487,74 +1409,11 @@ __global__ void __launch_bounds__(128, MINB)
                 compiler_fence();
                 my_samples++;
 
-                /* ---- state update: trace_kernel's ---- */
-                bool settle = false;
-                bool publish = false;
+                /* ---- state update (lane_advance) ---- */
                 const int medium0 = SI(I_MEDIUM0);
                 double ds = SF(F_DS);
-                if (mode == MODE_INIT) {
-                        publish = true;
-                        SI(I_HASH) = (int)((2166136261u ^ (unsigned)(S.idx0 + 1)) * 16777619u);
-                        settle = true;
-                } else if (mode == MODE_TENT) {
-                        if (SHAPE == tb::SHAPE_STACK) {
-                                SF(F_POS) = moved[0];
-                                SF(F_POS + 1) = moved[1];
-                                SF(F_POS + 2) = moved[2];
-                        } else {
-                                SF(F_POS) += SF(F_DIR) * ds;
-                                SF(F_POS + 1) += SF(F_DIR + 1) * ds;
-                                SF(F_POS + 2) += SF(F_DIR + 2) * ds;
-                        }
-                        publish = true;
-                        if (S.idx0 != medium0) {
-                                SF(F_DS0) = -ds;
-                                SF(F_DS1) = 0.;
-                                mode = MODE_BISECT;
-                                settle = !(0. - (-ds) > 1E-08);
-                        } else {
-                                settle = true;
-                        }
-                } else {
-                        double ds0 = SF(F_DS0), ds1 = SF(F_DS1);
-                        const double ds2 = 0.5 * (ds0 + ds1);
-                        if (S.idx0 == medium0) {
-                                ds0 = ds2;
-                                SF(F_DS0) = ds0;
-                        } else {
-                                ds1 = ds2;
-                                SF(F_DS1) = ds1;
-                                publish = true;
-                                if (LLA) {
-                                        SF(F_LASTPOS) = SF(F_POS) + SF(F_DIR) * ds2;
-                                        SF(F_LASTPOS + 1) = SF(F_POS + 1) + SF(F_DIR + 1) * ds2;
-                                        SF(F_LASTPOS + 2) = SF(F_POS + 2) + SF(F_DIR + 2) * ds2;
-                                }
-                        }
-                        if (!(ds1 - ds0 > 1E-08)) {
-                                ds += ds1;
-                                SF(F_POS) += SF(F_DIR) * ds1;
-                                SF(F_POS + 1) += SF(F_DIR + 1) * ds1;
-                                SF(F_POS + 2) += SF(F_DIR + 2) * ds1;
-                                settle = true;
-                        }
-                }
-                if (publish) {
-                        SF(F_ALT) = S.alt;
-                        SF(F_ELEV0) = S.elev0;
-                        SF(F_ELEV1) = S.elev1;
-                        SI(I_IDX0) = S.idx0;
-                        SI(I_IDX1) = S.idx1;
-                }
-                if (!settle) continue;
-
-                tb::Sample last;
-                last.lat = last.lon = 0.;
-                last.alt = publish ? S.alt : SF(F_ALT);
-                last.elev0 = publish ? S.elev0 : SF(F_ELEV0);
-                last.elev1 = publish ? S.elev1 : SF(F_ELEV1);
-                last.idx0 = publish ? S.idx0 : SI(I_IDX0);
-                last.idx1 = publish ? S.idx1 : SI(I_IDX1);
+                tb::Sample last; /* stepper->last: this sample, or the one published before */
+                if (!lane_advance<LLA, SHAPE, true>(store, tid, mode, S, moved, medium0, ds, last)) continue;
                 double total = SF(F_TOTAL);
                 int n_steps = SI(I_NSTEPS);
                 const unsigned long long ray =
@@ -1639,16 +1498,7 @@ __global__ void __launch_bounds__(128, MINB)
                         }
                 }
 
-                int status = -1;
-                if (last.idx0 < 0)
-                        status = TURTLE_TRACE_DOMAIN;
-                else if (!(last.alt < A.altitude_max) || !(last.alt > A.altitude_min))
-                        status = TURTLE_TRACE_ALTITUDE;
-                else if (total >= A.length_max)
-                        status = TURTLE_TRACE_LENGTH;
-                else if (n_steps >= A.max_steps)
-                        status = TURTLE_TRACE_STEPS;
-
+                const int status = stop_status(A, last, total, n_steps);
                 if (status >= 0) {
                         SI(I_MEDIUM0) = status;
                         int count = vi[VI_COUNT][tid];
@@ -1661,20 +1511,8 @@ __global__ void __launch_bounds__(128, MINB)
                         mode = MODE_TENT;
                 }
         }
-#undef SF
-#undef SI
 
-        unsigned long long steps64 = my_steps, samples64 = my_samples, rebuilds64 = my_rebuilds;
-        for (int o = 16; o > 0; o >>= 1) {
-                steps64 += __shfl_down_sync(FULL, steps64, o);
-                samples64 += __shfl_down_sync(FULL, samples64, o);
-                if (LLA) rebuilds64 += __shfl_down_sync(FULL, rebuilds64, o);
-        }
-        if (lane == 0u) {
-                atomicAdd(A.cursor + 1, steps64);
-                atomicAdd(A.cursor + 2, samples64);
-                if (LLA) atomicAdd(A.cursor + 4, rebuilds64);
-        }
+        flush_counters<LLA>(A.cursor, lane, my_steps, my_samples, my_rebuilds);
 }
 
 /* Longest-expected-first scheduling: the number of steps of a ray grows as it runs
@@ -1763,13 +1601,12 @@ template <bool LLA, bool PROJ, bool STATES, bool MULTI = false>
 __global__ void __launch_bounds__(128, 5)
     walk_kernel(const __grid_constant__ tb::Geometry G, const StepArgs A)
 {
+        constexpr int NF = N_F, NI = N_I;
         __shared__ LaneStore store;
         extern __shared__ double lla_store[]; /* LLA: scratch (no states), or the state (MULTI) */
         const unsigned tid = threadIdx.x;
         const unsigned lane = tid & 31u;
         const unsigned FULL = 0xffffffffu;
-#define SF(k) store.f[k][tid]
-#define SI(k) store.i[k][tid]
 
         int mode = MODE_IDLE;
         typename WalkView<STATES && !MULTI>::type V;
@@ -2111,20 +1948,11 @@ __global__ void __launch_bounds__(128, 5)
                 }
                 mode = MODE_IDLE;
         }
+        flush_counters<LLA>(A.counters, lane, my_steps, my_samples, my_rebuilds);
+}
+
 #undef SF
 #undef SI
-        unsigned long long steps64 = my_steps, samples64 = my_samples, rebuilds64 = my_rebuilds;
-        for (int o = 16; o > 0; o >>= 1) {
-                steps64 += __shfl_down_sync(FULL, steps64, o);
-                samples64 += __shfl_down_sync(FULL, samples64, o);
-                rebuilds64 += __shfl_down_sync(FULL, rebuilds64, o);
-        }
-        if (lane == 0u) {
-                atomicAdd(A.counters + 1, steps64);
-                atomicAdd(A.counters + 2, samples64);
-                atomicAdd(A.counters + 4, rebuilds64);
-        }
-}
 
 /* turtle_stepper_reset for every particle (stepper.c:602-615): last position and every
  * reference point at DBL_MAX; the last sample is cleared, no Jacobian is stale. */
@@ -3141,6 +2969,23 @@ static size_t lla_bytes(const struct turtle_plan * plan)
         return (plan->G.range > 0.) ? (size_t)plan->G.lla_rows * 128 * sizeof(double) : 0;
 }
 
+/* The kernel variant of a plan's geometry: the local approximation (range > 0), any
+ * projected map (else the projection code is compiled out), and the single-stack
+ * specialisation (turtle_plan_specialise_set). */
+struct Variant {
+        bool lla, proj, stack_shape;
+};
+static Variant variant_of(const struct turtle_plan * plan)
+{
+        Variant v;
+        v.lla = plan->G.range > 0.;
+        v.proj = false;
+        for (int t = 0; t < plan->G.n_transforms; t++)
+                if (plan->G.transforms[t].type != tb::PROJ_GEODETIC) v.proj = true;
+        v.stack_shape = plan->specialise && (tb::geometry_shape(plan->G) == tb::SHAPE_STACK);
+        return v;
+}
+
 /* Grid of the persistent kernel: a multiple of the SM count. With the local approximation
  * the lane store of a CTA grows by the state of the transforms the geometry uses, and the
  * CTAs per SM are what fits the 227 kB of shared memory (4 for one projected transform). */
@@ -3335,10 +3180,7 @@ static cudaError_t launch_trace(struct turtle_plan * plan, int slot, size_t n,
         A.max_steps = rule->max_steps;
         int blocks, threads;
         const int per_sm = trace_grid(plan, n, &blocks, &threads);
-        const bool lla = plan->G.range > 0.;
-        bool proj = false; /* any projected map? else the projection code is compiled out */
-        for (int t = 0; t < plan->G.n_transforms; t++)
-                if (plan->G.transforms[t].type != tb::PROJ_GEODETIC) proj = true;
+        const auto [lla, proj, stack_shape] = variant_of(plan);
         /* the register budget follows the requested residency (in units of 128 threads);
          * the kernels of the local approximation are built for 4 CTAs per SM (trace_grid) */
 #define TRACE_LAUNCH(MINB)                                                             \
@@ -3349,7 +3191,6 @@ static cudaError_t launch_trace(struct turtle_plan * plan, int slot, size_t n,
                         trace_start<false, false, MINB, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none); \
         } while (0)
         const int minb = per_sm * threads / 128;
-        const bool stack_shape = plan->specialise && (tb::geometry_shape(plan->G) == tb::SHAPE_STACK);
         const bool compact = (io.fan != NULL) || (io.fields != NULL);
         if (compact) {
                 /* fan input and / or field outputs: the COMPACT kernels, at the default
@@ -4211,11 +4052,7 @@ static cudaError_t launch_horizon(struct turtle_plan * plan, int slot, size_t n_
         const int per_sm = trace_grid(plan, 0, &blocks, &threads);
         const size_t warps = (size_t)threads / 32;
         blocks = (int)std::min<size_t>((size_t)plan->sm_count * per_sm, (items + warps - 1) / warps);
-        const bool lla = plan->G.range > 0.;
-        bool proj = false;
-        for (int t = 0; t < plan->G.n_transforms; t++)
-                if (plan->G.transforms[t].type != tb::PROJ_GEODETIC) proj = true;
-        const bool stack_shape = plan->specialise && (tb::geometry_shape(plan->G) == tb::SHAPE_STACK);
+        const auto [lla, proj, stack_shape] = variant_of(plan);
         void (*kernel)(const tb::Geometry, const HorizonArgs) =
             stack_shape ? horizon_kernel<false, false, 6, tb::SHAPE_STACK> :
             (lla && proj) ? horizon_kernel<true, true, 4, tb::SHAPE_GENERIC> :
@@ -4489,10 +4326,8 @@ static enum turtle_return launch_walk(turtle_function_t * fn, struct turtle_plan
                 if (ring) release_device_slot(plan, slot, st, err);
                 CUDA_TRY(fn, err);
         }
-        const bool lla = plan->G.range > 0.;
-        bool proj = false;
-        for (int t = 0; t < plan->G.n_transforms; t++)
-                if (plan->G.transforms[t].type != tb::PROJ_GEODETIC) proj = true;
+        const auto [lla, proj, stack_shape] = variant_of(plan); /* (no walk kernel for the stack shape) */
+        (void)stack_shape;
         /* the CTAs per SM get the carve-out they need and no more: the rest is L1 for the
          * DEM gathers (as for the trace kernel) */
         void (*kernel)(const tb::Geometry, const StepArgs);
@@ -4725,11 +4560,7 @@ static cudaError_t launch_voxels(struct turtle_plan * plan, int slot, size_t n,
                 A.size[a] = grid->size[a];
                 A.cells[a] = grid->n[a];
         }
-        const bool lla = plan->G.range > 0.;
-        bool proj = false;
-        for (int t = 0; t < plan->G.n_transforms; t++)
-                if (plan->G.transforms[t].type != tb::PROJ_GEODETIC) proj = true;
-        const bool stack_shape = plan->specialise && (tb::geometry_shape(plan->G) == tb::SHAPE_STACK);
+        const auto [lla, proj, stack_shape] = variant_of(plan);
         void (*kernel)(const tb::Geometry, const VoxelArgs) =
             stack_shape ? voxel_kernel<false, false, 6, tb::SHAPE_STACK> :
             (lla && proj) ? voxel_kernel<true, true, 4, tb::SHAPE_GENERIC> :
