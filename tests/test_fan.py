@@ -77,8 +77,9 @@ def test_fan_equals_rays_with_reference_directions(small_stack, bundle):
 
 @pytest.mark.gpu
 def test_fields_only_and_rounds(small_stack):
-    """Only what is asked for is written; calls above the staging bound go in rounds (the
-    fan's ray index carries over); device-pointer variants agree."""
+    """Only what is asked for is written; host fans go in slices and calls above the staging
+    bound in rounds (the field arrays of each begin at its first ray); device-pointer variants
+    agree."""
     import torch
     sc = Scene(stacks=[small_stack], ops=[(H.ADD_STACK, 0, 0.)], range=0.)
     stepper, _, _ = sc.product()
@@ -92,17 +93,7 @@ def test_fields_only_and_rounds(small_stack):
     fan = tb.Plan.make_fan(lat, lon, origin, az, el, bundle=32)
     rec = np.zeros(n, dtype=tb.TRACE_RESULT)
     plan.trace_fan(fan, rule, results=rec)
-    # (the fan call cuts the fan in resident slices; the streamed kernel, in rounds, is the
-    # path of calls that stream rays in: held to the same answers here)
-    os.environ["TURTLE_B200_FAN_STREAMED"] = "1"
-    os.environ["TURTLE_B200_STREAM_MAX_RAYS"] = str(1 << 18)  # three rounds
     two = tb.Plan.host_fields(n, ["length0", "status"])
-    two["length0"][:] = -7.
-    plan.trace_fan(fan, rule, fields=two)
-    del os.environ["TURTLE_B200_STREAM_MAX_RAYS"], os.environ["TURTLE_B200_FAN_STREAMED"]
-    assert np.array_equal(two["length0"], rec["length"][:, 0])
-    assert np.array_equal(two["status"], rec["status"])
-    assert plan.counters()["rays"] == n
     two["length0"][:] = -7.
     os.environ["TURTLE_B200_FAN_SLICE_RAYS"] = str(1 << 17)  # five slices on two streams
     plan.trace_fan(fan, rule, fields=two)
@@ -114,6 +105,15 @@ def test_fields_only_and_rounds(small_stack):
     ora = sc.oracle()
     dirs = fan_rays(ora, lat, lon, az, el, 32)
     pos = np.repeat(origin[None], n, 0)
+    # (the streamed kernel, in rounds: the field arrays of each round begin at its first ray)
+    os.environ["TURTLE_B200_STREAM_MAX_RAYS"] = str(1 << 18)  # three rounds
+    rounds = tb.Plan.host_fields(n, ["length0", "status"])
+    rounds["length0"][:] = -7.
+    plan.trace_fields(pos, dirs, rule, rounds)
+    del os.environ["TURTLE_B200_STREAM_MAX_RAYS"]
+    assert np.array_equal(rounds["length0"], rec["length"][:, 0])
+    assert np.array_equal(rounds["status"], rec["status"])
+    assert plan.counters()["rays"] == n
     three = plan.trace_fields(pos, dirs, rule, tb.Plan.host_fields(n, ["total", "n_steps", "index"]))
     assert np.array_equal(three["total"], rec["total"])
     assert np.array_equal(three["n_steps"], rec["n_steps"])

@@ -84,20 +84,23 @@ struct TraceArgs {
         int max_crossings;
 };
 
+/* Device tables of a fan (fan_upload): ray r belongs to station s = r / per_station and starts
+ * at its origin; direction of ray (i, j) from the host's sines / cosines of the angles,
+ * az[i] = { sin az, cos az }, el[j] = { cos el, sin el }, and the station's East / North / Up
+ * vectors (ecef.c:136-178). */
+struct FanTables {
+        const double2 * az;
+        const double2 * el;
+        const double * station; /* [n_station][12]: origin, East, North, Up */
+        unsigned long long naz, bundle, per_station;
+        unsigned long long ray0; /* first ray of this launch */
+};
+
 /* Compact input / output (turtle_stepper_trace_fan / _fields): a kernel parameter of its
  * own, of the COMPACT kernels only -- the mere presence of these members in TraceArgs
  * costs every trace kernel four registers. */
 struct CompactArgs {
-        /* fan input (turtle_stepper_trace_fan[s]; TraceArgs::position == NULL): ray r belongs to
-         * station s = r / fan_per_station and starts at its origin; direction of ray (i, j)
-         * from the host's sines / cosines of the angles, fan_az[i] = { sin az, cos az },
-         * fan_el[j] = { cos el, sin el }, and the station's East / North / Up vectors
-         * (ecef.c:136-178). fan_station[12 s ...]: origin, East, North, Up of station s. */
-        const double2 * fan_az;
-        const double2 * fan_el;
-        const double * fan_station;
-        unsigned long long fan_naz, fan_bundle, fan_per_station;
-        unsigned long long fan_ray0; /* first ray of this launch */
+        FanTables fan; /* fan input (turtle_stepper_trace_fan[s]; TraceArgs::position == NULL) */
         /* field outputs (turtle_trace_fields: device arrays, any NULL), when use_fields */
         turtle_trace_fields fields;
         int use_fields;
@@ -396,18 +399,19 @@ __device__ __forceinline__ void flush_counters(unsigned long long * cursor, unsi
 __device__ __forceinline__ void fan_ray(const CompactArgs & A, unsigned long long r, double pos[3],
     double dir[3])
 {
-        const unsigned long long per_band = A.fan_naz * A.fan_bundle;
-        const unsigned long long rs = r + A.fan_ray0;
-        const unsigned long long s = rs / A.fan_per_station;
-        const unsigned long long rr = rs - s * A.fan_per_station;
+        const FanTables & T = A.fan;
+        const unsigned long long per_band = T.naz * T.bundle;
+        const unsigned long long rs = r + T.ray0;
+        const unsigned long long s = rs / T.per_station;
+        const unsigned long long rr = rs - s * T.per_station;
         const unsigned long long band = rr / per_band;
         const unsigned long long rem = rr - band * per_band;
-        const unsigned long long i = rem / A.fan_bundle;
-        const unsigned long long j = band * A.fan_bundle + (rem - i * A.fan_bundle);
-        const double2 az = __ldg(A.fan_az + i);
-        const double2 el = __ldg(A.fan_el + j);
+        const unsigned long long i = rem / T.bundle;
+        const unsigned long long j = band * T.bundle + (rem - i * T.bundle);
+        const double2 az = __ldg(T.az + i);
+        const double2 el = __ldg(T.el + j);
         const double r0 = el.x * az.x, r1 = el.x * az.y, r2 = el.y;
-        const double * f = A.fan_station + 12ull * s;
+        const double * f = T.station + 12ull * s;
 #pragma unroll
         for (int c = 0; c < 3; c++) {
                 pos[c] = __ldg(f + c);
@@ -2385,7 +2389,7 @@ struct turtle_plan {
         unsigned * h_flags;                  /* pinned + mapped: chunk completion flags */
         size_t stream_chunks;
         cudaEvent_t ev_reset;
-        cudaStream_t drain[4]; /* N_DRAINS result streams */
+        cudaStream_t drain[N_DRAINS]; /* result streams */
         /* fan tables (turtle_stepper_trace_fan[s], _horizon[s]), per slot: pinned host copy +
          * device copy of the angles' sines / cosines and the stations' frames (fan_upload) */
         double2 * h_fan[ALL_SLOTS];
@@ -2814,7 +2818,7 @@ extern "C" void turtle_plan_destroy(struct turtle_plan ** plan_)
         if (plan->h_marks != NULL) cudaFreeHost(plan->h_marks);
         if (plan->h_flags != NULL) cudaFreeHost(plan->h_flags);
         if (plan->ev_reset != NULL) cudaEventDestroy(plan->ev_reset);
-        for (int j = 0; j < 4; j++)
+        for (int j = 0; j < N_DRAINS; j++)
                 if (plan->drain[j] != NULL) cudaStreamDestroy(plan->drain[j]);
         cudaFree(plan->pool);
         cudaFree(plan->d_maps);
@@ -2920,6 +2924,60 @@ extern "C" enum turtle_return turtle_plan_gather_set(struct turtle_plan * plan, 
         return TURTLE_RETURN_SUCCESS;
 }
 
+/* A staging buffer of a plan: device memory, or pinned host memory allocated with
+ * cudaHostAlloc(`host_flags`) when host_flags >= 0. */
+struct Staging {
+        void ** p;
+        size_t bytes;
+        int host_flags = -1;
+};
+
+/* Grow-only staging: while `*have` (in the caller's unit) is below `need`, the buffers are
+ * freed and allocated again at their `bytes`. `*have` becomes `need` once all of them are
+ * allocated, and stays 0 after a failure so that the next call tries again. */
+template <size_t K>
+static cudaError_t grow(size_t * have, size_t need, const Staging (&buffers)[K])
+{
+        if (*have >= need) return cudaSuccess;
+        *have = 0;
+        for (const Staging & b : buffers) {
+                if (b.host_flags < 0)
+                        cudaFree(*b.p);
+                else if (*b.p != NULL)
+                        cudaFreeHost(*b.p);
+                *b.p = NULL;
+        }
+        for (const Staging & b : buffers) {
+                const cudaError_t err = (b.host_flags < 0) ? cudaMalloc(b.p, b.bytes) :
+                                                             cudaHostAlloc(b.p, b.bytes, b.host_flags);
+                if (err != cudaSuccess) return err;
+        }
+        *have = need;
+        return cudaSuccess;
+}
+
+/* Small RAII helper for the host-pointer wrappers of the simple kernels. */
+namespace {
+struct DeviceBuffers {
+        std::vector<void *> ptrs;
+        ~DeviceBuffers()
+        {
+                for (size_t i = 0; i < ptrs.size(); i++) cudaFree(ptrs[i]);
+        }
+        /* allocate `bytes` and optionally copy from host; NULL host + copy_in=false = output */
+        cudaError_t get(void ** dev, const void * host, size_t bytes, bool copy_in)
+        {
+                *dev = NULL;
+                cudaError_t err = cudaMalloc(dev, std::max<size_t>(bytes, 8));
+                if (err != cudaSuccess) return err;
+                ptrs.push_back(*dev);
+                if (copy_in && (host != NULL) && bytes)
+                        err = cudaMemcpy(*dev, host, bytes, cudaMemcpyHostToDevice);
+                return err;
+        }
+};
+}
+
 /* Build the queue order of a launch (longest-expected-first) in plan->d_sched. */
 static cudaError_t schedule_rays(struct turtle_plan * plan, int slot, size_t n,
     const double * d_position, const double * d_direction, cudaStream_t stream,
@@ -2929,20 +2987,15 @@ static cudaError_t schedule_rays(struct turtle_plan * plan, int slot, size_t n,
         if ((plan->schedule == 0) || (n < 2) || (n > 0x7fffffffull)) return cudaSuccess;
         cudaError_t err = cudaSuccess;
         if (plan->sched_rays[slot] < n) {
-                cudaFree(plan->d_sched[slot]);
-                cudaFree(plan->d_sched_tmp[slot]);
-                plan->d_sched[slot] = NULL;
-                plan->d_sched_tmp[slot] = NULL;
-                plan->sched_rays[slot] = 0;
                 size_t tmp = 0;
                 err = cub::DeviceRadixSort::SortPairs(NULL, tmp, (const unsigned *)NULL,
                     (unsigned *)NULL, (const unsigned *)NULL, (unsigned *)NULL, (int)n, 0, 31,
                     stream);
                 if (err == cudaSuccess)
-                        err = cudaMalloc((void **)&plan->d_sched[slot], 4 * n * sizeof(unsigned));
-                if (err == cudaSuccess) err = cudaMalloc(&plan->d_sched_tmp[slot], tmp);
+                        err = grow(&plan->sched_rays[slot], n,
+                            { { (void **)&plan->d_sched[slot], 4 * n * sizeof(unsigned) },
+                                { &plan->d_sched_tmp[slot], tmp } });
                 if (err != cudaSuccess) return err;
-                plan->sched_rays[slot] = n;
                 plan->sched_tmp_bytes[slot] = tmp;
         }
         unsigned * keys = plan->d_sched[slot];
@@ -2984,6 +3037,22 @@ static Variant variant_of(const struct turtle_plan * plan)
                 if (plan->G.transforms[t].type != tb::PROJ_GEODETIC) v.proj = true;
         v.stack_shape = plan->specialise && (tb::geometry_shape(plan->G) == tb::SHAPE_STACK);
         return v;
+}
+
+template <bool LLA_, bool PROJ_, int SHAPE_, int MINB_> struct VariantOf {
+        static const bool LLA = LLA_, PROJ = PROJ_;
+        static const int SHAPE = SHAPE_, MINB = MINB_;
+};
+
+/* f(VariantOf<LLA, PROJ, SHAPE, MINB>()) for the variant `v`, at the default residency of its
+ * kernels: 4 CTAs per SM with the local approximation (trace_grid), else 6. */
+template <class F> static auto with_variant(const Variant & v, F && f)
+{
+        if (v.stack_shape) return f(VariantOf<false, false, tb::SHAPE_STACK, 6>());
+        if (v.lla && v.proj) return f(VariantOf<true, true, tb::SHAPE_GENERIC, 4>());
+        if (v.lla) return f(VariantOf<true, false, tb::SHAPE_GENERIC, 4>());
+        if (v.proj) return f(VariantOf<false, true, tb::SHAPE_GENERIC, 6>());
+        return f(VariantOf<false, false, tb::SHAPE_GENERIC, 6>());
 }
 
 /* Grid of the persistent kernel: a multiple of the SM count. With the local approximation
@@ -3110,20 +3179,30 @@ static cudaError_t release_device_slot(struct turtle_plan * plan, int slot, cuda
         return (err != cudaSuccess) ? err : rec;
 }
 
+/* The frame of a device-pointer call: on the plan's device, the counters reset to a call of
+ * `rays` rays (unless `reset` is false: a walk keeps them), a slot of the ring taken,
+ * body(slot) queued on `stream`, and the slot released with the body's status. */
+template <class Body>
+static enum turtle_return device_call(turtle_function_t * fn, struct turtle_plan * plan,
+    bool reset, size_t rays, cudaStream_t stream, Body && body)
+{
+        CUDA_TRY(fn, cudaSetDevice(plan->device));
+        if (reset) {
+                memset(&plan->counters, 0x0, sizeof(plan->counters));
+                plan->counters.rays = rays;
+        }
+        int slot;
+        CUDA_TRY(fn, next_device_slot(plan, &slot));
+        CUDA_TRY(fn, release_device_slot(plan, slot, stream, body(slot)));
+        return TURTLE_RETURN_SUCCESS;
+}
+
 /* Device state of a streamed call: [0] watermark, then one counter per chunk. */
 struct StreamState {
         int chunk_shift;
         const unsigned long long * watermark;
         unsigned * chunk_done;
         unsigned * chunk_flags;
-};
-
-/* Device tables of a fan: sines / cosines of its angles and the frames of its stations. */
-struct FanTables {
-        const double2 * az;
-        const double2 * el;
-        const double * station; /* [n_station][12]: origin, East, North, Up */
-        unsigned long long naz, bundle, per_station, ray0;
 };
 
 /* What one launch reads and writes: DEVICE memory throughout. */
@@ -3162,13 +3241,7 @@ static cudaError_t launch_trace(struct turtle_plan * plan, int slot, size_t n,
         const NoCompactArgs none = { 0 };
         if (io.fan != NULL) {
                 A.position = A.direction = NULL;
-                C.fan_az = io.fan->az;
-                C.fan_el = io.fan->el;
-                C.fan_station = io.fan->station;
-                C.fan_naz = io.fan->naz;
-                C.fan_bundle = io.fan->bundle;
-                C.fan_per_station = io.fan->per_station;
-                C.fan_ray0 = io.fan->ray0;
+                C.fan = *io.fan;
         }
         A.results = io.results;
         C.use_fields = (io.fields != NULL);
@@ -3180,61 +3253,33 @@ static cudaError_t launch_trace(struct turtle_plan * plan, int slot, size_t n,
         A.max_steps = rule->max_steps;
         int blocks, threads;
         const int per_sm = trace_grid(plan, n, &blocks, &threads);
-        const auto [lla, proj, stack_shape] = variant_of(plan);
-        /* the register budget follows the requested residency (in units of 128 threads);
-         * the kernels of the local approximation are built for 4 CTAs per SM (trace_grid) */
-#define TRACE_LAUNCH(MINB)                                                             \
-        do {                                                                           \
-                if (proj)                                                              \
-                        trace_start<false, true, MINB, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none); \
-                else                                                                   \
-                        trace_start<false, false, MINB, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none); \
-        } while (0)
-        const int minb = per_sm * threads / 128;
+        const Variant v = variant_of(plan);
         const bool compact = (io.fan != NULL) || (io.fields != NULL);
-        if (compact) {
-                /* fan input and / or field outputs: the COMPACT kernels, at the default
-                 * residency of their shape */
+        /* the register budget of a resident kernel without the local approximation follows the
+         * requested residency (in units of 128 threads) */
+        const int minb = per_sm * threads / 128;
+        if (compact || (streamed != NULL) || v.lla) {
+                /* fan input and / or field outputs (the COMPACT kernels), streamed calls (the
+                 * kernels waiting for their rays) and the local approximation: the default
+                 * residency of the variant */
                 const int sm6 = (per_sm < 6) ? per_sm : 6;
                 if (blocks > plan->sm_count * sm6) blocks = plan->sm_count * sm6;
-#define COMPACT_LAUNCH(STREAMED)                                                       \
-        do {                                                                           \
-                if (stack_shape)                                                       \
-                        trace_start<false, false, 6, tb::SHAPE_STACK, STREAMED, true>(plan, sm6, blocks, threads, stream, A, C); \
-                else if (lla && proj)                                                  \
-                        trace_start<true, true, 4, tb::SHAPE_GENERIC, STREAMED, true>(plan, sm6, blocks, threads, stream, A, C); \
-                else if (lla)                                                          \
-                        trace_start<true, false, 4, tb::SHAPE_GENERIC, STREAMED, true>(plan, sm6, blocks, threads, stream, A, C); \
-                else if (proj)                                                         \
-                        trace_start<false, true, 6, tb::SHAPE_GENERIC, STREAMED, true>(plan, sm6, blocks, threads, stream, A, C); \
-                else                                                                   \
-                        trace_start<false, false, 6, tb::SHAPE_GENERIC, STREAMED, true>(plan, sm6, blocks, threads, stream, A, C); \
-        } while (0)
-                if (streamed != NULL)
-                        COMPACT_LAUNCH(true);
-                else
-                        COMPACT_LAUNCH(false);
-#undef COMPACT_LAUNCH
-        } else if (streamed != NULL) {
-                /* streamed calls: the kernels waiting for their rays, 6 CTAs per SM */
-                const int cap = plan->sm_count * ((per_sm < 6) ? per_sm : 6);
-                if (blocks > cap) blocks = cap;
-                const int sm6 = (per_sm < 6) ? per_sm : 6;
-                if (stack_shape)
-                        trace_start<false, false, 6, tb::SHAPE_STACK, true>(plan, sm6, blocks, threads, stream, A, none);
-                else if (lla && proj)
-                        trace_start<true, true, 4, tb::SHAPE_GENERIC, true>(plan, sm6, blocks, threads, stream, A, none);
-                else if (lla)
-                        trace_start<true, false, 4, tb::SHAPE_GENERIC, true>(plan, sm6, blocks, threads, stream, A, none);
-                else if (proj)
-                        trace_start<false, true, 6, tb::SHAPE_GENERIC, true>(plan, sm6, blocks, threads, stream, A, none);
-                else
-                        trace_start<false, false, 6, tb::SHAPE_GENERIC, true>(plan, sm6, blocks, threads, stream, A, none);
-        } else if (lla && proj)
-                trace_start<true, true, 4, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none);
-        else if (lla)
-                trace_start<true, false, 4, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none);
-        else if (stack_shape) {
+                with_variant(v, [&](auto V) {
+                        typedef decltype(V) K;
+                        if (compact && (streamed != NULL))
+                                trace_start<K::LLA, K::PROJ, K::MINB, K::SHAPE, true, true>(
+                                    plan, sm6, blocks, threads, stream, A, C);
+                        else if (compact)
+                                trace_start<K::LLA, K::PROJ, K::MINB, K::SHAPE, false, true>(
+                                    plan, sm6, blocks, threads, stream, A, C);
+                        else if (streamed != NULL)
+                                trace_start<K::LLA, K::PROJ, K::MINB, K::SHAPE, true>(
+                                    plan, sm6, blocks, threads, stream, A, none);
+                        else
+                                trace_start<K::LLA, K::PROJ, K::MINB, K::SHAPE>(
+                                    plan, sm6, blocks, threads, stream, A, none);
+                });
+        } else if (v.stack_shape) {
                 if ((minb <= 6) && (plan->gather == GATHER_PACKED))
                         trace_start<false, false, 6, tb::SHAPE_STACK, false, false, GATHER_PACKED>(
                             plan, per_sm, blocks, threads, stream, A, none);
@@ -3247,15 +3292,26 @@ static cudaError_t launch_trace(struct turtle_plan * plan, int slot, size_t n,
                         trace_start<false, false, 6, tb::SHAPE_STACK>(plan, per_sm, blocks, threads, stream, A, none);
                 else
                         trace_start<false, false, 8, tb::SHAPE_STACK>(plan, per_sm, blocks, threads, stream, A, none);
-        } else if (minb <= 4)
-                TRACE_LAUNCH(4);
-        else if (minb == 5)
-                TRACE_LAUNCH(5);
-        else if (minb <= 7)
-                TRACE_LAUNCH(6);
-        else
-                TRACE_LAUNCH(8);
-#undef TRACE_LAUNCH
+        } else if (minb <= 4) {
+                if (v.proj)
+                        trace_start<false, true, 4, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none);
+                else
+                        trace_start<false, false, 4, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none);
+        } else if (minb == 5) {
+                if (v.proj)
+                        trace_start<false, true, 5, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none);
+                else
+                        trace_start<false, false, 5, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none);
+        } else if (minb <= 7) {
+                if (v.proj)
+                        trace_start<false, true, 6, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none);
+                else
+                        trace_start<false, false, 6, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none);
+        } else if (v.proj) {
+                trace_start<false, true, 8, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none);
+        } else {
+                trace_start<false, false, 8, tb::SHAPE_GENERIC>(plan, per_sm, blocks, threads, stream, A, none);
+        }
         plan->counters.launches++;
         return cudaGetLastError();
 }
@@ -3265,20 +3321,15 @@ extern "C" enum turtle_return turtle_stepper_trace_batch_device(
     const double * direction, const struct turtle_trace_rule * rule,
     struct turtle_trace_result * results, void * stream)
 {
-        enum turtle_return rc = check_rule(FN(&turtle_stepper_trace_batch_device), rule);
+        turtle_function_t * fn = FN(&turtle_stepper_trace_batch_device);
+        enum turtle_return rc = check_rule(fn, rule);
         if (rc != TURTLE_RETURN_SUCCESS) return rc;
         if (n == 0) return TURTLE_RETURN_SUCCESS;
-        CUDA_TRY(&turtle_stepper_trace_batch_device, cudaSetDevice(plan->device));
-        memset(&plan->counters, 0x0, sizeof(plan->counters));
-        plan->counters.rays = n;
-        int slot;
-        CUDA_TRY(&turtle_stepper_trace_batch_device, next_device_slot(plan, &slot));
         const DeviceIo io = { position, direction, NULL, results, NULL };
-        const cudaError_t err = launch_trace(plan, slot, n, io, rule,
-            plan->d_counters + CTR * slot, (cudaStream_t)stream);
-        CUDA_TRY(&turtle_stepper_trace_batch_device,
-            release_device_slot(plan, slot, (cudaStream_t)stream, err));
-        return TURTLE_RETURN_SUCCESS;
+        return device_call(fn, plan, true, n, (cudaStream_t)stream, [&](int slot) {
+                return launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
+                    (cudaStream_t)stream);
+        });
 }
 
 extern "C" enum turtle_return turtle_stepper_trace_crossings_device(
@@ -3294,17 +3345,12 @@ extern "C" enum turtle_return turtle_stepper_trace_crossings_device(
                 return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
                     "invalid crossings buffer");
         if (n == 0) return TURTLE_RETURN_SUCCESS;
-        CUDA_TRY(fn, cudaSetDevice(plan->device));
-        memset(&plan->counters, 0x0, sizeof(plan->counters));
-        plan->counters.rays = n;
-        int slot;
-        CUDA_TRY(fn, next_device_slot(plan, &slot));
         const DeviceIo io = { position, direction, NULL, results, NULL };
-        const cudaError_t err = launch_trace(plan, slot, n, io, rule,
-            plan->d_counters + CTR * slot, (cudaStream_t)stream, NULL,
-            (max_crossings > 0) ? crossings : NULL, max_crossings);
-        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
-        return TURTLE_RETURN_SUCCESS;
+        return device_call(fn, plan, true, n, (cudaStream_t)stream, [&](int slot) {
+                return launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
+                    (cudaStream_t)stream, NULL, (max_crossings > 0) ? crossings : NULL,
+                    max_crossings);
+        });
 }
 
 /* Lazily create the streams and staging buffers of the host-pointer pipeline. */
@@ -3318,37 +3364,44 @@ static cudaError_t plan_pipeline(struct turtle_plan * plan, size_t rays)
                         if (err == cudaSuccess) err = cudaEventCreate(&plan->ev1[s]);
                 }
         }
-        if ((err == cudaSuccess) && (plan->slot_rays < rays)) {
-                for (int s = 0; s < N_SLOTS; s++) {
-                        cudaFree(plan->d_in[s]);
-                        cudaFree(plan->d_out[s]);
-                        plan->d_in[s] = NULL;
-                        plan->d_out[s] = NULL;
-                }
-                plan->slot_rays = 0;
-                for (int s = 0; (s < N_SLOTS) && (err == cudaSuccess); s++) {
-                        err = cudaMalloc((void **)&plan->d_in[s], rays * 6 * sizeof(double));
-                        if (err == cudaSuccess)
-                                err = cudaMalloc((void **)&plan->d_out[s],
-                                    rays * sizeof(turtle_trace_result));
-                }
-                if (err == cudaSuccess) plan->slot_rays = rays;
+        if (err != cudaSuccess) return err;
+        Staging buffers[2 * N_SLOTS];
+        for (int s = 0; s < N_SLOTS; s++) {
+                buffers[2 * s] = { (void **)&plan->d_in[s], rays * 6 * sizeof(double) };
+                buffers[2 * s + 1] = { (void **)&plan->d_out[s], rays * sizeof(turtle_trace_result) };
         }
-        return err;
+        return grow(&plan->slot_rays, rays, buffers);
+}
+
+/* Adds the steps, samples and rebuilds of the k <= HOST_SLICES counter blocks from block
+ * `first`, whose launches are over, to `to`; c (or NULL): every counter summed over the k
+ * blocks. */
+static cudaError_t add_counters(const struct turtle_plan * plan, int first, int k,
+    turtle_plan_counters & to, unsigned long long * c = NULL)
+{
+        unsigned long long blocks[HOST_SLICES][CTR], sum[CTR] = { 0 };
+        const cudaError_t err = cudaMemcpy(blocks, plan->d_counters + CTR * first,
+            k * sizeof blocks[0], cudaMemcpyDeviceToHost);
+        if (err != cudaSuccess) return err;
+        for (int b = 0; b < k; b++)
+                for (int j = 0; j < CTR; j++) sum[j] += blocks[b][j];
+        to.steps += sum[1];
+        to.samples += sum[2];
+        to.rebuilds += sum[4];
+        if (c != NULL) memcpy(c, sum, sizeof sum);
+        return cudaSuccess;
 }
 
 /* The step / sample counters of the launch that used counter block `slot`, once it is over. */
 static void read_counters(struct turtle_plan * plan, int slot)
 {
+        turtle_plan_counters read = plan->counters;
+        read.steps = read.samples = read.rebuilds = 0;
         unsigned long long c[CTR];
-        if (cudaMemcpy(c, plan->d_counters + CTR * slot, sizeof c,
-                cudaMemcpyDeviceToHost) == cudaSuccess) {
-                plan->counters.steps = c[1];
-                plan->counters.samples = c[2];
-                plan->counters.rebuilds = c[4];
-                plan->counters.window_hits = c[5];
-                if (c[6] != 0ull) plan->counters.rays = c[6]; /* the probes of a horizon search */
-        }
+        if (add_counters(plan, slot, 1, read, c) != cudaSuccess) return;
+        read.window_hits = c[5];
+        if (c[6] != 0ull) read.rays = c[6]; /* the probes of a horizon search */
+        plan->counters = read;
 }
 
 extern "C" void turtle_plan_counters_sync(struct turtle_plan * plan)
@@ -3437,19 +3490,10 @@ static cudaError_t fan_upload(struct turtle_plan * plan, int slot, const struct 
 {
         const size_t angles = fans->n_azimuth + fans->n_elevation;
         const size_t entries = angles + 6 * fans->n_station; /* in double2 */
-        if (plan->fan_entries[slot] < entries) {
-                if (plan->h_fan[slot] != NULL) cudaFreeHost(plan->h_fan[slot]);
-                cudaFree(plan->d_fan[slot]);
-                plan->h_fan[slot] = NULL;
-                plan->d_fan[slot] = NULL;
-                plan->fan_entries[slot] = 0;
-                cudaError_t err = cudaHostAlloc((void **)&plan->h_fan[slot], entries * sizeof(double2),
-                    cudaHostAllocDefault);
-                if (err == cudaSuccess)
-                        err = cudaMalloc((void **)&plan->d_fan[slot], entries * sizeof(double2));
-                if (err != cudaSuccess) return err;
-                plan->fan_entries[slot] = entries;
-        }
+        const cudaError_t err = grow(&plan->fan_entries[slot], entries,
+            { { (void **)&plan->h_fan[slot], entries * sizeof(double2), cudaHostAllocDefault },
+                { (void **)&plan->d_fan[slot], entries * sizeof(double2) } });
+        if (err != cudaSuccess) return err;
         double2 * h = plan->h_fan[slot];
         for (size_t i = 0; i < fans->n_azimuth; i++) {
                 const double az = fans->azimuth[i] * M_PI / 180.;
@@ -3478,11 +3522,10 @@ static cudaError_t fan_upload(struct turtle_plan * plan, int slot, const struct 
             cudaMemcpyHostToDevice, stream);
 }
 
-/* The field arrays of a call, one after the other: (pointer slot, bytes per ray). */
+/* The field arrays of a call, one after the other. */
 struct FieldSpec {
-        void * const * host; /* where the caller's pointer sits in its turtle_trace_fields */
-        size_t offset;       /* ... as a byte offset, to address the device copy alike */
-        size_t bytes;        /* per ray */
+        size_t offset; /* of the array's pointer in struct turtle_trace_fields */
+        size_t bytes;  /* per ray */
 };
 
 static int field_specs(const struct turtle_trace_fields * f, FieldSpec specs[12])
@@ -3490,7 +3533,6 @@ static int field_specs(const struct turtle_trace_fields * f, FieldSpec specs[12]
         int k = 0;
 #define FIELD(member, size)                                                          \
         if (f->member != NULL) {                                                     \
-                specs[k].host = (void * const *)&f->member;                          \
                 specs[k].offset = (size_t)((const char *)&f->member - (const char *)f); \
                 specs[k].bytes = (size);                                             \
                 k++;                                                                 \
@@ -3502,11 +3544,75 @@ static int field_specs(const struct turtle_trace_fields * f, FieldSpec specs[12]
         return k;
 }
 
+/* The array of `spec` in `f`, and setting it (the members are pointers of several types). */
+static char * field_array(const struct turtle_trace_fields & f, const FieldSpec & spec)
+{
+        char * p;
+        memcpy(&p, (const char *)&f + spec.offset, sizeof p);
+        return p;
+}
+static void set_field_array(struct turtle_trace_fields & f, const FieldSpec & spec, char * p)
+{
+        memcpy((char *)&f + spec.offset, &p, sizeof p);
+}
+
+/* The arrays of `f` from ray `first` on. */
+static struct turtle_trace_fields offset_fields(struct turtle_trace_fields f, size_t first)
+{
+        FieldSpec specs[12];
+        const int k = field_specs(&f, specs);
+        for (int i = 0; i < k; i++)
+                set_field_array(f, specs[i], field_array(f, specs[i]) + first * specs[i].bytes);
+        return f;
+}
+
+/* Device staging of the field arrays of a host-pointer call of n rays, carved from the plan's
+ * field pool, each on a 256-byte boundary: *d_fields has an array where `fields` (or NULL) has
+ * one, *n_fields of them. */
+static cudaError_t stage_fields(struct turtle_plan * plan, size_t n,
+    const struct turtle_trace_fields * fields, struct turtle_trace_fields * d_fields, int * n_fields)
+{
+        memset(d_fields, 0x0, sizeof *d_fields);
+        FieldSpec specs[12];
+        *n_fields = (fields != NULL) ? field_specs(fields, specs) : 0;
+        size_t need = 0;
+        for (int k = 0; k < *n_fields; k++) need += (n * specs[k].bytes + 255) / 256 * 256;
+        const cudaError_t err = grow(&plan->field_pool_bytes, need, { { &plan->d_field_pool, need } });
+        if (err != cudaSuccess) return err;
+        size_t at = 0;
+        for (int k = 0; k < *n_fields; k++) {
+                set_field_array(*d_fields, specs[k], (char *)plan->d_field_pool + at);
+                at += (n * specs[k].bytes + 255) / 256 * 256;
+        }
+        return cudaSuccess;
+}
+
+/* Queue on `stream` the copy of rays [first, first + m) of a host-pointer call from the plan's
+ * staging (plan->d_all_out, the fields of stage_fields) to the caller's `results` and `fields`
+ * (either NULL). */
+static cudaError_t copy_out(const struct turtle_plan * plan, size_t first, size_t m,
+    struct turtle_trace_result * results, const struct turtle_trace_fields * fields,
+    const struct turtle_trace_fields & d_fields, cudaStream_t stream)
+{
+        cudaError_t err = cudaSuccess;
+        if (results != NULL)
+                err = cudaMemcpyAsync(results + first, plan->d_all_out + first,
+                    m * sizeof(turtle_trace_result), cudaMemcpyDeviceToHost, stream);
+        if (fields == NULL) return err;
+        FieldSpec specs[12];
+        const int k = field_specs(fields, specs);
+        const struct turtle_trace_fields dst = offset_fields(*fields, first);
+        const struct turtle_trace_fields src = offset_fields(d_fields, first);
+        for (int f = 0; (f < k) && (err == cudaSuccess); f++)
+                err = cudaMemcpyAsync(field_array(dst, specs[f]), field_array(src, specs[f]),
+                    m * specs[f].bytes, cudaMemcpyDeviceToHost, stream);
+        return err;
+}
+
 /* Host-pointer call, streamed: ONE persistent trace kernel over all the rays while the
  * copy engines feed and drain it.
  *   stream 1 (H2D): for each chunk, positions and directions, then the new watermark
- *                   (an 8-byte copy, ordered after the data of the chunk) -- a fan has no
- *                   rays to copy: its tables go first and the watermark is raised at once;
+ *                   (an 8-byte copy, ordered after the data of the chunk);
  *   stream 0      : the trace kernel -- a lane that holds ticket q waits until the
  *                   watermark has passed q (MODE_WAIT), and every finished ray is counted
  *                   for its chunk after a __threadfence;
@@ -3514,80 +3620,40 @@ static int field_specs(const struct turtle_trace_fields * f, FieldSpec specs[12]
  *                   mapped host memory; the calling thread watches the flags and queues the
  *                   copy of each chunk's records and / or field slices as it completes.
  * Compared with one kernel per chunk there is a single kernel tail instead of one per
- * chunk, and no lane ever idles between chunks. */
+ * chunk, and no lane ever idles between chunks. The call adds its counts to the plan's
+ * counters. */
 static enum turtle_return trace_streamed(turtle_function_t * fn, struct turtle_plan * plan,
-    size_t n, size_t ray0, const double * position, const double * direction,
-    const struct turtle_fans * fan, size_t bundle, const struct turtle_trace_rule * rule,
-    struct turtle_trace_result * results, const struct turtle_trace_fields * fields,
-    int chunk_shift)
+    size_t n, const double * position, const double * direction,
+    const struct turtle_trace_rule * rule, struct turtle_trace_result * results,
+    const struct turtle_trace_fields * fields)
 {
-        const size_t chunk = (size_t)1 << chunk_shift;
+        const size_t chunk = STREAM_CHUNK_RAYS;
         const size_t n_chunks = (n + chunk - 1) / chunk;
         CUDA_TRY(fn, plan_pipeline(plan, 1)); /* the three streams and their events */
         if (plan->ev_reset == NULL) CUDA_TRY(fn, cudaEventCreate(&plan->ev_reset));
-        if ((fan == NULL) && (plan->all_rays < n)) {
-                cudaFree(plan->d_all_in);
-                plan->d_all_in = NULL;
-                plan->all_rays = 0;
-                CUDA_TRY(fn, cudaMalloc((void **)&plan->d_all_in, (n * 6 + 32) * sizeof(double)));
-                plan->all_rays = n;
-        }
-        if ((results != NULL) && (plan->all_records < n)) {
-                cudaFree(plan->d_all_out);
-                plan->d_all_out = NULL;
-                plan->all_records = 0;
-                CUDA_TRY(fn, cudaMalloc((void **)&plan->d_all_out, n * sizeof(turtle_trace_result)));
-                plan->all_records = n;
-        }
-        /* device copies of the field arrays the caller asked for */
-        FieldSpec specs[12];
-        const int n_fields = (fields != NULL) ? field_specs(fields, specs) : 0;
+        CUDA_TRY(fn, grow(&plan->all_rays, n,
+                         { { (void **)&plan->d_all_in, (n * 6 + 32) * sizeof(double) } }));
+        if (results != NULL)
+                CUDA_TRY(fn, grow(&plan->all_records, n,
+                                 { { (void **)&plan->d_all_out, n * sizeof(turtle_trace_result) } }));
         struct turtle_trace_fields d_fields;
-        memset(&d_fields, 0x0, sizeof d_fields);
-        if (n_fields > 0) {
-                size_t need = 0;
-                for (int k = 0; k < n_fields; k++) need += (n * specs[k].bytes + 255) / 256 * 256;
-                if (plan->field_pool_bytes < need) {
-                        cudaFree(plan->d_field_pool);
-                        plan->d_field_pool = NULL;
-                        plan->field_pool_bytes = 0;
-                        CUDA_TRY(fn, cudaMalloc(&plan->d_field_pool, need));
-                        plan->field_pool_bytes = need;
-                }
-                size_t at = 0;
-                for (int k = 0; k < n_fields; k++) {
-                        *(void **)((char *)&d_fields + specs[k].offset) =
-                            (char *)plan->d_field_pool + at;
-                        at += (n * specs[k].bytes + 255) / 256 * 256;
-                }
-        }
-        if (plan->stream_chunks < n_chunks) {
-                cudaFree(plan->d_stream_state);
-                if (plan->h_marks != NULL) cudaFreeHost(plan->h_marks);
-                if (plan->h_flags != NULL) cudaFreeHost(plan->h_flags);
-                plan->d_stream_state = NULL;
-                plan->h_marks = NULL;
-                plan->h_flags = NULL;
-                plan->stream_chunks = 0;
-                CUDA_TRY(fn, cudaMalloc((void **)&plan->d_stream_state,
-                                 (n_chunks + 2) * sizeof(unsigned long long)));
-                CUDA_TRY(fn, cudaHostAlloc((void **)&plan->h_marks,
-                                 (n_chunks + 1) * sizeof(unsigned long long), cudaHostAllocDefault));
-                CUDA_TRY(fn, cudaHostAlloc((void **)&plan->h_flags, n_chunks * sizeof(unsigned),
-                                 cudaHostAllocMapped));
-                plan->stream_chunks = n_chunks;
-        }
+        int n_fields;
+        CUDA_TRY(fn, stage_fields(plan, n, fields, &d_fields, &n_fields));
+        CUDA_TRY(fn, grow(&plan->stream_chunks, n_chunks,
+                         { { (void **)&plan->d_stream_state, (n_chunks + 2) * sizeof(unsigned long long) },
+                             { (void **)&plan->h_marks, (n_chunks + 1) * sizeof(unsigned long long),
+                                 cudaHostAllocDefault },
+                             { (void **)&plan->h_flags, n_chunks * sizeof(unsigned), cudaHostAllocMapped } }));
         cudaStream_t compute = plan->stream[0], h2d = plan->stream[1];
         for (int j = 0; j < N_DRAINS; j++)
                 if (plan->drain[j] == NULL)
                         CUDA_TRY(fn, cudaStreamCreateWithFlags(&plan->drain[j], cudaStreamNonBlocking));
-        unsigned long long * d_counters = plan->d_counters + CTR * 0;
         /* both arrays start on a 256-byte boundary and a chunk is a multiple of 128 bytes:
          * no cache line holds rays of two chunks */
         double * d_pos = plan->d_all_in;
-        double * d_dir = (plan->d_all_in != NULL) ? plan->d_all_in + (3 * n + 31) / 32 * 32 : NULL;
+        double * d_dir = plan->d_all_in + (3 * n + 31) / 32 * 32;
         StreamState st;
-        st.chunk_shift = chunk_shift;
+        st.chunk_shift = STREAM_CHUNK_SHIFT;
         st.watermark = plan->d_stream_state;
         st.chunk_done = (unsigned *)(plan->d_stream_state + 1);
         CUDA_TRY(fn, cudaHostGetDevicePointer((void **)&st.chunk_flags, plan->h_flags, 0));
@@ -3600,17 +3666,8 @@ static enum turtle_return trace_streamed(turtle_function_t * fn, struct turtle_p
                          (n_chunks + 2) * sizeof(unsigned long long), compute));
         CUDA_TRY(fn, cudaEventRecord(plan->ev_reset, compute));
         CUDA_TRY(fn, cudaStreamWaitEvent(h2d, plan->ev_reset, 0));
-        plan->counters.launches = 0;
         cudaError_t err = cudaSuccess;
-        FanTables tables;
-        if (fan != NULL) {
-                err = fan_upload(plan, 0, fan, bundle, ray0, h2d, &tables);
-                plan->h_marks[0] = n;
-                if (err == cudaSuccess)
-                        err = cudaMemcpyAsync(plan->d_stream_state, &plan->h_marks[0],
-                            sizeof(unsigned long long), cudaMemcpyHostToDevice, h2d);
-        }
-        for (size_t k = 0; (fan == NULL) && (k < n_chunks) && (err == cudaSuccess); k++) {
+        for (size_t k = 0; (k < n_chunks) && (err == cudaSuccess); k++) {
                 const size_t i0 = k * chunk;
                 const size_t m = std::min(chunk, n - i0);
                 plan->h_marks[k] = i0 + m;
@@ -3629,13 +3686,12 @@ static enum turtle_return trace_streamed(turtle_function_t * fn, struct turtle_p
                     "CUDA error in the streamed trace: %s", cudaGetErrorString(err));
         }
         CUDA_TRY(fn, cudaEventRecord(plan->ev0[0], compute));
-        const DeviceIo io = { (fan == NULL) ? d_pos : NULL, (fan == NULL) ? d_dir : NULL,
-                (fan != NULL) ? &tables : NULL, (results != NULL) ? plan->d_all_out : NULL,
+        const DeviceIo io = { d_pos, d_dir, NULL, (results != NULL) ? plan->d_all_out : NULL,
                 (n_fields > 0) ? &d_fields : NULL };
-        err = launch_trace(plan, 0, n, io, rule, d_counters, compute, &st);
+        err = launch_trace(plan, 0, n, io, rule, plan->d_counters, compute, &st);
         if (err == cudaSuccess) err = cudaEventRecord(plan->ev1[0], compute);
         /* Drain the chunks in the order they COMPLETE (a chunk waits for its longest ray:
-         * the first chunks of a fan sorted longest-first complete late): the thread that
+         * the first chunks of a batch sorted longest-first complete late): the thread that
          * counts the last ray of a chunk raises its flag in mapped host memory, this thread
          * watches the flags and queues the copies, round robin on N_DRAINS streams. */
         std::vector<char> drained(n_chunks, 0);
@@ -3648,15 +3704,8 @@ static enum turtle_return trace_streamed(turtle_function_t * fn, struct turtle_p
                         if (!kernel_over && (*(volatile unsigned *)(plan->h_flags + k) == 0u))
                                 continue;
                         const size_t i0 = k * chunk;
-                        const size_t m = std::min(chunk, n - i0);
-                        cudaStream_t out = plan->drain[(n_chunks - remaining) % N_DRAINS];
-                        if (results != NULL)
-                                err = cudaMemcpyAsync(results + i0, plan->d_all_out + i0,
-                                    m * sizeof(turtle_trace_result), cudaMemcpyDeviceToHost, out);
-                        for (int f = 0; (f < n_fields) && (err == cudaSuccess); f++)
-                                err = cudaMemcpyAsync((char *)*specs[f].host + i0 * specs[f].bytes,
-                                    *(char **)((char *)&d_fields + specs[f].offset) + i0 * specs[f].bytes,
-                                    m * specs[f].bytes, cudaMemcpyDeviceToHost, out);
+                        err = copy_out(plan, i0, std::min(chunk, n - i0), results, fields, d_fields,
+                            plan->drain[(n_chunks - remaining) % N_DRAINS]);
                         drained[k] = 1;
                         remaining--;
                         progress = true;
@@ -3685,57 +3734,37 @@ static enum turtle_return trace_streamed(turtle_function_t * fn, struct turtle_p
         for (int j = 0; j < N_DRAINS; j++) CUDA_TRY(fn, cudaStreamSynchronize(plan->drain[j]));
         float ms = 0.f;
         cudaEventElapsedTime(&ms, plan->ev0[0], plan->ev1[0]);
-        unsigned long long c4[CTR];
-        CUDA_TRY(fn, cudaMemcpy(c4, d_counters, sizeof c4, cudaMemcpyDeviceToHost));
-        plan->counters.rays = n;
-        plan->counters.steps = c4[1];
-        plan->counters.samples = c4[2];
-        plan->counters.rebuilds = c4[4];
-        plan->counters.kernel_ms = ms;
+        unsigned long long c[CTR];
+        CUDA_TRY(fn, add_counters(plan, 0, 1, plan->counters, c));
+        plan->counters.rays += n;
+        plan->counters.kernel_ms += ms;
         plan->counters.launches += 1;
-        if (c4[3] != 0ull)
+        if (c[3] != 0ull)
                 return tbh::raise(fn, TURTLE_RETURN_LIBRARY_ERROR, BATCH_CU, __LINE__,
                     "the streamed trace timed out waiting for its rays to reach the device");
         return TURTLE_RETURN_SUCCESS;
 }
 
 /* A host-pointer call in rounds of at most STREAM_MAX_RAYS rays, which bounds the device
- * staging of a call whatever the size of the batch. */
+ * staging of a call whatever the size of the batch. The caller has reset the counters. */
 static enum turtle_return trace_rounds(turtle_function_t * fn, struct turtle_plan * plan,
-    size_t n, const double * position, const double * direction, const struct turtle_fans * fan,
-    size_t bundle, const struct turtle_trace_rule * rule, struct turtle_trace_result * results,
+    size_t n, const double * position, const double * direction,
+    const struct turtle_trace_rule * rule, struct turtle_trace_result * results,
     const struct turtle_trace_fields * fields)
 {
-        turtle_plan_counters sum;
-        memset(&sum, 0x0, sizeof(sum));
         size_t round_rays = STREAM_MAX_RAYS;
         if (getenv("TURTLE_B200_STREAM_MAX_RAYS") != NULL) { /* tests: small rounds */
                 const long long v = atoll(getenv("TURTLE_B200_STREAM_MAX_RAYS"));
                 if (v >= (long long)STREAM_CHUNK_RAYS) round_rays = (size_t)v;
         }
-        FieldSpec specs[12];
-        const int n_fields = (fields != NULL) ? field_specs(fields, specs) : 0;
         for (size_t first = 0; first < n; first += round_rays) {
-                const size_t m = std::min(round_rays, n - first);
-                struct turtle_trace_fields part;
-                memset(&part, 0x0, sizeof part);
-                for (int k = 0; k < n_fields; k++)
-                        *(void **)((char *)&part + specs[k].offset) =
-                            (char *)*specs[k].host + first * specs[k].bytes;
-                const enum turtle_return rc = trace_streamed(fn, plan, m, first,
-                    (position != NULL) ? position + 3 * first : NULL,
-                    (direction != NULL) ? direction + 3 * first : NULL, fan, bundle, rule,
-                    (results != NULL) ? results + first : NULL, (n_fields > 0) ? &part : NULL,
-                    STREAM_CHUNK_SHIFT);
+                const struct turtle_trace_fields part =
+                    (fields != NULL) ? offset_fields(*fields, first) : turtle_trace_fields();
+                const enum turtle_return rc = trace_streamed(fn, plan, std::min(round_rays, n - first),
+                    position + 3 * first, direction + 3 * first, rule,
+                    (results != NULL) ? results + first : NULL, (fields != NULL) ? &part : NULL);
                 if (rc != TURTLE_RETURN_SUCCESS) return rc;
-                sum.rays += plan->counters.rays;
-                sum.steps += plan->counters.steps;
-                sum.samples += plan->counters.samples;
-                sum.rebuilds += plan->counters.rebuilds;
-                sum.launches += plan->counters.launches;
-                sum.kernel_ms += plan->counters.kernel_ms;
         }
-        plan->counters = sum;
         return TURTLE_RETURN_SUCCESS;
 }
 
@@ -3748,38 +3777,20 @@ static enum turtle_return trace_rounds(turtle_function_t * fn, struct turtle_pla
  * head of the next (concurrent launches on one plan). Only the copy
  * of the last slice is exposed. (The streamed kernel -- chunk flags, fences, a lane-side
  * watermark -- does the same at 5 % more kernel time; it stays the path of calls that
- * must stream rays in.) */
+ * must stream rays in.) The call adds its counts to the plan's counters, which the caller
+ * has reset. */
 static enum turtle_return trace_fan_sliced(turtle_function_t * fn, struct turtle_plan * plan,
     size_t n, const struct turtle_fans * fan, size_t bundle, const struct turtle_trace_rule * rule,
     struct turtle_trace_result * results, const struct turtle_trace_fields * fields)
 {
+        CUDA_TRY(fn, cudaSetDevice(plan->device));
         CUDA_TRY(fn, plan_pipeline(plan, 1)); /* the streams and their events */
-        if ((results != NULL) && (plan->all_records < n)) {
-                cudaFree(plan->d_all_out);
-                plan->d_all_out = NULL;
-                plan->all_records = 0;
-                CUDA_TRY(fn, cudaMalloc((void **)&plan->d_all_out, n * sizeof(turtle_trace_result)));
-                plan->all_records = n;
-        }
-        FieldSpec specs[12];
-        const int n_fields = (fields != NULL) ? field_specs(fields, specs) : 0;
-        char * d_field[12] = { NULL };
-        if (n_fields > 0) {
-                size_t need = 0;
-                for (int k = 0; k < n_fields; k++) need += (n * specs[k].bytes + 255) / 256 * 256;
-                if (plan->field_pool_bytes < need) {
-                        cudaFree(plan->d_field_pool);
-                        plan->d_field_pool = NULL;
-                        plan->field_pool_bytes = 0;
-                        CUDA_TRY(fn, cudaMalloc(&plan->d_field_pool, need));
-                        plan->field_pool_bytes = need;
-                }
-                size_t at = 0;
-                for (int k = 0; k < n_fields; k++) {
-                        d_field[k] = (char *)plan->d_field_pool + at;
-                        at += (n * specs[k].bytes + 255) / 256 * 256;
-                }
-        }
+        if (results != NULL)
+                CUDA_TRY(fn, grow(&plan->all_records, n,
+                                 { { (void **)&plan->d_all_out, n * sizeof(turtle_trace_result) } }));
+        struct turtle_trace_fields d_fields;
+        int n_fields;
+        CUDA_TRY(fn, stage_fields(plan, n, fields, &d_fields, &n_fields));
         /* slices: whole bands of the fan (bundle x n_azimuth rays), about 2 Mi rays each */
         const size_t band = std::max<size_t>(bundle * fan->n_azimuth, 1);
         size_t slice_rays = (size_t)1 << 21;
@@ -3798,29 +3809,18 @@ static enum turtle_return trace_fan_sliced(turtle_function_t * fn, struct turtle
         CUDA_TRY(fn, cudaStreamWaitEvent(lanes[1], plan->ev0[0], 0));
         /* a host-pointer call: counter blocks of its own, none of the device-pointer ring */
         unsigned long long * d_counters = plan->d_counters + CTR * ALL_SLOTS;
-        plan->counters.launches = 0;
         for (size_t k = 0; k < n_slices; k++) {
                 const size_t first = k * per_slice;
                 const size_t m = std::min(per_slice, n - first);
                 cudaStream_t st = lanes[k & 1];
                 FanTables slice = tables;
                 slice.ray0 = first;
-                struct turtle_trace_fields d_fields;
-                memset(&d_fields, 0x0, sizeof d_fields);
-                for (int f = 0; f < n_fields; f++)
-                        *(void **)((char *)&d_fields + specs[f].offset) =
-                            d_field[f] + first * specs[f].bytes;
+                const struct turtle_trace_fields slice_fields = offset_fields(d_fields, first);
                 const DeviceIo io = { NULL, NULL, &slice,
                         (results != NULL) ? plan->d_all_out + first : NULL,
-                        (n_fields > 0) ? &d_fields : NULL };
+                        (n_fields > 0) ? &slice_fields : NULL };
                 CUDA_TRY(fn, launch_trace(plan, 0, m, io, rule, d_counters + CTR * k, st));
-                if (results != NULL)
-                        CUDA_TRY(fn, cudaMemcpyAsync(results + first, plan->d_all_out + first,
-                                         m * sizeof(turtle_trace_result), cudaMemcpyDeviceToHost, st));
-                for (int f = 0; f < n_fields; f++)
-                        CUDA_TRY(fn, cudaMemcpyAsync((char *)*specs[f].host + first * specs[f].bytes,
-                                         d_field[f] + first * specs[f].bytes, m * specs[f].bytes,
-                                         cudaMemcpyDeviceToHost, st));
+                CUDA_TRY(fn, copy_out(plan, first, m, results, fields, d_fields, st));
         }
         CUDA_TRY(fn, cudaEventRecord(plan->ev1[0], lanes[0]));
         CUDA_TRY(fn, cudaEventRecord(plan->ev1[1], lanes[1]));
@@ -3830,17 +3830,8 @@ static enum turtle_return trace_fan_sliced(turtle_function_t * fn, struct turtle
         cudaEventElapsedTime(&ms, plan->ev0[0], plan->ev1[0]);
         cudaEventElapsedTime(&ms1, plan->ev0[0], plan->ev1[1]);
         if (ms1 > ms) ms = ms1;
-        const uint64_t launches = plan->counters.launches;
-        memset(&plan->counters, 0x0, sizeof(plan->counters));
-        for (size_t k = 0; k < n_slices; k++) {
-                unsigned long long c[CTR];
-                CUDA_TRY(fn, cudaMemcpy(c, d_counters + CTR * k, sizeof c, cudaMemcpyDeviceToHost));
-                plan->counters.steps += c[1];
-                plan->counters.samples += c[2];
-                plan->counters.rebuilds += c[4];
-        }
+        CUDA_TRY(fn, add_counters(plan, ALL_SLOTS, (int)n_slices, plan->counters));
         plan->counters.rays = n;
-        plan->counters.launches = launches;
         plan->counters.kernel_ms = ms;
         return TURTLE_RETURN_SUCCESS;
 }
@@ -3855,35 +3846,20 @@ static enum turtle_return check_plan(turtle_function_t * fn, const struct turtle
         return TURTLE_RETURN_SUCCESS;
 }
 
-/* The n > 0 rays of checked fans, host-pointer results. */
-static enum turtle_return trace_fans_host(turtle_function_t * fn, struct turtle_plan * plan,
-    const struct turtle_fans * fans, size_t n, size_t bundle, const struct turtle_trace_rule * rule,
-    struct turtle_trace_result * results, const struct turtle_trace_fields * fields)
-{
-        CUDA_TRY(fn, cudaSetDevice(plan->device));
-        if (getenv("TURTLE_B200_FAN_STREAMED") != NULL) /* development: the streamed kernel */
-                return trace_rounds(fn, plan, n, NULL, NULL, fans, bundle, rule, results, fields);
-        return trace_fan_sliced(fn, plan, n, fans, bundle, rule, results, fields);
-}
-
 /* The n > 0 rays of checked fans, device-pointer results: ONE launch, asynchronous. */
 static enum turtle_return trace_fans_device(turtle_function_t * fn, struct turtle_plan * plan,
     const struct turtle_fans * fans, size_t n, size_t bundle, const struct turtle_trace_rule * rule,
     struct turtle_trace_result * results, const struct turtle_trace_fields * fields, void * stream)
 {
-        CUDA_TRY(fn, cudaSetDevice(plan->device));
-        memset(&plan->counters, 0x0, sizeof(plan->counters));
-        plan->counters.rays = n;
-        int slot;
-        CUDA_TRY(fn, next_device_slot(plan, &slot));
-        FanTables tables;
-        cudaError_t err = fan_upload(plan, slot, fans, bundle, 0, (cudaStream_t)stream, &tables);
-        const DeviceIo io = { NULL, NULL, &tables, results, fields };
-        if (err == cudaSuccess)
-                err = launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
-                    (cudaStream_t)stream);
-        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
-        return TURTLE_RETURN_SUCCESS;
+        return device_call(fn, plan, true, n, (cudaStream_t)stream, [&](int slot) {
+                FanTables tables;
+                cudaError_t err = fan_upload(plan, slot, fans, bundle, 0, (cudaStream_t)stream, &tables);
+                const DeviceIo io = { NULL, NULL, &tables, results, fields };
+                if (err == cudaSuccess)
+                        err = launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
+                            (cudaStream_t)stream);
+                return err;
+        });
 }
 
 extern "C" enum turtle_return turtle_stepper_trace_fan(struct turtle_plan * plan,
@@ -3899,7 +3875,7 @@ extern "C" enum turtle_return turtle_stepper_trace_fan(struct turtle_plan * plan
         memset(&plan->counters, 0x0, sizeof(plan->counters));
         if (n == 0) return TURTLE_RETURN_SUCCESS;
         const struct turtle_fans fans = one_station(fan);
-        return trace_fans_host(fn, plan, &fans, n, bundle, rule, results, fields);
+        return trace_fan_sliced(fn, plan, n, &fans, bundle, rule, results, fields);
 }
 
 extern "C" enum turtle_return turtle_stepper_trace_fan_device(struct turtle_plan * plan,
@@ -3931,7 +3907,7 @@ extern "C" enum turtle_return turtle_stepper_trace_fans(struct turtle_plan * pla
         rc = check_plan(fn, plan);
         if (rc != TURTLE_RETURN_SUCCESS) return rc;
         memset(&plan->counters, 0x0, sizeof(plan->counters));
-        return trace_fans_host(fn, plan, fans, n, bundle, rule, results, fields);
+        return trace_fan_sliced(fn, plan, n, fans, bundle, rule, results, fields);
 }
 
 extern "C" enum turtle_return turtle_stepper_trace_fans_device(struct turtle_plan * plan,
@@ -3960,7 +3936,7 @@ extern "C" enum turtle_return turtle_stepper_trace_fields(struct turtle_plan * p
         memset(&plan->counters, 0x0, sizeof(plan->counters));
         if (n == 0) return TURTLE_RETURN_SUCCESS;
         CUDA_TRY(fn, cudaSetDevice(plan->device));
-        return trace_rounds(fn, plan, n, position, direction, NULL, 1, rule, NULL, fields);
+        return trace_rounds(fn, plan, n, position, direction, rule, NULL, fields);
 }
 
 extern "C" enum turtle_return turtle_stepper_trace_fields_device(struct turtle_plan * plan,
@@ -3972,16 +3948,11 @@ extern "C" enum turtle_return turtle_stepper_trace_fields_device(struct turtle_p
         enum turtle_return rc = check_rule(fn, rule);
         if (rc != TURTLE_RETURN_SUCCESS) return rc;
         if (n == 0) return TURTLE_RETURN_SUCCESS;
-        CUDA_TRY(fn, cudaSetDevice(plan->device));
-        memset(&plan->counters, 0x0, sizeof(plan->counters));
-        plan->counters.rays = n;
-        int slot;
-        CUDA_TRY(fn, next_device_slot(plan, &slot));
         const DeviceIo io = { position, direction, NULL, NULL, fields };
-        const cudaError_t err = launch_trace(plan, slot, n, io, rule,
-            plan->d_counters + CTR * slot, (cudaStream_t)stream);
-        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
-        return TURTLE_RETURN_SUCCESS;
+        return device_call(fn, plan, true, n, (cudaStream_t)stream, [&](int slot) {
+                return launch_trace(plan, slot, n, io, rule, plan->d_counters + CTR * slot,
+                    (cudaStream_t)stream);
+        });
 }
 
 /* ---- the horizon of a station ---------------------------------------------------------- */
@@ -4015,7 +3986,6 @@ static cudaError_t launch_horizon(struct turtle_plan * plan, int slot, size_t n_
     const double * azimuth, double elevation_min, double elevation_max, double tolerance,
     const struct turtle_trace_rule * rule, struct turtle_horizon * results, cudaStream_t stream)
 {
-        memset(&plan->counters, 0x0, sizeof(plan->counters));
         unsigned long long * d_counters = plan->d_counters + CTR * slot;
         struct turtle_fans fans;
         memset(&fans, 0x0, sizeof fans);
@@ -4052,14 +4022,12 @@ static cudaError_t launch_horizon(struct turtle_plan * plan, int slot, size_t n_
         const int per_sm = trace_grid(plan, 0, &blocks, &threads);
         const size_t warps = (size_t)threads / 32;
         blocks = (int)std::min<size_t>((size_t)plan->sm_count * per_sm, (items + warps - 1) / warps);
-        const auto [lla, proj, stack_shape] = variant_of(plan);
-        void (*kernel)(const tb::Geometry, const HorizonArgs) =
-            stack_shape ? horizon_kernel<false, false, 6, tb::SHAPE_STACK> :
-            (lla && proj) ? horizon_kernel<true, true, 4, tb::SHAPE_GENERIC> :
-            lla ? horizon_kernel<true, false, 4, tb::SHAPE_GENERIC> :
-            proj ? horizon_kernel<false, true, 6, tb::SHAPE_GENERIC> :
-                   horizon_kernel<false, false, 6, tb::SHAPE_GENERIC>;
-        const size_t dynamic = lla ? lla_bytes(plan) : 0;
+        const Variant v = variant_of(plan);
+        void (*kernel)(const tb::Geometry, const HorizonArgs) = with_variant(v, [](auto V) {
+                typedef decltype(V) K;
+                return horizon_kernel<K::LLA, K::PROJ, K::MINB, K::SHAPE>;
+        });
+        const size_t dynamic = v.lla ? lla_bytes(plan) : 0;
         if (dynamic > 0)
                 cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dynamic);
         kernel<<<blocks, threads, dynamic, stream>>>(plan->G, A);
@@ -4074,14 +4042,12 @@ static enum turtle_return horizons_device(turtle_function_t * fn, struct turtle_
     double tolerance, const struct turtle_trace_rule * rule, struct turtle_horizon * results,
     void * stream)
 {
-        CUDA_TRY(fn, cudaSetDevice(plan->device));
-        int slot;
-        CUDA_TRY(fn, next_device_slot(plan, &slot));
-        const cudaError_t err = launch_horizon(plan, slot, n_station, latitude, longitude, position,
-            n_azimuth, azimuth, elevation_min, elevation_max, tolerance, rule, results,
-            (cudaStream_t)stream);
-        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
-        return TURTLE_RETURN_SUCCESS;
+        /* the counters report the probes, read back by turtle_plan_counters_sync */
+        return device_call(fn, plan, true, 0, (cudaStream_t)stream, [&](int slot) {
+                return launch_horizon(plan, slot, n_station, latitude, longitude, position,
+                    n_azimuth, azimuth, elevation_min, elevation_max, tolerance, rule, results,
+                    (cudaStream_t)stream);
+        });
 }
 
 /* Checked arguments, items > 0: host-pointer results. */
@@ -4091,15 +4057,15 @@ static enum turtle_return horizons_host(turtle_function_t * fn, struct turtle_pl
     double tolerance, const struct turtle_trace_rule * rule, struct turtle_horizon * results)
 {
         CUDA_TRY(fn, cudaSetDevice(plan->device));
-        struct turtle_horizon * d_results = NULL;
+        DeviceBuffers buf;
+        struct turtle_horizon * d_results;
         const size_t bytes = n_station * n_azimuth * sizeof(*d_results);
-        CUDA_TRY(fn, cudaMalloc((void **)&d_results, bytes));
+        CUDA_TRY(fn, buf.get((void **)&d_results, NULL, bytes, false));
         /* a host-pointer call: the counter block and tables of the host pipeline's slot 0 */
-        cudaError_t err = launch_horizon(plan, 0, n_station, latitude, longitude, position,
-            n_azimuth, azimuth, elevation_min, elevation_max, tolerance, rule, d_results, NULL);
-        if (err == cudaSuccess) err = cudaMemcpy(results, d_results, bytes, cudaMemcpyDeviceToHost);
-        cudaFree(d_results);
-        CUDA_TRY(fn, err);
+        memset(&plan->counters, 0x0, sizeof(plan->counters));
+        CUDA_TRY(fn, launch_horizon(plan, 0, n_station, latitude, longitude, position, n_azimuth,
+                         azimuth, elevation_min, elevation_max, tolerance, rule, d_results, NULL));
+        CUDA_TRY(fn, cudaMemcpy(results, d_results, bytes, cudaMemcpyDeviceToHost));
         read_counters(plan, 0);
         return TURTLE_RETURN_SUCCESS;
 }
@@ -4171,20 +4137,13 @@ extern "C" enum turtle_return turtle_stepper_trace_batch(
          * call (144 bytes per ray) to 4.6 GB whatever the size of the batch */
         if ((plan->schedule == 0) && (plan->pipeline_mode != 1) && (n > STREAM_CHUNK_RAYS))
                 return trace_rounds(FN(&turtle_stepper_trace_batch), plan, n, position, direction,
-                    NULL, 1, rule, results, NULL);
-        size_t chunk_rays = CHUNK_RAYS;
-        if (getenv("TURTLE_B200_CHUNK_RAYS") != NULL) { /* development: pipeline sweep */
-                const long long v = atoll(getenv("TURTLE_B200_CHUNK_RAYS"));
-                if (v >= 1024) chunk_rays = (size_t)v;
-        }
-        const size_t chunk = std::min(n, chunk_rays);
+                    rule, results, NULL);
+        const size_t chunk = std::min(n, CHUNK_RAYS);
         CUDA_TRY(&turtle_stepper_trace_batch, plan_pipeline(plan, chunk));
 
         /* chunked 3-deep pipeline: H2D(c+1) | kernel(c) | D2H(c-1) on 3 streams */
         const size_t n_chunks = (n + chunk - 1) / chunk;
-        std::vector<unsigned long long> totals(CTR, 0ull);
         double kernel_ms = 0.;
-        unsigned long long c4[CTR];
         for (size_t c = 0; c < n_chunks + N_SLOTS; c++) {
                 const int s = (int)(c % N_SLOTS);
                 if (c >= N_SLOTS) { /* drain the slot before reusing it */
@@ -4192,12 +4151,7 @@ extern "C" enum turtle_return turtle_stepper_trace_batch(
                         float ms = 0.f;
                         cudaEventElapsedTime(&ms, plan->ev0[s], plan->ev1[s]);
                         kernel_ms += ms;
-                        CUDA_TRY(&turtle_stepper_trace_batch,
-                            cudaMemcpy(c4, plan->d_counters + CTR * s, sizeof c4,
-                                cudaMemcpyDeviceToHost));
-                        totals[1] += c4[1];
-                        totals[2] += c4[2];
-                        totals[4] += c4[4];
+                        CUDA_TRY(&turtle_stepper_trace_batch, add_counters(plan, s, 1, plan->counters));
                 }
                 if (c >= n_chunks) continue;
                 const size_t i0 = c * chunk;
@@ -4221,9 +4175,6 @@ extern "C" enum turtle_return turtle_stepper_trace_batch(
                         m * sizeof(turtle_trace_result), cudaMemcpyDeviceToHost, st));
         }
         plan->counters.rays = n;
-        plan->counters.steps = totals[1];
-        plan->counters.samples = totals[2];
-        plan->counters.rebuilds = totals[4];
         plan->counters.kernel_ms = kernel_ms;
         return TURTLE_RETURN_SUCCESS;
 }
@@ -4287,20 +4238,24 @@ extern "C" enum turtle_return turtle_states_reset(struct turtle_states * states)
         return TURTLE_RETURN_SUCCESS;
 }
 
-/* Launch the walk kernel: n particles, n_steps turtle_stepper_step each (1: the step_batch
- * calls, states used in place; > 1: turtle_stepper_walk_batch, state resident in the lane
- * store for the whole launch). A device-pointer call (`ring`) takes its counter block from
- * the ring of in-flight calls, a host-pointer call uses the one of the host pipeline. */
-static enum turtle_return launch_walk(turtle_function_t * fn, struct turtle_plan * plan,
-    struct turtle_states * states, size_t n, int n_steps, bool multi, double * position,
-    const double * direction, double * latitude, double * longitude, double * altitude,
-    double * elevation, double * step, int * index, void * stream, bool ring)
+/* The states, if any, of a call of n particles on `plan`. */
+static enum turtle_return check_states(turtle_function_t * fn, const struct turtle_plan * plan,
+    const struct turtle_states * states, size_t n)
 {
         if ((states != NULL) && ((states->plan != plan) || (states->n < n)))
                 return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
                     "states do not match the plan or are too few");
-        if (n == 0) return TURTLE_RETURN_SUCCESS;
-        CUDA_TRY(fn, cudaSetDevice(plan->device));
+        return TURTLE_RETURN_SUCCESS;
+}
+
+/* Queue the walk kernel on `stream` with the counter block of `slot`: n particles, n_steps
+ * turtle_stepper_step each (1: the step_batch calls, states used in place; > 1:
+ * turtle_stepper_walk_batch, state resident in the lane store for the whole launch). */
+static cudaError_t launch_walk(struct turtle_plan * plan, int slot, struct turtle_states * states,
+    size_t n, int n_steps, bool multi, double * position, const double * direction,
+    double * latitude, double * longitude, double * altitude, double * elevation, double * step,
+    int * index, cudaStream_t stream)
+{
         StepArgs A;
         A.n = n;
         A.states = (states != NULL) ? states->d_states : NULL;
@@ -4314,40 +4269,26 @@ static enum turtle_return launch_walk(turtle_function_t * fn, struct turtle_plan
         A.step = step;
         A.index = index;
         A.n_steps = n_steps;
-        int slot = 0;
-        if (ring) CUDA_TRY(fn, next_device_slot(plan, &slot));
         A.counters = plan->d_counters + CTR * slot;
         const int threads = 128;
         int blocks = (int)std::min<size_t>((n + threads - 1) / threads,
             (size_t)plan->sm_count * 5);
-        cudaStream_t st = (cudaStream_t)stream;
-        cudaError_t err = cudaMemsetAsync(A.counters, 0x0, CTR * sizeof(unsigned long long), st);
-        if (err != cudaSuccess) {
-                if (ring) release_device_slot(plan, slot, st, err);
-                CUDA_TRY(fn, err);
-        }
-        const auto [lla, proj, stack_shape] = variant_of(plan); /* (no walk kernel for the stack shape) */
-        (void)stack_shape;
-        /* the CTAs per SM get the carve-out they need and no more: the rest is L1 for the
-         * DEM gathers (as for the trace kernel) */
-        void (*kernel)(const tb::Geometry, const StepArgs);
-        if (multi)
-                kernel = (lla && proj) ? walk_kernel<true, true, true, true> :
-                    (lla ? walk_kernel<true, false, true, true> :
-                           (proj ? walk_kernel<false, true, true, true> :
-                                   walk_kernel<false, false, true, true>));
-        else if (states != NULL)
-                kernel = (lla && proj) ? walk_kernel<true, true, true> :
-                    (lla ? walk_kernel<true, false, true> :
-                           (proj ? walk_kernel<false, true, true> : walk_kernel<false, false, true>));
-        else
-                kernel = (lla && proj) ? walk_kernel<true, true, false> :
-                    (lla ? walk_kernel<true, false, false> :
-                           (proj ? walk_kernel<false, true, false> : walk_kernel<false, false, false>));
+        cudaError_t err = cudaMemsetAsync(A.counters, 0x0, CTR * sizeof(unsigned long long), stream);
+        if (err != cudaSuccess) return err;
+        Variant v = variant_of(plan);
+        v.stack_shape = false; /* no walk kernel for the stack shape: the generic ones */
+        void (*kernel)(const tb::Geometry, const StepArgs) = with_variant(v, [&](auto V) {
+                typedef decltype(V) K;
+                return multi ? walk_kernel<K::LLA, K::PROJ, true, true> :
+                    (states != NULL) ? walk_kernel<K::LLA, K::PROJ, true> :
+                                       walk_kernel<K::LLA, K::PROJ, false>;
+        });
         /* the local approximations live in the device states (one step), else in dynamic
          * shared memory (no states: every particle starts from a reset stepper; several
          * steps: the state moves in and out once) */
-        const size_t dynamic = (lla && (multi || (states == NULL))) ? lla_bytes(plan) : 0;
+        const size_t dynamic = (v.lla && (multi || (states == NULL))) ? lla_bytes(plan) : 0;
+        /* the CTAs per SM get the carve-out they need and no more: the rest is L1 for the
+         * DEM gathers (as for the trace kernel) */
         cudaFuncAttributes attr;
         if (cudaFuncGetAttributes(&attr, kernel) == cudaSuccess) {
                 const size_t cta = attr.sharedSizeBytes + dynamic + 1024;
@@ -4363,14 +4304,11 @@ static enum turtle_return launch_walk(turtle_function_t * fn, struct turtle_plan
                 cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
                     (int)dynamic);
         cudaGetLastError();
-        kernel<<<blocks, threads, dynamic, st>>>(plan->G, A);
+        kernel<<<blocks, threads, dynamic, stream>>>(plan->G, A);
         plan->counters.launches++;
         plan->counters.rays = n;
         plan->counters.steps = (direction != NULL) ? n * (size_t)n_steps : 0;
-        err = cudaGetLastError();
-        if (ring) err = release_device_slot(plan, slot, st, err);
-        CUDA_TRY(fn, err);
-        return TURTLE_RETURN_SUCCESS;
+        return cudaGetLastError();
 }
 
 extern "C" enum turtle_return turtle_stepper_step_batch_device(
@@ -4379,9 +4317,14 @@ extern "C" enum turtle_return turtle_stepper_step_batch_device(
     double * longitude, double * altitude, double * elevation, double * step,
     int * index, void * stream)
 {
-        return launch_walk(FN(&turtle_stepper_step_batch_device), plan, states, n, 1, false,
-            position, direction, latitude, longitude, altitude, elevation, step, index, stream,
-            true);
+        turtle_function_t * fn = FN(&turtle_stepper_step_batch_device);
+        const enum turtle_return rc = check_states(fn, plan, states, n);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        /* the counters of a walk are not reset: launch_walk sets its rays and steps */
+        return device_call(fn, plan, false, 0, (cudaStream_t)stream, [&](int slot) {
+                return launch_walk(plan, slot, states, n, 1, false, position, direction, latitude,
+                    longitude, altitude, elevation, step, index, (cudaStream_t)stream);
+        });
 }
 
 /* n_steps successive turtle_stepper_step per particle in one launch (turtle_b200.h). */
@@ -4394,30 +4337,12 @@ extern "C" enum turtle_return turtle_stepper_walk_batch_device(struct turtle_pla
         if ((n_steps < 1) || (direction == NULL))
                 return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
                     "a walk needs at least one step and its directions");
-        return launch_walk(fn, plan, states, n, n_steps, true, position, direction, latitude,
-            longitude, altitude, elevation, step, index, stream, true);
-}
-
-/* Small RAII helper for the host-pointer wrappers of the simple kernels. */
-namespace {
-struct DeviceBuffers {
-        std::vector<void *> ptrs;
-        ~DeviceBuffers()
-        {
-                for (size_t i = 0; i < ptrs.size(); i++) cudaFree(ptrs[i]);
-        }
-        /* allocate `bytes` and optionally copy from host; NULL host + copy_in=false = output */
-        cudaError_t get(void ** dev, const void * host, size_t bytes, bool copy_in)
-        {
-                *dev = NULL;
-                cudaError_t err = cudaMalloc(dev, std::max<size_t>(bytes, 8));
-                if (err != cudaSuccess) return err;
-                ptrs.push_back(*dev);
-                if (copy_in && (host != NULL) && bytes)
-                        err = cudaMemcpy(*dev, host, bytes, cudaMemcpyHostToDevice);
-                return err;
-        }
-};
+        const enum turtle_return rc = check_states(fn, plan, states, n);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        return device_call(fn, plan, false, 0, (cudaStream_t)stream, [&](int slot) {
+                return launch_walk(plan, slot, states, n, n_steps, true, position, direction,
+                    latitude, longitude, altitude, elevation, step, index, (cudaStream_t)stream);
+        });
 }
 
 #define DEV_IN(fn, B, dptr, hptr, bytes)                                           \
@@ -4535,13 +4460,7 @@ static cudaError_t launch_voxels(struct turtle_plan * plan, int slot, size_t n,
         A.direction = d_direction;
         if (fan != NULL) {
                 A.position = A.direction = NULL;
-                A.fan.fan_az = fan->az;
-                A.fan.fan_el = fan->el;
-                A.fan.fan_station = fan->station;
-                A.fan.fan_naz = fan->naz;
-                A.fan.fan_bundle = fan->bundle;
-                A.fan.fan_per_station = fan->per_station;
-                A.fan.fan_ray0 = fan->ray0;
+                A.fan.fan = *fan;
         }
         A.results = results;
         A.entries = entries;
@@ -4560,14 +4479,12 @@ static cudaError_t launch_voxels(struct turtle_plan * plan, int slot, size_t n,
                 A.size[a] = grid->size[a];
                 A.cells[a] = grid->n[a];
         }
-        const auto [lla, proj, stack_shape] = variant_of(plan);
-        void (*kernel)(const tb::Geometry, const VoxelArgs) =
-            stack_shape ? voxel_kernel<false, false, 6, tb::SHAPE_STACK> :
-            (lla && proj) ? voxel_kernel<true, true, 4, tb::SHAPE_GENERIC> :
-            lla ? voxel_kernel<true, false, 4, tb::SHAPE_GENERIC> :
-            proj ? voxel_kernel<false, true, 6, tb::SHAPE_GENERIC> :
-                   voxel_kernel<false, false, 6, tb::SHAPE_GENERIC>;
-        const size_t dynamic = lla ? lla_bytes(plan) : 0;
+        const Variant v = variant_of(plan);
+        void (*kernel)(const tb::Geometry, const VoxelArgs) = with_variant(v, [](auto V) {
+                typedef decltype(V) K;
+                return voxel_kernel<K::LLA, K::PROJ, K::MINB, K::SHAPE>;
+        });
+        const size_t dynamic = v.lla ? lla_bytes(plan) : 0;
         if (dynamic > 0)
                 cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dynamic);
         /* the grid of the trace kernels, at most the CTAs that fit an SM with the rows of the
@@ -4629,19 +4546,16 @@ static enum turtle_return voxels_device(turtle_function_t * fn, struct turtle_pl
     struct turtle_trace_result * results, struct turtle_voxel_entry * entries, int capacity,
     int32_t * count, void * stream)
 {
-        CUDA_TRY(fn, cudaSetDevice(plan->device));
-        memset(&plan->counters, 0x0, sizeof(plan->counters));
-        plan->counters.rays = n;
-        int slot;
-        CUDA_TRY(fn, next_device_slot(plan, &slot));
-        FanTables T;
-        cudaError_t err = cudaSuccess;
-        if (fans != NULL) err = fan_upload(plan, slot, fans, bundle, 0, (cudaStream_t)stream, &T);
-        if (err == cudaSuccess)
-                err = launch_voxels(plan, slot, n, position, direction, (fans != NULL) ? &T : NULL,
-                    rule, grid, results, entries, capacity, count, (cudaStream_t)stream);
-        CUDA_TRY(fn, release_device_slot(plan, slot, (cudaStream_t)stream, err));
-        return TURTLE_RETURN_SUCCESS;
+        return device_call(fn, plan, true, n, (cudaStream_t)stream, [&](int slot) {
+                FanTables T;
+                cudaError_t err = cudaSuccess;
+                if (fans != NULL) err = fan_upload(plan, slot, fans, bundle, 0, (cudaStream_t)stream, &T);
+                if (err == cudaSuccess)
+                        err = launch_voxels(plan, slot, n, position, direction,
+                            (fans != NULL) ? &T : NULL, rule, grid, results, entries, capacity, count,
+                            (cudaStream_t)stream);
+                return err;
+        });
 }
 
 extern "C" enum turtle_return turtle_stepper_trace_voxels(struct turtle_plan * plan, size_t n,
@@ -4755,6 +4669,8 @@ extern "C" enum turtle_return turtle_stepper_step_batch(struct turtle_plan * pla
     double * altitude, double * elevation, double * step, int * index)
 {
         if (n == 0) return TURTLE_RETURN_SUCCESS;
+        const enum turtle_return rc = check_states(FN(&turtle_stepper_step_batch), plan, states, n);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
         CUDA_TRY(&turtle_stepper_step_batch, cudaSetDevice(plan->device));
         DeviceBuffers B;
         double *d_pos, *d_dir = NULL, *d_lat, *d_lon, *d_alt, *d_el, *d_step;
@@ -4768,9 +4684,8 @@ extern "C" enum turtle_return turtle_stepper_step_batch(struct turtle_plan * pla
         DEV_OUT(&turtle_stepper_step_batch, B, d_el, elevation, n * 2 * sizeof(double));
         DEV_OUT(&turtle_stepper_step_batch, B, d_step, step, n * sizeof(double));
         DEV_OUT(&turtle_stepper_step_batch, B, d_idx, index, n * 2 * sizeof(int));
-        enum turtle_return rc = launch_walk(FN(&turtle_stepper_step_batch), plan, states, n, 1,
-            false, d_pos, d_dir, d_lat, d_lon, d_alt, d_el, d_step, d_idx, NULL, false);
-        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        CUDA_TRY(&turtle_stepper_step_batch, launch_walk(plan, 0, states, n, 1, false, d_pos,
+                                                 d_dir, d_lat, d_lon, d_alt, d_el, d_step, d_idx, NULL));
         CUDA_TRY(&turtle_stepper_step_batch, cudaDeviceSynchronize());
         if (direction != NULL)
                 DEV_BACK(&turtle_stepper_step_batch, position, d_pos, n * 3 * sizeof(double));
@@ -4793,6 +4708,8 @@ extern "C" enum turtle_return turtle_stepper_walk_batch(struct turtle_plan * pla
                 return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
                     "a walk needs at least one step and its directions");
         if (n == 0) return TURTLE_RETURN_SUCCESS;
+        const enum turtle_return rc = check_states(fn, plan, states, n);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
         CUDA_TRY(fn, cudaSetDevice(plan->device));
         const size_t m = n * (size_t)n_steps;
         DeviceBuffers B;
@@ -4806,9 +4723,8 @@ extern "C" enum turtle_return turtle_stepper_walk_batch(struct turtle_plan * pla
         DEV_OUT(fn, B, d_el, elevation, m * 2 * sizeof(double));
         DEV_OUT(fn, B, d_step, step, m * sizeof(double));
         DEV_OUT(fn, B, d_idx, index, m * 2 * sizeof(int));
-        enum turtle_return rc = launch_walk(fn, plan, states, n, n_steps, true, d_pos, d_dir,
-            d_lat, d_lon, d_alt, d_el, d_step, d_idx, NULL, false);
-        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        CUDA_TRY(fn, launch_walk(plan, 0, states, n, n_steps, true, d_pos, d_dir, d_lat, d_lon,
+                         d_alt, d_el, d_step, d_idx, NULL));
         CUDA_TRY(fn, cudaDeviceSynchronize());
         DEV_BACK(fn, position, d_pos, n * 3 * sizeof(double));
         DEV_BACK(fn, latitude, d_lat, m * sizeof(double));
