@@ -99,7 +99,8 @@ struct turtle_plan_counters {
 
 /* Threading: a plan carries the streams, staging buffers and counters of the calls made
  * through it, and is used from one host thread at a time. HOST-pointer calls (`*_batch`,
- * `_trace_fan[s]`, `_trace_fields`, `_trace_crossings`, `_horizon[s]`, `_trace_[fans_]voxels`)
+ * `_trace_fan[s]`, `_trace_fields`, `_trace_crossings`, `_horizon[s]`, `_trace_[fans_]voxels`,
+ * `_trace_[fans_]opacity`)
  * return when their results are in place: ONE at a time per plan. DEVICE-pointer calls (`*_device`) are asynchronous on the
  * caller's stream: that is how a caller with several batches hides the tail of one (a launch
  * ends when its slowest ray does) behind the head of the next. A device-pointer call is IN
@@ -110,7 +111,7 @@ struct turtle_plan_counters {
  * that took its slot first is over. Host-pointer calls have slots of their own and may be
  * made while device-pointer calls are in flight; those that stage their arrays in device
  * memory of their own (turtle_stepper_step_batch, _walk_batch, _trace_crossings, _horizon[s],
- * _trace_[fans_]voxels) free it before they return, which waits for the device to be idle. After the caller has
+ * _trace_[fans_]voxels, _trace_[fans_]opacity) free it before they return, which waits for the device to be idle. After the caller has
  * synchronised, turtle_plan_counters_sync reports the device-pointer call issued last.
  * Several plans (one per host thread or per device) are independent; they share nothing but
  * read-only tiles of their own. This is the batched form of the reference's rule "one
@@ -465,6 +466,69 @@ TURTLE_API enum turtle_return turtle_stepper_trace_fans_voxels_device(struct tur
     const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
     const struct turtle_voxel_grid * grid, struct turtle_trace_result * results,
     struct turtle_voxel_entry * entries, int capacity, int32_t * count, void * stream);
+
+/* ---- opacity and its gradient over a voxel grid, without storing the matrix ----------------
+ * What a solver does with the L of turtle_stepper_trace_voxels is apply it (L rho, the forward
+ * model) and its transpose (L^T w, the gradient of a misfit with respect to the densities).
+ * These calls do both while they trace, and store no entry.
+ *
+ * L. Exactly the L of turtle_stepper_trace_voxels / _trace_fans_voxels on the same rays and
+ * grid: the row of ray i is its entries (k = 0 .. count[i] - 1, in order along the ray), with
+ * their media merged as a CSR matrix sums them.
+ * Rays and records. Rays are traced exactly as turtle_stepper_trace_voxels (for the fans form,
+ * turtle_stepper_trace_fans_voxels) traces them: same ray order, same steps, same bits.
+ * `results` (may be NULL) receives the plain trace's records byte for byte.
+ * Forward, exact. opacity[i] is acc = 0; for k in the entries of ray i, in order:
+ * acc = acc + density[voxel_k] * length_k, each product and each sum rounded on its own, in that
+ * order, with no fused multiply-add, on the very `length` doubles turtle_stepper_trace_voxels
+ * stores: bit for bit that loop on the host over its entries. Rays without an entry, and
+ * TURTLE_TRACE_INVALID rays, give 0.
+ * Outside. outside[i] is the length of the steps in selected media (grid->media) that lies
+ * outside the grid's box, summed in stepping order: the column of L for the rock the grid does
+ * not cover. A step that meets the box adds its parts before and after the box; a step that
+ * misses it adds its length. On a grid that encloses the ray it is exactly 0.
+ * Adjoint. Each entry k of ray i adds weight[i] * length_k (one rounded product) to
+ * gradient[voxel_k] with a device atomic. The order of the sums across rays is unspecified: the
+ * result is the exact sum of those products within (m_j - 1) * eps * sum |p| for the m_j
+ * products p of cell j. `gradient` is ADDED TO, never cleared: several calls may add into one
+ * array, device calls in flight together included. Zeroing it is the caller's job.
+ * Outputs. Each output is optional and needs only its own input: opacity needs density,
+ * gradient needs weight; the forward and the adjoint may be asked for in one call. Densities
+ * and weights are the caller's data and are not checked: a NaN propagates.
+ * Checks. The arguments are checked before the plan or the device is used. The grid is checked
+ * as by turtle_stepper_trace_voxels, with the same codes and messages. A missing opacity, grid
+ * or fans struct, missing positions or directions (n > 0), opacity without density, or gradient
+ * without weight are TURTLE_RETURN_BAD_ADDRESS. n = 0 or an empty fan grid does nothing.
+ * Memory. turtle_stepper_trace_opacity and _fans_opacity take HOST memory and return when the
+ * results are in place: density and gradient (n[0] * n[1] * n[2] doubles) and the per-ray arrays
+ * are staged in device memory of their own, gradient copied in and back, all freed before the
+ * return. The _device variants take DEVICE memory (the fans' arrays stay on the host, as for
+ * turtle_stepper_trace_fans_device), are one asynchronous launch on `stream` and hold one of
+ * the plan's 8 slots. The plan counters report rays, steps and samples as a trace does. */
+struct turtle_voxel_opacity {
+        const double * density; /* [n[0] * n[1] * n[2]] rho_j (cell index of turtle_voxel_entry), or NULL */
+        double * opacity;       /* [n] sum_j L_ij rho_j; needs density; or NULL */
+        double * outside;       /* [n] metres of the selected steps given to no cell, or NULL */
+        const double * weight;  /* [n] w_i, or NULL */
+        double * gradient;      /* [n[0] * n[1] * n[2]] ADDED TO: += sum_i w_i L_ij; needs weight; or NULL */
+};
+TURTLE_API enum turtle_return turtle_stepper_trace_opacity(struct turtle_plan * plan, size_t n,
+    const double * position, const double * direction, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, const struct turtle_voxel_opacity * opacity,
+    struct turtle_trace_result * results);
+TURTLE_API enum turtle_return turtle_stepper_trace_opacity_device(struct turtle_plan * plan,
+    size_t n, const double * position, const double * direction,
+    const struct turtle_trace_rule * rule, const struct turtle_voxel_grid * grid,
+    const struct turtle_voxel_opacity * opacity, struct turtle_trace_result * results,
+    void * stream);
+TURTLE_API enum turtle_return turtle_stepper_trace_fans_opacity(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, const struct turtle_voxel_opacity * opacity,
+    struct turtle_trace_result * results);
+TURTLE_API enum turtle_return turtle_stepper_trace_fans_opacity_device(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, const struct turtle_voxel_opacity * opacity,
+    struct turtle_trace_result * results, void * stream);
 
 /* ---- one turtle_stepper_step for n independent particles -------------------
  * Same outputs as the scalar call (any output pointer may be NULL; direction

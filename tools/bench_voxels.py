@@ -31,6 +31,43 @@ import bench  # noqa: E402  (the stack of the C2 / C3 configurations, unchanged)
 from bench_horizon import card  # noqa: E402
 
 
+class Survey:
+    """The scene, stations, fans and grid of the module docstring: plan, rule, fans, grid, n
+    (rays) and cells (along E, N, U)."""
+
+    def __init__(self, stations=8, n=256, cell=50.):
+        import turtle_b200 as tb
+        from oracle import harness as H
+        from tests.common import lambert_map
+
+        bench.make_stack()
+        lat0, lon0 = bench.DET_LAT, bench.DET_LON
+        lm = lambert_map(H.Driver(H.best_oracle()), lat_c=lat0, lon_c=lon0, n=401, half=12000.,
+                         nodes_per_degree=3600, lat0=bench.STACK_LAT0, lon0=bench.STACK_LON0)
+        stack = tb.Stack(bench.stack_dir())
+        lmap = tb.Map(lm["nx"], lm["ny"], lm["x"], lm["y"], lm["z"], lm["projection"], lm["values"])
+        stepper = tb.Stepper(range=0.)
+        stepper.add_stack(stack, 0.)
+        stepper.add_map(lmap, 0.)
+        self.plan = plan = stepper.freeze(0)
+        self.rule = tb.trace_rule(bench.ALTITUDE_MAX, max_steps=bench.MAX_STEPS)
+
+        rng = np.random.default_rng(2025)
+        la = lat0 + rng.uniform(-0.04, 0.04, stations)
+        lo = lon0 + rng.uniform(-0.05, 0.05, stations)
+        pos, index = plan.position(la, lo, np.ones(stations), 0)
+        assert (index >= 0).all()
+        az = (np.arange(n) + 0.5) * (360. / n)
+        el = -5. + 50. * (np.arange(n) + 0.5) / n
+        self.fans = tb.Plan.make_fans(la, lo, pos, az, el, bundle=32 if n % 32 == 0 else 1)
+        self.n = stations * n * n
+        half = 10000.
+        c = int(round(2 * half / cell))
+        self.cells = [c, c, int(round(5000. / cell))]
+        self.grid = tb.voxel_grid(lat0, lon0, 0., (-half, -half, -1000.), (cell,) * 3,
+                                  self.cells, 0b1)
+
+
 def main():
     p = argparse.ArgumentParser(description=__doc__.split("\n")[0])
     p.add_argument("--stations", type=int, default=8)
@@ -40,36 +77,11 @@ def main():
     args = p.parse_args()
 
     import torch
-    import turtle_b200 as tb
-    from oracle import harness as H
-    from tests.common import lambert_map
 
     who = card()
-    bench.make_stack()
-    lat0, lon0 = bench.DET_LAT, bench.DET_LON
-    lm = lambert_map(H.Driver(H.best_oracle()), lat_c=lat0, lon_c=lon0, n=401, half=12000.,
-                     nodes_per_degree=3600, lat0=bench.STACK_LAT0, lon0=bench.STACK_LON0)
-    stack = tb.Stack(bench.stack_dir())
-    lmap = tb.Map(lm["nx"], lm["ny"], lm["x"], lm["y"], lm["z"], lm["projection"], lm["values"])
-    stepper = tb.Stepper(range=0.)
-    stepper.add_stack(stack, 0.)
-    stepper.add_map(lmap, 0.)
-    plan = stepper.freeze(0)
-    rule = tb.trace_rule(bench.ALTITUDE_MAX, max_steps=bench.MAX_STEPS)
-
-    rng = np.random.default_rng(2025)
-    la = lat0 + rng.uniform(-0.04, 0.04, args.stations)
-    lo = lon0 + rng.uniform(-0.05, 0.05, args.stations)
-    pos, index = plan.position(la, lo, np.ones(args.stations), 0)
-    assert (index >= 0).all()
-    az = (np.arange(args.n) + 0.5) * (360. / args.n)
-    el = -5. + 50. * (np.arange(args.n) + 0.5) / args.n
-    fans = tb.Plan.make_fans(la, lo, pos, az, el, bundle=32 if args.n % 32 == 0 else 1)
-    n = args.stations * args.n * args.n
-    half = 10000.
-    cells = int(round(2 * half / args.cell))
-    grid = tb.voxel_grid(lat0, lon0, 0., (-half, -half, -1000.), (args.cell,) * 3,
-                         (cells, cells, int(round(5000. / args.cell))), 0b1)
+    sv = Survey(args.stations, args.n, args.cell)
+    plan, rule, fans, grid, n = sv.plan, sv.rule, sv.fans, sv.grid, sv.n
+    cells = sv.cells[0]
 
     count = torch.empty(n, dtype=torch.int32, device="cuda")
     plan.trace_fans_voxels_device(fans, rule, grid, 0, None, count)  # counting pass

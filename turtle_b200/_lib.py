@@ -80,6 +80,12 @@ class VoxelEntry(C.Structure):
     _fields_ = [("length", C.c_double), ("voxel", C.c_int32), ("medium", C.c_int32)]
 
 
+class VoxelOpacity(C.Structure):
+    """struct turtle_voxel_opacity (include/turtle_b200.h): the arrays of L @ rho and L.T @ w."""
+    _fields_ = [("density", C.c_void_p), ("opacity", C.c_void_p), ("outside", C.c_void_p),
+                ("weight", C.c_void_p), ("gradient", C.c_void_p)]
+
+
 class PlanCounters(C.Structure):
     """struct turtle_plan_counters (include/turtle_b200.h)."""
     _fields_ = [("rays", C.c_uint64), ("steps", C.c_uint64),
@@ -205,6 +211,16 @@ SIGNATURES = {
                                               C.POINTER(VoxelGrid), _P, _P, _I, _P]),
     "turtle_stepper_trace_fans_voxels_device": (_I, [_P, C.POINTER(Fans), C.POINTER(TraceRule),
                                                      C.POINTER(VoxelGrid), _P, _P, _I, _P, _P]),
+    "turtle_stepper_trace_opacity": (_I, [_P, _N, _P, _P, C.POINTER(TraceRule),
+                                          C.POINTER(VoxelGrid), C.POINTER(VoxelOpacity), _P]),
+    "turtle_stepper_trace_opacity_device": (_I, [_P, _N, _P, _P, C.POINTER(TraceRule),
+                                                 C.POINTER(VoxelGrid), C.POINTER(VoxelOpacity),
+                                                 _P, _P]),
+    "turtle_stepper_trace_fans_opacity": (_I, [_P, C.POINTER(Fans), C.POINTER(TraceRule),
+                                               C.POINTER(VoxelGrid), C.POINTER(VoxelOpacity), _P]),
+    "turtle_stepper_trace_fans_opacity_device": (_I, [_P, C.POINTER(Fans), C.POINTER(TraceRule),
+                                                      C.POINTER(VoxelGrid),
+                                                      C.POINTER(VoxelOpacity), _P, _P]),
     "turtle_stepper_horizon": (_I, [_P, _D, _D, _P, _N, _P, _D, _D, _D, C.POINTER(TraceRule), _P]),
     "turtle_stepper_horizon_device": (_I, [_P, _D, _D, _P, _N, _P, _D, _D, _D,
                                            C.POINTER(TraceRule), _P, _P]),

@@ -10,7 +10,7 @@ import ctypes as C
 import numpy as np
 
 from ._lib import (ERROR_HANDLER, Fan, Fans, MapInfo, PlanCounters, TraceFields, Residency, ResidencyReport, TraceRule,
-                   VoxelGrid, lib)
+                   VoxelGrid, VoxelOpacity, lib)
 
 TRACE_RESULT = np.dtype([
     ("position", "<f8", (3,)), ("altitude", "<f8"), ("length", "<f8", (4,)),
@@ -601,6 +601,82 @@ class Plan:
         _check(lib.turtle_stepper_trace_fans_voxels_device(
             self._p, C.byref(fans[0]), C.byref(rule), C.byref(grid), _ptr(results),
             _ptr(entries), capacity, _ptr(count), C.c_void_p(stream) if stream else None))
+
+    # ---- L @ rho and L.T @ w without storing L (turtle_stepper_trace_opacity) ---------------
+    @staticmethod
+    def _opacity_in(n, grid, density, weight, gradient, outside):
+        """Host arrays of a host call: (records, opacity, outside, gradient, struct)."""
+        cells = grid.n[0] * grid.n[1] * grid.n[2]
+        if density is not None:
+            density = _f8(density, (cells,))
+        if weight is not None:
+            weight = _f8(weight, (n,))
+            if gradient is None:
+                gradient = np.zeros(cells)
+        if gradient is not None and not (isinstance(gradient, np.ndarray) and
+                                         gradient.dtype == np.float64 and gradient.shape == (cells,)
+                                         and gradient.flags.c_contiguous and gradient.flags.writeable):
+            raise ValueError("gradient: a writeable contiguous float64 array of %d cells, added to"
+                             % cells)
+        opacity = np.zeros(n) if density is not None else None
+        outside = np.zeros(n) if outside else None
+        s = VoxelOpacity(*(a.ctypes.data if a is not None else None
+                           for a in (density, opacity, outside, weight, gradient)))
+        s._keep = (density, weight)
+        return np.zeros(n, dtype=TRACE_RESULT), opacity, outside, gradient, s
+
+    def trace_opacity(self, position, direction, rule, grid, density=None, weight=None,
+                      gradient=None, outside=False):
+        """turtle_stepper_trace_opacity: host rays in -> (records, opacity [n] = L @ density or
+        None, outside [n] (metres of the selected steps outside the grid) or None, gradient
+        [cells] or None). L is the matrix of trace_voxels on the same rays. With `weight` [n],
+        L.T @ weight is ADDED to `gradient` (a float64 array of grid.n[0] * n[1] * n[2] cells,
+        zeros when not given)."""
+        position, direction = _f8(position, (-1, 3)), _f8(direction, (-1, 3))
+        n = len(position)
+        results, opacity, out, gradient, s = self._opacity_in(n, grid, density, weight,
+                                                              gradient, outside)
+        _check(lib.turtle_stepper_trace_opacity(
+            self._p, n, _ptr(position), _ptr(direction), C.byref(rule), C.byref(grid),
+            C.byref(s), _ptr(results)))
+        return results, opacity, out, gradient
+
+    def trace_fans_opacity(self, fans, rule, grid, density=None, weight=None, gradient=None,
+                           outside=False):
+        """turtle_stepper_trace_fans_opacity: trace_opacity on the rays of make_fans(...), ray
+        order of trace_fans."""
+        f = fans[0]
+        n = f.n_station * f.n_azimuth * f.n_elevation
+        results, opacity, out, gradient, s = self._opacity_in(n, grid, density, weight,
+                                                              gradient, outside)
+        _check(lib.turtle_stepper_trace_fans_opacity(
+            self._p, C.byref(f), C.byref(rule), C.byref(grid), C.byref(s), _ptr(results)))
+        return results, opacity, out, gradient
+
+    @staticmethod
+    def _opacity_device(density, opacity, outside, weight, gradient):
+        return VoxelOpacity(*(_ptr(a).value if a is not None else None
+                              for a in (density, opacity, outside, weight, gradient)))
+
+    def trace_opacity_device(self, n, position, direction, rule, grid, density=None,
+                             opacity=None, outside=None, weight=None, gradient=None, results=None,
+                             stream=None):
+        """turtle_stepper_trace_opacity_device: device tensors in / out, one launch,
+        asynchronous; L.T @ weight is added to `gradient`."""
+        s = self._opacity_device(density, opacity, outside, weight, gradient)
+        _check(lib.turtle_stepper_trace_opacity_device(
+            self._p, n, _ptr(position), _ptr(direction), C.byref(rule), C.byref(grid),
+            C.byref(s), _ptr(results), C.c_void_p(stream) if stream else None))
+
+    def trace_fans_opacity_device(self, fans, rule, grid, density=None, opacity=None,
+                                  outside=None, weight=None, gradient=None, results=None,
+                                  stream=None):
+        """turtle_stepper_trace_fans_opacity_device: device tensors in / out, one launch,
+        asynchronous; L.T @ weight is added to `gradient`."""
+        s = self._opacity_device(density, opacity, outside, weight, gradient)
+        _check(lib.turtle_stepper_trace_fans_opacity_device(
+            self._p, C.byref(fans[0]), C.byref(rule), C.byref(grid), C.byref(s), _ptr(results),
+            C.c_void_p(stream) if stream else None))
 
     # ---- the horizon of a station (turtle_stepper_horizon) -------------------------------
     def horizon(self, latitude, longitude, position, azimuth, rule, elevation=(-90., 90.),

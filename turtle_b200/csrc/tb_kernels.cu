@@ -1191,11 +1191,19 @@ struct VoxelArgs {
         double frame[12];            /* origin, East, North, Up of the grid (fan_upload's frame) */
         double corner[3], size[3];
         int cells[3];
+        /* the opacity form (turtle_voxel_opacity): each pointer or NULL */
+        const double * density;  /* [cells] */
+        double * opacity;        /* [n] */
+        double * outside;        /* [n] */
+        const double * weight;   /* [n] */
+        double * gradient;       /* [cells], added to */
 };
 
 /* Per-ray rows of the voxel walk, next to the lane store: the ray in grid coordinates, the
- * path lengths where its line enters and leaves the grid, and the open entry. */
-enum { VF_U0 = 0, VF_V = 3, VF_TIN = 6, VF_TOUT, VF_OPEN, N_VF };
+ * path lengths where its line enters and leaves the grid, and the open entry; the opacity form
+ * adds its running sums and the ray's weight. */
+enum { VF_U0 = 0, VF_V = 3, VF_TIN = 6, VF_TOUT, VF_OPEN, N_VF,
+       VF_OPACITY = N_VF, VF_OUTSIDE, VF_WEIGHT, N_VF_OPACITY };
 enum { VI_CELL = 0, VI_MEDIUM, VI_COUNT, N_VI };
 
 /* Path length at which the ray line u0 + s v meets plane k of axis a of the grid. */
@@ -1204,12 +1212,20 @@ __device__ __forceinline__ double voxel_plane(const VoxelArgs & A, int a, int k,
         return (A.corner[a] + (double)k * A.size[a] - u0) / v;
 }
 
-/* Close the open entry of a lane: store it if it fits, count it. */
+/* Close the open entry of a lane: store it if it fits, count it. The opacity form consumes it
+ * instead: density x length into the lane's opacity, weight x length into the cell's gradient. */
+template <bool OPACITY, int NVF>
 __device__ __forceinline__ void voxel_close(const VoxelArgs & A, unsigned long long ray, int cell,
-    int medium, double length, int & count)
+    int medium, double length, int & count, double (&vf)[NVF][128], unsigned tid)
 {
         if (cell < 0) return;
-        if (count < A.capacity) {
+        if constexpr (OPACITY) {
+                if (A.density != NULL)
+                        vf[VF_OPACITY][tid] = __dadd_rn(vf[VF_OPACITY][tid],
+                            __dmul_rn(__ldg(A.density + cell), length));
+                if (A.gradient != NULL)
+                        atomicAdd(A.gradient + cell, __dmul_rn(vf[VF_WEIGHT][tid], length));
+        } else if (count < A.capacity) {
                 turtle_voxel_entry * e = A.entries + ray * (unsigned long long)A.capacity + count;
                 e->length = length;
                 e->voxel = cell;
@@ -1220,14 +1236,16 @@ __device__ __forceinline__ void voxel_close(const VoxelArgs & A, unsigned long l
 
 /* trace_kernel's rays (same samples, steps and bits, same queue and settle point), where the
  * length of every step that starts in a selected medium is split over the cells of the grid
- * by a 3-D DDA along the ray line, with cell planes at absolute path lengths. */
-template <bool LLA, bool PROJ, int MINB, int SHAPE>
+ * by a 3-D DDA along the ray line, with cell planes at absolute path lengths. OPACITY: the
+ * entries are consumed where they close (voxel_close) and the parts of the selected steps
+ * outside the grid are summed; the ray ends with its opacity and outside instead of a count. */
+template <bool LLA, bool PROJ, int MINB, int SHAPE, bool OPACITY>
 __global__ void __launch_bounds__(128, MINB)
     voxel_kernel(const __grid_constant__ tb::Geometry G, const __grid_constant__ VoxelArgs A)
 {
         constexpr int NF = LLA ? N_F_LLA : N_F_BASE, NI = LLA ? N_I : N_I_BASE;
         __shared__ LaneStoreT<NF, NI> store;
-        __shared__ double vf[N_VF][128];
+        __shared__ double vf[OPACITY ? N_VF_OPACITY : N_VF][128];
         __shared__ int vi[N_VI][128];
         const unsigned tid = threadIdx.x;
         const unsigned lane = tid & 31u;
@@ -1254,7 +1272,12 @@ __global__ void __launch_bounds__(128, MINB)
                                 reinterpret_cast<unsigned long long *>(A.results + ray)[lane] =
                                     record_field(store, t, lane);
                         if (lane == src) {
-                                A.count[ray] = vi[VI_COUNT][tid];
+                                if constexpr (OPACITY) {
+                                        if (A.opacity != NULL) A.opacity[ray] = vf[VF_OPACITY][tid];
+                                        if (A.outside != NULL) A.outside[ray] = vf[VF_OUTSIDE][tid];
+                                } else {
+                                        A.count[ray] = vi[VI_COUNT][tid];
+                                }
                                 mode = MODE_IDLE;
                         }
                 }
@@ -1284,6 +1307,12 @@ __global__ void __launch_bounds__(128, MINB)
                                                 mode = ray_start<LLA>(G, V, store, tid, r, pos, dir);
                                                 vi[VI_CELL][tid] = -1;
                                                 vi[VI_COUNT][tid] = 0;
+                                                if constexpr (OPACITY) {
+                                                        vf[VF_OPACITY][tid] = 0.;
+                                                        vf[VF_OUTSIDE][tid] = 0.;
+                                                        vf[VF_WEIGHT][tid] = (A.gradient != NULL) ?
+                                                            __ldg(A.weight + r) : 0.;
+                                                }
                                                 /* the ray in grid coordinates, and where its line
                                                  * enters and leaves the grid (+inf: never) */
                                                 double t_in = -DBL_MAX, t_out = DBL_MAX;
@@ -1440,6 +1469,13 @@ __global__ void __launch_bounds__(128, MINB)
                         /* ---- the step's segment through the grid ---- */
                         double s = fmax(s0, vf[VF_TIN][tid]);
                         const double s_end = fmin(total, vf[VF_TOUT][tid]);
+                        if constexpr (OPACITY) {
+                                /* the parts of a selected step before and after the box, or
+                                 * all of it when it misses the box */
+                                if (((unsigned)medium0 < 32u) && ((A.media >> medium0) & 1u))
+                                        vf[VF_OUTSIDE][tid] = __dadd_rn(vf[VF_OUTSIDE][tid], (s < s_end) ?
+                                            __dadd_rn(__dsub_rn(s, s0), __dsub_rn(total, s_end)) : ds);
+                        }
                         if (((unsigned)medium0 < 32u) && ((A.media >> medium0) & 1u) && (s < s_end)) {
                                 int i[3];
                                 double next[3];
@@ -1476,7 +1512,8 @@ __global__ void __launch_bounds__(128, MINB)
                                                 if ((cell == open_cell) && (medium0 == open_medium)) {
                                                         open_length += e - s;
                                                 } else {
-                                                        voxel_close(A, ray, open_cell, open_medium, open_length, count);
+                                                        voxel_close<OPACITY>(A, ray, open_cell, open_medium,
+                                                            open_length, count, vf, tid);
                                                         open_cell = cell;
                                                         open_medium = medium0;
                                                         open_length = e - s;
@@ -1506,7 +1543,8 @@ __global__ void __launch_bounds__(128, MINB)
                 if (status >= 0) {
                         SI(I_MEDIUM0) = status;
                         int count = vi[VI_COUNT][tid];
-                        voxel_close(A, ray, vi[VI_CELL][tid], vi[VI_MEDIUM][tid], vf[VF_OPEN][tid], count);
+                        voxel_close<OPACITY>(A, ray, vi[VI_CELL][tid], vi[VI_MEDIUM][tid], vf[VF_OPEN][tid],
+                            count, vf, tid);
                         vi[VI_COUNT][tid] = count;
                         mode = MODE_DONE;
                 } else {
@@ -4402,6 +4440,31 @@ extern "C" enum turtle_return turtle_stepper_trace_crossings(
 
 /* ---- rock length per cell of a voxel grid ------------------------------------------------ */
 
+/* The cells, frame and media of a grid (its address is checked by the caller). */
+static enum turtle_return check_voxel_grid(turtle_function_t * fn,
+    const struct turtle_voxel_grid * grid)
+{
+        const int32_t * c = grid->n;
+        if ((c[0] <= 0) || (c[1] <= 0) || (c[2] <= 0) ||
+            ((long long)c[0] * (long long)c[1] * (long long)c[2] > (long long)INT32_MAX))
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "invalid voxel grid of %d x %d x %d cells (must be > 0, at most %d in all)",
+                    c[0], c[1], c[2], INT32_MAX);
+        const double * s = grid->size;
+        if (!(isfinite(s[0]) && (s[0] > 0.) && isfinite(s[1]) && (s[1] > 0.) && isfinite(s[2]) &&
+                (s[2] > 0.)))
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "invalid voxel size %g x %g x %g m (must be finite and > 0)", s[0], s[1], s[2]);
+        if (!(isfinite(grid->latitude) && isfinite(grid->longitude) && isfinite(grid->height) &&
+                isfinite(grid->corner[0]) && isfinite(grid->corner[1]) && isfinite(grid->corner[2])))
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "invalid voxel grid origin or corner (must be finite)");
+        if (grid->media == 0u)
+                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
+                    "invalid voxel media 0 (select at least one medium)");
+        return TURTLE_RETURN_SUCCESS;
+}
+
 /* Arguments first (no plan, no device needed). `rays`: the position and direction arrays of
  * the explicit form are needed (n > 0, not a fan). */
 static enum turtle_return check_voxels(turtle_function_t * fn, size_t n, bool rays,
@@ -4421,34 +4484,44 @@ static enum turtle_return check_voxels(turtle_function_t * fn, size_t n, bool ra
         if (capacity < 0)
                 return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
                     "invalid voxel capacity %d (must be >= 0)", capacity);
-        const int32_t * c = grid->n;
-        if ((c[0] <= 0) || (c[1] <= 0) || (c[2] <= 0) ||
-            ((long long)c[0] * (long long)c[1] * (long long)c[2] > (long long)INT32_MAX))
-                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
-                    "invalid voxel grid of %d x %d x %d cells (must be > 0, at most %d in all)",
-                    c[0], c[1], c[2], INT32_MAX);
-        const double * s = grid->size;
-        if (!(isfinite(s[0]) && (s[0] > 0.) && isfinite(s[1]) && (s[1] > 0.) && isfinite(s[2]) &&
-                (s[2] > 0.)))
-                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
-                    "invalid voxel size %g x %g x %g m (must be finite and > 0)", s[0], s[1], s[2]);
-        if (!(isfinite(grid->latitude) && isfinite(grid->longitude) && isfinite(grid->height) &&
-                isfinite(grid->corner[0]) && isfinite(grid->corner[1]) && isfinite(grid->corner[2])))
-                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
-                    "invalid voxel grid origin or corner (must be finite)");
-        if (grid->media == 0u)
-                return tbh::raise(fn, TURTLE_RETURN_DOMAIN_ERROR, BATCH_CU, __LINE__,
-                    "invalid voxel media 0 (select at least one medium)");
+        const enum turtle_return rc = check_voxel_grid(fn, grid);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        return check_rule(fn, rule);
+}
+
+/* The same for the opacity form: its arrays instead of entries and counts. */
+static enum turtle_return check_opacity(turtle_function_t * fn, size_t n, bool rays,
+    const double * position, const double * direction, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, const struct turtle_voxel_opacity * opacity)
+{
+        if (grid == NULL)
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
+                    "missing voxel grid");
+        if (opacity == NULL)
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
+                    "missing voxel opacity arrays");
+        if ((n > 0) && rays && ((position == NULL) || (direction == NULL)))
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
+                    "missing ray positions or directions");
+        if ((opacity->opacity != NULL) && (opacity->density == NULL))
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
+                    "missing voxel densities (an opacity needs them)");
+        if ((opacity->gradient != NULL) && (opacity->weight == NULL))
+                return tbh::raise(fn, TURTLE_RETURN_BAD_ADDRESS, BATCH_CU, __LINE__,
+                    "missing ray weights (a gradient needs them)");
+        const enum turtle_return rc = check_voxel_grid(fn, grid);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
         return check_rule(fn, rule);
 }
 
 /* Queue the voxel kernel on `stream` with the counter block of `slot`: the rays of
- * `d_position` / `d_direction` (device memory), or of the fan tables `fan`. */
+ * `d_position` / `d_direction` (device memory), or of the fan tables `fan`. `opacity` (device
+ * arrays) selects the opacity form, which takes no entries or counts. */
 static cudaError_t launch_voxels(struct turtle_plan * plan, int slot, size_t n,
     const double * d_position, const double * d_direction, const FanTables * fan,
     const struct turtle_trace_rule * rule, const struct turtle_voxel_grid * grid,
     struct turtle_trace_result * results, struct turtle_voxel_entry * entries, int capacity,
-    int32_t * count, cudaStream_t stream)
+    int32_t * count, const struct turtle_voxel_opacity * opacity, cudaStream_t stream)
 {
         unsigned long long * d_counters = plan->d_counters + CTR * slot;
         cudaError_t err = cudaMemsetAsync(d_counters, 0x0, CTR * sizeof(unsigned long long), stream);
@@ -4479,11 +4552,23 @@ static cudaError_t launch_voxels(struct turtle_plan * plan, int slot, size_t n,
                 A.size[a] = grid->size[a];
                 A.cells[a] = grid->n[a];
         }
+        if (opacity != NULL) {
+                A.density = opacity->density;
+                A.opacity = opacity->opacity;
+                A.outside = opacity->outside;
+                A.weight = opacity->weight;
+                A.gradient = opacity->gradient;
+        }
         const Variant v = variant_of(plan);
-        void (*kernel)(const tb::Geometry, const VoxelArgs) = with_variant(v, [](auto V) {
-                typedef decltype(V) K;
-                return voxel_kernel<K::LLA, K::PROJ, K::MINB, K::SHAPE>;
-        });
+        void (*kernel)(const tb::Geometry, const VoxelArgs) = (opacity != NULL) ?
+            with_variant(v, [](auto V) {
+                    typedef decltype(V) K;
+                    return voxel_kernel<K::LLA, K::PROJ, K::MINB, K::SHAPE, true>;
+            }) :
+            with_variant(v, [](auto V) {
+                    typedef decltype(V) K;
+                    return voxel_kernel<K::LLA, K::PROJ, K::MINB, K::SHAPE, false>;
+            });
         const size_t dynamic = v.lla ? lla_bytes(plan) : 0;
         if (dynamic > 0)
                 cudaFuncSetAttribute(kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)dynamic);
@@ -4502,12 +4587,12 @@ static cudaError_t launch_voxels(struct turtle_plan * plan, int slot, size_t n,
 }
 
 /* Checked arguments, n > 0: host memory, results in place on return. `fans` NULL: the rays of
- * position / direction. */
+ * position / direction. `opacity` (host arrays): the opacity form, without entries or counts. */
 static enum turtle_return voxels_host(turtle_function_t * fn, struct turtle_plan * plan, size_t n,
     const double * position, const double * direction, const struct turtle_fans * fans,
     size_t bundle, const struct turtle_trace_rule * rule, const struct turtle_voxel_grid * grid,
     struct turtle_trace_result * results, struct turtle_voxel_entry * entries, int capacity,
-    int32_t * count)
+    int32_t * count, const struct turtle_voxel_opacity * opacity = NULL)
 {
         CUDA_TRY(fn, cudaSetDevice(plan->device));
         DeviceBuffers buf;
@@ -4524,27 +4609,51 @@ static enum turtle_return voxels_host(turtle_function_t * fn, struct turtle_plan
         /* the caller's slots past each count stay as they are: staged in, copied back whole */
         if (capacity > 0) DEV_IN(fn, buf, d_entries, entries, entry_bytes);
         DEV_OUT(fn, buf, d_count, count, n * sizeof(*d_count));
+        /* the opacity form: densities and weights in, the gradient in and back (it is added
+         * to), opacity and outside out */
+        turtle_voxel_opacity D;
+        memset(&D, 0x0, sizeof D);
+        const size_t cell_bytes = (size_t)grid->n[0] * (size_t)grid->n[1] * (size_t)grid->n[2] *
+            sizeof(double);
+        if (opacity != NULL) {
+                double *d_density = NULL, *d_weight = NULL, *d_gradient = NULL;
+                if (opacity->density != NULL) DEV_IN(fn, buf, d_density, opacity->density, cell_bytes);
+                if (opacity->weight != NULL) DEV_IN(fn, buf, d_weight, opacity->weight, n * sizeof(double));
+                if (opacity->gradient != NULL) DEV_IN(fn, buf, d_gradient, opacity->gradient, cell_bytes);
+                DEV_OUT(fn, buf, D.opacity, opacity->opacity, n * sizeof(double));
+                DEV_OUT(fn, buf, D.outside, opacity->outside, n * sizeof(double));
+                D.density = d_density;
+                D.weight = d_weight;
+                D.gradient = d_gradient;
+        }
         /* a host-pointer call: the counter block and tables of the host pipeline's slot 0 */
         memset(&plan->counters, 0x0, sizeof(plan->counters));
         plan->counters.rays = n;
         FanTables T;
         if (fans != NULL) CUDA_TRY(fn, fan_upload(plan, 0, fans, bundle, 0, NULL, &T));
         CUDA_TRY(fn, launch_voxels(plan, 0, n, d_pos, d_dir, (fans != NULL) ? &T : NULL, rule,
-                         grid, d_res, d_entries, capacity, d_count, NULL));
+                         grid, d_res, d_entries, capacity, d_count, (opacity != NULL) ? &D : NULL,
+                         NULL));
         CUDA_TRY(fn, cudaDeviceSynchronize());
         read_counters(plan, 0);
         DEV_BACK(fn, results, d_res, n * sizeof(*d_res));
         if (capacity > 0) DEV_BACK(fn, entries, d_entries, entry_bytes);
         DEV_BACK(fn, count, d_count, n * sizeof(*d_count));
+        if (opacity != NULL) {
+                DEV_BACK(fn, opacity->opacity, D.opacity, n * sizeof(double));
+                DEV_BACK(fn, opacity->outside, D.outside, n * sizeof(double));
+                DEV_BACK(fn, opacity->gradient, D.gradient, cell_bytes);
+        }
         return TURTLE_RETURN_SUCCESS;
 }
 
-/* Checked arguments, n > 0: device memory, one launch, asynchronous on `stream`. */
+/* Checked arguments, n > 0: device memory, one launch, asynchronous on `stream`. `opacity`
+ * (device arrays): the opacity form. */
 static enum turtle_return voxels_device(turtle_function_t * fn, struct turtle_plan * plan, size_t n,
     const double * position, const double * direction, const struct turtle_fans * fans,
     size_t bundle, const struct turtle_trace_rule * rule, const struct turtle_voxel_grid * grid,
     struct turtle_trace_result * results, struct turtle_voxel_entry * entries, int capacity,
-    int32_t * count, void * stream)
+    int32_t * count, void * stream, const struct turtle_voxel_opacity * opacity = NULL)
 {
         return device_call(fn, plan, true, n, (cudaStream_t)stream, [&](int slot) {
                 FanTables T;
@@ -4553,7 +4662,7 @@ static enum turtle_return voxels_device(turtle_function_t * fn, struct turtle_pl
                 if (err == cudaSuccess)
                         err = launch_voxels(plan, slot, n, position, direction,
                             (fans != NULL) ? &T : NULL, rule, grid, results, entries, capacity, count,
-                            (cudaStream_t)stream);
+                            opacity, (cudaStream_t)stream);
                 return err;
         });
 }
@@ -4621,6 +4730,71 @@ extern "C" enum turtle_return turtle_stepper_trace_fans_voxels_device(struct tur
         if (rc != TURTLE_RETURN_SUCCESS) return rc;
         return voxels_device(fn, plan, n, NULL, NULL, fans, bundle, rule, grid, results, entries,
             capacity, count, stream);
+}
+
+/* ---- L rho and L^T w over a voxel grid without storing L ------------------------------------ */
+
+extern "C" enum turtle_return turtle_stepper_trace_opacity(struct turtle_plan * plan, size_t n,
+    const double * position, const double * direction, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, const struct turtle_voxel_opacity * opacity,
+    struct turtle_trace_result * results)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_trace_opacity);
+        enum turtle_return rc = check_opacity(fn, n, true, position, direction, rule, grid, opacity);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        rc = check_plan(fn, plan);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        return voxels_host(fn, plan, n, position, direction, NULL, 1, rule, grid, results, NULL, 0,
+            NULL, opacity);
+}
+
+extern "C" enum turtle_return turtle_stepper_trace_opacity_device(struct turtle_plan * plan,
+    size_t n, const double * position, const double * direction,
+    const struct turtle_trace_rule * rule, const struct turtle_voxel_grid * grid,
+    const struct turtle_voxel_opacity * opacity, struct turtle_trace_result * results,
+    void * stream)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_trace_opacity_device);
+        enum turtle_return rc = check_opacity(fn, n, true, position, direction, rule, grid, opacity);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        rc = check_plan(fn, plan);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        return voxels_device(fn, plan, n, position, direction, NULL, 1, rule, grid, results, NULL,
+            0, NULL, stream, opacity);
+}
+
+extern "C" enum turtle_return turtle_stepper_trace_fans_opacity(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, const struct turtle_voxel_opacity * opacity,
+    struct turtle_trace_result * results)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_trace_fans_opacity);
+        size_t n, bundle;
+        enum turtle_return rc = check_fans(fn, fans, &n, &bundle);
+        if (rc == TURTLE_RETURN_SUCCESS)
+                rc = check_opacity(fn, n, false, NULL, NULL, rule, grid, opacity);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        rc = check_plan(fn, plan);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        return voxels_host(fn, plan, n, NULL, NULL, fans, bundle, rule, grid, results, NULL, 0,
+            NULL, opacity);
+}
+
+extern "C" enum turtle_return turtle_stepper_trace_fans_opacity_device(struct turtle_plan * plan,
+    const struct turtle_fans * fans, const struct turtle_trace_rule * rule,
+    const struct turtle_voxel_grid * grid, const struct turtle_voxel_opacity * opacity,
+    struct turtle_trace_result * results, void * stream)
+{
+        turtle_function_t * fn = FN(&turtle_stepper_trace_fans_opacity_device);
+        size_t n, bundle;
+        enum turtle_return rc = check_fans(fn, fans, &n, &bundle);
+        if (rc == TURTLE_RETURN_SUCCESS)
+                rc = check_opacity(fn, n, false, NULL, NULL, rule, grid, opacity);
+        if ((rc != TURTLE_RETURN_SUCCESS) || (n == 0)) return rc;
+        rc = check_plan(fn, plan);
+        if (rc != TURTLE_RETURN_SUCCESS) return rc;
+        return voxels_device(fn, plan, n, NULL, NULL, fans, bundle, rule, grid, results, NULL, 0,
+            NULL, stream, opacity);
 }
 
 extern "C" enum turtle_return turtle_map_resample(struct turtle_map * map,
@@ -5386,6 +5560,10 @@ extern "C" const char * tb_batch_function_name(turtle_function_t * caller)
         NAME(turtle_stepper_trace_voxels_device);
         NAME(turtle_stepper_trace_fans_voxels);
         NAME(turtle_stepper_trace_fans_voxels_device);
+        NAME(turtle_stepper_trace_opacity);
+        NAME(turtle_stepper_trace_opacity_device);
+        NAME(turtle_stepper_trace_fans_opacity);
+        NAME(turtle_stepper_trace_fans_opacity_device);
         NAME(turtle_b200_peer_alloc);
         NAME(turtle_b200_peer_free);
         NAME(turtle_b200_peer_export);
